@@ -1,6 +1,7 @@
 """bench.py -- LatentAugment hot path throughput: augmented images / second.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--config c2|c3|c5|c1] [--precision bf16]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
 
@@ -21,10 +22,15 @@ the gathered per-rank lists), ``c3_strong_split`` (batch 128 split over the N ra
 (all four criteria at the author's weights).  ``--no-extras`` skips them; a
 watchdog (``--extras-timeout``) prints the line without them if a leg wedges, and ``destroy_process_group`` runs under its
 own (tests/test_bench_flow.py exercises all of this on CPU with stand-ins for the CUDA-facing pieces).
+
+``--dump-outputs DIR`` writes what the last timed step of the headline leg returned (``img``, ``w_aug``) as
+``DIR/<name>.npy`` in float32, so that two builds can be compared output for output: every input, and the random noise of
+the final synthesis, comes from fixed seeds, so the same arguments give the same inputs in every run.
 """
 import argparse
 import json
 import os
+import random
 import subprocess
 import sys
 import threading
@@ -40,6 +46,7 @@ CONFIGS = {          # BASELINE.json configs; oracle/synthetic.py holds the same
     'tiny': dict(img_resolution=32, img_channels=2, batch=4, steps=3, bank=64, img_bank=8, channel_base=2048, channel_max=64),
 }
 C5 = dict(codes=1 << 20, queries=1024, dim=512, k=4)
+DUMP_LIMIT = 64 << 20        # bytes that --dump-outputs writes at most
 
 
 def layer_table(res, img_c, channel_base=32768, channel_max=512):
@@ -219,7 +226,7 @@ class PluginTimer:
 
     def resident(self, warmup, steps, clocks=None):
         """-> (ms per step as the max over ranks, launches of this rank, the device-resident code batches); ``self.mark`` =
-        the clock sampler's position when the timed region starts"""
+        the clock sampler's position when the timed region starts, ``self.last`` = what the last timed step returned"""
         import torch
         aug, core = self.aug, self.core
         w_dev = [aug.sample_from_inversion(self.batch_data(i)['A_paths']).to(self.dev) for i in range(warmup + steps)]
@@ -231,7 +238,7 @@ class PluginTimer:
         ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         ev0.record()
         for i in range(steps):
-            core.forward(w_dev[warmup + i])
+            self.last = core.forward(w_dev[warmup + i])
         ev1.record()
         self.barrier()
         launches = sum(e.launch_count for e in core.engines) - l0
@@ -254,6 +261,22 @@ class PluginTimer:
         torch.cuda.synchronize()
         t1 = time.perf_counter()
         return self.max_over_ranks(t1 - t0) / steps, out
+
+
+def dump_outputs(path, arrays, limit=DUMP_LIMIT):
+    """Writes each tensor of ``arrays`` as ``path/<name>.npy`` in float32.  When they exceed ``limit`` bytes in all, each
+    keeps the same fixed, seeded subset of its leading-dimension rows (in ascending order), sized to fit."""
+    import numpy as np
+    import torch
+    os.makedirs(path, exist_ok=True)
+    total = sum(4 * t.numel() for t in arrays.values())
+    for name, t in arrays.items():
+        t = t.detach().float()
+        if total > limit:
+            n = t.shape[0]
+            rows = torch.randperm(n, generator=torch.Generator().manual_seed(0))[:max(1, n * limit // total)].sort().values
+            t = t[rows.to(t.device)]
+        np.save(os.path.join(path, f'{name}.npy'), t.cpu().numpy())
 
 
 def _full_cfg(cfg_name):
@@ -604,7 +627,13 @@ def main():
     ap.add_argument('--teardown-timeout', type=float, default=30.0, help='watchdog of destroy_process_group, seconds')
     ap.add_argument('--profile', action='store_true', help='short run for ncu: skips the e2e leg, the baselines and the per-GEMM timing')
     ap.add_argument('--layers-out', default='', help='write the per-layer tap-GEMM timing table (JSON) here')
+    ap.add_argument('--dump-outputs', default='', metavar='DIR',
+                    help="write rank 0's outputs of the last timed step (img, w_aug) as DIR/<name>.npy, float32, at most 64 MB "
+                         'in all (beyond that, a fixed seeded subset of the batch)')
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl == 'reference' or args.config == 'c5'):
+        ap.error('--dump-outputs writes the outputs of the synthesis path: not with --impl reference or --config c5')
+    sys.dont_write_bytecode = True          # the tree may be read-only: no bytecode caches are written into it
     if args.impl == 'reference':
         return run_reference(args)
     if args.config == 'c5':
@@ -618,6 +647,8 @@ def main():
     world = int(os.environ.get('WORLD_SIZE', '1'))
     if args.warmup < 3:
         args.warmup = 3
+    random.seed(0)            # crop windows of the perceptual term
+    torch.manual_seed(0)      # noise of the final synthesis
     torch.cuda.set_device(local_rank)
     dev = cuda_device(local_rank)
     # stdout carries exactly ONE JSON line: everything else (plugin banners, the NCCL version line that
@@ -649,6 +680,8 @@ def main():
     ms, launches, w_dev = pt.resident(args.warmup, args.steps, clocks)
     mark = pt.mark
     value = world * B / (ms * 1e-3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, dict(zip(('img', 'w_aug'), pt.last)))
 
     if args.profile:
         clocks.stop(mark)

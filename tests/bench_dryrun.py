@@ -98,7 +98,7 @@ class FakeCore:
 
     def forward(self, w):
         self.engines[0].launch_count += 64
-        return torch.zeros([self.B, self.C, 4, 4]), w
+        return torch.full([self.B, self.C, 4, 4], float(self.engines[0].launch_count // 64)), w      # pixel = number of this call
 
 
 class FakeAug:

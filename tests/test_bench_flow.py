@@ -49,6 +49,35 @@ def test_one_line_with_both_extra_legs_single_process():
     assert rc == 0 and len(lines) == 1 and 'c5_sharded_search' not in json.loads(lines[0]), err[-2000:]
 
 
+def test_dump_outputs_of_the_last_timed_step(tmp_path):
+    import numpy as np
+    out = tmp_path / 'out'
+    rc, lines, _, err = _run(1, ['--no-extras', '--warmup', '3', '--steps', '4', '--dump-outputs', str(out)])
+    assert rc == 0 and len(lines) == 1, err[-2000:]
+    assert json.loads(lines[0])['steps'] == 4
+    assert sorted(os.listdir(out)) == ['img.npy', 'w_aug.npy']
+    img, w = np.load(out / 'img.npy'), np.load(out / 'w_aug.npy')
+    assert img.dtype == w.dtype == np.float32 and img.shape == (2, 3, 4, 4) and w.shape == (2, 1, 8)
+    assert (img == 3 + 4).all()                  # the stand-in's pixels count its calls: 3 warm-up + 4 timed steps
+
+
+def test_dump_outputs_sample_fixed_rows_beyond_the_limit(tmp_path):
+    import numpy as np
+    import torch
+
+    import bench
+    a, b = torch.arange(64.0).reshape(16, 4), -torch.arange(32.0).reshape(16, 2)
+    for d in ('x', 'y'):
+        bench.dump_outputs(str(tmp_path / d), {'a': a, 'b': b.double()}, limit=200)
+    ra, rb = np.load(tmp_path / 'x' / 'a.npy'), np.load(tmp_path / 'x' / 'b.npy')
+    assert ra.dtype == rb.dtype == np.float32 and ra.nbytes + rb.nbytes <= 200 and ra.shape == (8, 4) and rb.shape == (8, 2)
+    rows = ra[:, 0].astype(np.int64) // 4
+    assert (np.diff(rows) > 0).all() and (rb[:, 0] == -2 * rows).all()          # the same ascending rows of both arrays
+    assert (np.load(tmp_path / 'y' / 'a.npy') == ra).all()                       # and the same rows in every run
+    bench.dump_outputs(str(tmp_path / 'z'), {'a': a}, limit=a.numel() * 4)
+    assert (np.load(tmp_path / 'z' / 'a.npy') == a.numpy()).all()
+
+
 def test_two_ranks_gloo_merge_check_and_teardown():
     rc, lines, _, err = _run(2)
     assert rc == 0 and len(lines) == 1, err[-2000:]
