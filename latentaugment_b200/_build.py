@@ -22,7 +22,7 @@ CSRC = os.path.join(PKG, 'csrc')
 LIB = os.path.join(PKG, 'liblatentaugment_b200.so')
 STAMP = LIB + '.srchash'
 SOURCES = ['tapgemm.cu', 'kernels.cu', 'distance.cu', 'engine.cu', 'disc.cu', 'filtered_lrelu.cu', 'lpips.cu']
-HEADERS = ['tapgemm.cuh', 'kernels.cuh', 'sm100.cuh', 'plan.cuh', 'disc.cuh', 'lpips.cuh',
+HEADERS = ['act.cuh', 'tapgemm.cuh', 'kernels.cuh', 'sm100.cuh', 'plan.cuh', 'disc.cuh', 'lpips.cuh',
            os.path.join(ROOT, 'include', 'latentaugment_b200.h')]
 NVCC_FLAGS = ['-gencode', 'arch=compute_100a,code=sm_100a', '-lineinfo', '-O3', '-std=c++17',
               '-Xcompiler', '-fPIC', '-Xcompiler', '-fvisibility=hidden']

@@ -74,12 +74,30 @@ def reference_network_pickle_path(opt):
     return os.path.join(dir_model, runs[0], opt.network_pkl_stylegan)
 
 
+def network_kwargs(nets):
+    """The constructor arguments of a network pickle's modules that change what the engine computes, read from their
+    ``init_kwargs`` (``torch_utils/persistence.py``): ``conv_clamp`` of G's synthesis network (``None`` for ``--cfg stylegan2``
+    networks), ``disc_conv_clamp`` and ``mbstd_group_size`` of D (8 for the ``paper256`` / ``paper512`` configs).  Only the
+    keys the pickle carries are returned; ``None`` means no clamp."""
+    out = {}
+    g_kw = getattr(nets.get('G_ema'), 'init_kwargs', None) or {}
+    if 'conv_clamp' in (g_kw.get('synthesis_kwargs') or {}):
+        out['conv_clamp'] = g_kw['synthesis_kwargs']['conv_clamp']
+    d_kw = getattr(nets.get('D'), 'init_kwargs', None) or {}
+    if 'conv_clamp' in d_kw:
+        out['disc_conv_clamp'] = d_kw['conv_clamp']
+    if 'mbstd_group_size' in (d_kw.get('epilogue_kwargs') or {}):
+        out['mbstd_group_size'] = d_kw['epilogue_kwargs']['mbstd_group_size']
+    return out
+
+
 def load_stylegan_states(path):
     """``G_ema`` / ``D`` of a reference network pickle as plain ``state_dict``s (:473-484 keeps the modules; the engine reads
-    parameters only).  The pickles embed the source of their classes and need the reference's ``torch_utils`` / ``dnnlib``
-    importable (``torch_utils/persistence.py:118-227``) -- true inside the reference's code base, which is where this
-    plugin is dropped in; elsewhere convert once with ``tools/export_reference_pickle.py``.  Plain ``pickle.load`` as in the
-    reference: only open files you trust."""
+    parameters only), and the modules' constructor arguments the engine needs (``network_kwargs``).  The pickles embed the
+    source of their classes and need the reference's ``torch_utils`` / ``dnnlib`` importable
+    (``torch_utils/persistence.py:118-227``) -- true inside the reference's code base, which is where this plugin is dropped
+    in; elsewhere convert once with ``tools/export_reference_pickle.py``.  Plain ``pickle.load`` as in the reference: only
+    open files you trust."""
     import pickle
     print(f'Loading stylegan from "{path}"...')
     try:
@@ -93,7 +111,7 @@ def load_stylegan_states(path):
     def sd(net):
         return {k: v.detach().cpu().float() for k, v in net.state_dict().items()}
     print('Done.')
-    return sd(nets['G_ema']), (sd(nets['D']) if 'D' in nets else None)
+    return sd(nets['G_ema']), (sd(nets['D']) if 'D' in nets else None), network_kwargs(nets)
 
 
 class InvertedCodeTable:
@@ -158,13 +176,13 @@ class LatentAug:
         self.module = self
 
         # ---- generator (reference: load_stylegan, :466-484)
-        pickle_disc_state = None
+        pickle_disc_state, net_kw = None, {}
         if generator_state is None:
             pkl = None if getattr(opt, 'generator_state', '') else reference_network_pickle_path(opt)
             if getattr(opt, 'generator_state', ''):
                 generator_state = torch.load(opt.generator_state, map_location='cpu', weights_only=True)
             elif pkl is not None:                                    # the reference's own --model_dir tree and pickle
-                generator_state, pickle_disc_state = load_stylegan_states(pkl)
+                generator_state, pickle_disc_state, net_kw = load_stylegan_states(pkl)
             elif getattr(opt, 'synthetic', False):
                 generator_state = synthetic.random_generator_state(
                     img_resolution=opt.img_resolution, img_channels=opt.synthetic_channels,
@@ -178,7 +196,9 @@ class LatentAug:
         self.res, self.img_channels = kw['img_resolution'], kw['img_channels']
         self.w_dim, self.z_dim = kw['w_dim'], kw['z_dim']
         self.modalities = list(range(self.img_channels))
-        conv_clamp = getattr(opt, 'conv_clamp', 256.0)
+        # the pickle's own constructor arguments (None: no clamp); without a pickle the networks' defaults
+        default_clamp = getattr(opt, 'conv_clamp', 256.0)
+        conv_clamp = net_kw.get('conv_clamp', default_clamp)
         self.engines = []
         if self.micro > 1 and self.w_disc > 0:
             raise ValueError('--micro_batches > 1 changes the discriminator\'s minibatch-stddev groups: use 1 with w_disc > 0')
@@ -230,11 +250,12 @@ class LatentAug:
                 self.criteria['pix'].attach(e, self.X)
         # ---- discriminator of the realism term (reference: self.D from the same pickle, :117)
         if self.w_disc > 0:
-            disc_state = None
+            disc_state, disc_kw = None, dict(conv_clamp=default_clamp)
             if getattr(opt, 'discriminator_state', ''):
                 disc_state = torch.load(opt.discriminator_state, map_location='cpu', weights_only=True)
             elif pickle_disc_state is not None:                      # D of the same pickle, as the reference (:117)
                 disc_state = pickle_disc_state
+                disc_kw = dict(conv_clamp=net_kw.get('disc_conv_clamp', default_clamp), mbstd_group_size=net_kw.get('mbstd_group_size', 4))
             elif getattr(opt, 'synthetic', False):
                 disc_state = synthetic.random_discriminator_state(
                     img_resolution=self.res, img_channels=self.img_channels, channel_base=opt.synthetic_channel_base,
@@ -243,7 +264,7 @@ class LatentAug:
                 raise FileNotFoundError('w_disc > 0 needs a discriminator: --discriminator_state <state_dict.pt> '
                                         '(reference names, legacy.py:267-287) or --synthetic')
             for e in self.engines:
-                self.criteria['disc'].attach(e, disc_state, conv_clamp=conv_clamp)
+                self.criteria['disc'].attach(e, disc_state, **disc_kw)
         # ---- perceptual term (reference: self.vgg16 / self.lpips + register_buffer('fea_{mode}'), :125-131,160-181)
         if self.w_lpips > 0:
             vgg_state = None

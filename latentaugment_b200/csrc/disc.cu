@@ -21,6 +21,7 @@
 #include <string>
 #include <vector>
 
+#include "act.cuh"
 #include "kernels.cuh"
 #include "plan.cuh"
 #include "tapgemm.cuh"
@@ -83,10 +84,6 @@ __device__ __forceinline__ void st_sp2(unsigned* hi, unsigned* lo, long long i, 
 __device__ __forceinline__ float act_fwd(float z, float gain, float slope, float clamp) {
     z = (z > 0.f ? z : z * slope) * gain;
     return clamp >= 0.f ? fminf(fmaxf(z, -clamp), clamp) : z;
-}
-__device__ __forceinline__ float act_bwd(float g, float saved, float gain, float slope, float clamp) {
-    g = g * gain * (saved > 0.f ? 1.f : slope);
-    return (clamp >= 0.f && !(fabsf(saved) < clamp)) ? 0.f : g;
 }
 
 // ------------------------------------------------------------------------- weight preparation
@@ -278,7 +275,7 @@ __global__ void mbstd_gfeat_kernel(const bf16* __restrict__ gx4p, const bf16* __
 }
 // g_y[n][e] = gx4p[n][e] + gfeat[m] * (x - mean_g) / (G * 16C * sd);   g_z1 = g_y * act'(y1)
 __global__ void mbstd_bwd_kernel(const bf16* __restrict__ x, const bf16* __restrict__ x_lo, const bf16* __restrict__ gx4p,
-                                 const bf16* __restrict__ gx4p_lo, const float* __restrict__ gfeat, const bf16* __restrict__ y1, int B, int G, int C,
+                                 const bf16* __restrict__ gx4p_lo, const float* __restrict__ gfeat, const bf16* __restrict__ y1, const bf16* __restrict__ y1_lo, int B, int G, int C,
                                  int Cp, float gain, float slope, float clamp, bf16* g_y, bf16* g_y_lo, bf16* g_z1, bf16* g_z1_lo) {
     const int M = B / G, E = 16 * C;
     const long long idx = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x;
@@ -293,11 +290,12 @@ __global__ void mbstd_bwd_kernel(const bf16* __restrict__ x, const bf16* __restr
     const float sd = sqrtf(var / G + 1e-8f);
     const float k = gfeat[m] / (static_cast<float>(G) * E * sd);
     const int hw = e / C, c = e % C;
+    const float thr = act_saved_clamp(clamp, y1_lo != nullptr);
     for (int g = 0; g < G; ++g) {
         const long long n = g * M + m;
         const float gv = ld_sp(gx4p, gx4p_lo, (n * 16 + hw) * Cp + c) + k * (xv[g] - mean);
         st_sp(g_y, g_y_lo, n * E + e, gv);
-        st_sp(g_z1, g_z1_lo, n * E + e, act_bwd(gv, __bfloat162float(y1[n * E + e]), gain, slope, clamp));
+        st_sp(g_z1, g_z1_lo, n * E + e, act_grad(gv * gain, ld_sp(y1, y1_lo, n * E + e), slope, thr));
     }
 }
 
@@ -336,7 +334,7 @@ __global__ void out_bwd_kernel(const float* __restrict__ gl, const float* __rest
     const long long idx = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x;
     if (idx >= static_cast<long long>(B) * C) return;
     const int c = static_cast<int>(idx % C), n = static_cast<int>(idx / C);
-    st_sp(gz6, gz6_lo, idx, act_bwd(gl[n] * w[c] * wg, __bfloat162float(x6[idx]), gain, slope, -1.f));
+    st_sp(gz6, gz6_lo, idx, act_grad(gl[n] * w[c] * wg * gain, __bfloat162float(x6[idx]), slope, act_saved_clamp(-1.f, false)));
 }
 
 struct Bump {
@@ -530,7 +528,7 @@ int build_disc(la_disc* D) {
                     if (fabsf(U.fy[i / 4] * U.fx[i % 4] - U.fk[i]) > 1e-6f * fabsf(U.fk[bi])) U.separable = 0;
             }
             U.gy_hi = k.x0.hi; U.gy_lo = k.x0.lo; U.gt_hi = D->yb.hi; U.gt_lo = D->yb.lo;      // "backward" FIR direction = the blur
-            U.t_hi = D->g_yb.hi; U.t_lo = D->g_yb.lo; U.x_hi = D->g_z0.hi; U.x_lo = D->g_z0.lo; U.act_saved = k.x0.hi;
+            U.t_hi = D->g_yb.hi; U.t_lo = D->g_yb.lo; U.x_hi = D->g_z0.hi; U.x_lo = D->g_z0.lo; U.act_saved = k.x0.hi; U.act_saved_lo = k.x0.lo;
             U.act_gain = kSqrt2; U.act_clamp = clamp; U.act_slope = 0.2f;
             if (!split && U.separable && R >= 32 && !getenv("LA_NO_FIR_TMA")) {
                 const uint64_t Cc = C, Rr = R;
@@ -639,11 +637,11 @@ int build_disc(la_disc* D) {
             P.lin_add_down = D->g_ys.hi; P.lin_add_down_lo = D->g_ys.lo;      // FIRdown^T(g_ys) is evaluated inside the epilogue
             for (int i = 0; i < 16; ++i) P.lin_fir[i] = D->fir[i];
             if (b == 0) {                     // the producer is fromrgb (lrelu*sqrt2, clamp): its backward is fused (atomics into g_img)
-                P.lin_saved = k.x_in.hi; P.lin_rgb_w = D->rgb_w4;       // lin_rgb_g is set per call
+                P.lin_saved = k.x_in.hi; P.lin_saved_lo = k.x_in.lo; P.lin_rgb_w = D->rgb_w4;       // lin_rgb_g is set per call
                 P.act_gain = kSqrt2; P.act_clamp = clamp;
             } else {                          // the producer is conv1 of the block above (gain sqrt2*sqrt(.5), clamp*sqrt(.5))
                 Block& up = D->blk[b - 1];
-                P.lin_out = up.g_y.hi; P.lin_out_lo = up.g_y.lo; P.lin_saved = up.y1.hi; P.lin_gz = up.g_z1.hi; P.lin_gz_lo = up.g_z1.lo;
+                P.lin_out = up.g_y.hi; P.lin_out_lo = up.g_y.lo; P.lin_saved = up.y1.hi; P.lin_saved_lo = up.y1.lo; P.lin_gz = up.g_z1.hi; P.lin_gz_lo = up.g_z1.lo;
                 P.act_gain = kSqrt2 * kSqrtHalf; P.act_clamp = clamp >= 0.f ? clamp * kSqrtHalf : clamp;
             }
             P.err_flag = D->err_flag;
@@ -695,7 +693,7 @@ int build_disc(la_disc* D) {
         DLA(make_b_map(P, D->wfb, C4, 16 * C4, wm, bn));
         P.kchunks = C4 / 64;
         lin_epi(P, D, 16 * C4, bn, 1, 1);
-        P.lin_saved = D->x5.hi; P.lin_gz = D->gz5.hi; P.lin_gz_lo = D->gz5.lo;
+        P.lin_saved = D->x5.hi; P.lin_saved_lo = D->x5.lo; P.lin_gz = D->gz5.hi; P.lin_gz_lo = D->gz5.lo;
         P.act_gain = kSqrt2; P.act_clamp = d.conv_clamp;
         P.err_flag = D->err_flag;
         DLA(one_tap(D, P));
@@ -865,7 +863,7 @@ int disc_backward(la_disc* D, float w_disc, float4* g_img, int accumulate, float
     DLA(gemm(D, D->BE, s, launches));
     mbstd_gfeat_kernel<<<M, 128, 0, s>>>(D->gx4p.hi, D->gx4p.lo, B, M, C4, Cp, D->gfeat);
     mbstd_bwd_kernel<<<cdiv(static_cast<long long>(M) * 16 * C4, 256), 256, 0, s>>>(
-        last.y.hi, last.y.lo, D->gx4p.hi, D->gx4p.lo, D->gfeat, last.y1.hi, B, G, C4, Cp, kSqrt2 * kSqrtHalf, 0.2f,
+        last.y.hi, last.y.lo, D->gx4p.hi, D->gx4p.lo, D->gfeat, last.y1.hi, last.y1.lo, B, G, C4, Cp, kSqrt2 * kSqrtHalf, 0.2f,
         d.conv_clamp >= 0.f ? d.conv_clamp * kSqrtHalf : d.conv_clamp, last.g_y.hi, last.g_y.lo, last.g_z1.hi, last.g_z1.lo);
     DCU(cudaGetLastError());
     if (launches) *launches += 4;

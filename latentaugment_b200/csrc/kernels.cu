@@ -3,6 +3,7 @@
 
 #include <cuda_bf16.h>
 
+#include "act.cuh"
 #include "sm100.cuh"
 
 namespace la {
@@ -356,11 +357,11 @@ __global__ void __launch_bounds__(256, SEP ? 3 : 2) upfir_slide_kernel(const __g
             const long long o = obase + static_cast<long long>(x) * hc;
             if (FWD && P.act_saved) {
                 const unsigned sv = __ldg(reinterpret_cast<const unsigned*>(P.act_saved) + o);
-                const float s0 = __uint_as_float(sv << 16), s1 = __uint_as_float(sv & 0xffff0000u);
-                const float cl = P.act_clamp >= 0.f ? P.act_clamp : __int_as_float(0x7f800000);
-                float g0 = a0 * P.act_gain * (s0 > 0.f ? 1.f : P.act_slope), g1 = a1 * P.act_gain * (s1 > 0.f ? 1.f : P.act_slope);
-                g0 = fabsf(s0) < cl ? g0 : 0.f;
-                g1 = fabsf(s1) < cl ? g1 : 0.f;
+                const unsigned svl = P.act_saved_lo ? __ldg(reinterpret_cast<const unsigned*>(P.act_saved_lo) + o) : 0u;
+                const float s0 = __uint_as_float(sv << 16) + __uint_as_float(svl << 16);
+                const float s1 = __uint_as_float(sv & 0xffff0000u) + __uint_as_float(svl & 0xffff0000u);
+                const float thr = act_saved_clamp(P.act_clamp, P.act_saved_lo != nullptr);
+                const float g0 = act_grad(a0 * P.act_gain, s0, P.act_slope, thr), g1 = act_grad(a1 * P.act_gain, s1, P.act_slope, thr);
                 st_bf16x2(oh, ol, o, g0, g1);
             } else if (FWD) {
                 float z0 = fmaf(a0, dm.x, nzv[u]) + bs.x, z1 = fmaf(a1, dm.y, nzv[u]) + bs.y;
@@ -435,6 +436,7 @@ __global__ void __launch_bounds__(160) upfir_tma_kernel(const __grid_constant__ 
         if (P.s_next) sn = __ldg(reinterpret_cast<const float2*>(P.s_next + static_cast<long long>(n) * P.C + c));
     }
     const float clampv = P.act_clamp >= 0.f ? P.act_clamp : __int_as_float(0x7f800000);
+    const float saved_thr = act_saved_clamp(P.act_clamp, false);         // act_saved: hi plane only (bf16 mode)
     const int px0 = warp * 8;                                    // this warp's first output pixel inside the strip
     uint8_t* my_stage = stage + warp * 4096;
     if constexpr (!FWD) {
@@ -495,9 +497,8 @@ __global__ void __launch_bounds__(160) upfir_tma_kernel(const __grid_constant__ 
                 const float a1 = fmaf(wy[3], h3[i].y, fmaf(wy[2], h2[i].y, fmaf(wy[1], h1[i].y, wy[0] * h0[i].y)));
                 if (FWD && P.act_saved) {
                     const float s0 = __uint_as_float(svv[i] << 16), s1 = __uint_as_float(svv[i] & 0xffff0000u);
-                    float g0 = a0 * P.act_gain * (s0 > 0.f ? 1.f : P.act_slope), g1 = a1 * P.act_gain * (s1 > 0.f ? 1.f : P.act_slope);
-                    g0 = fabsf(s0) < clampv ? g0 : 0.f;
-                    g1 = fabsf(s1) < clampv ? g1 : 0.f;
+                    const float g0 = act_grad(a0 * P.act_gain, s0, P.act_slope, saved_thr);
+                    const float g1 = act_grad(a1 * P.act_gain, s1, P.act_slope, saved_thr);
                     reinterpret_cast<unsigned*>(sx)[i * 32 + lane] = pack2(g0, g1);
                 } else if (FWD) {
                     float z0 = fmaf(a0, dm.x, nzv[i]) + bs.x, z1 = fmaf(a1, dm.y, nzv[i]) + bs.y;
@@ -585,9 +586,8 @@ __global__ void __launch_bounds__(160) upfir_tma_kernel(const __grid_constant__ 
                 for (int k = 0; k < 4; ++k) { a0 = fmaf(wx[k], cs[i + k].x, a0); a1 = fmaf(wx[k], cs[i + k].y, a1); }
                 if (FWD && P.act_saved) {
                     const float s0 = __uint_as_float(svv[i] << 16), s1 = __uint_as_float(svv[i] & 0xffff0000u);
-                    float g0 = a0 * P.act_gain * (s0 > 0.f ? 1.f : P.act_slope), g1 = a1 * P.act_gain * (s1 > 0.f ? 1.f : P.act_slope);
-                    g0 = fabsf(s0) < clampv ? g0 : 0.f;
-                    g1 = fabsf(s1) < clampv ? g1 : 0.f;
+                    const float g0 = act_grad(a0 * P.act_gain, s0, P.act_slope, saved_thr);
+                    const float g1 = act_grad(a1 * P.act_gain, s1, P.act_slope, saved_thr);
                     reinterpret_cast<unsigned*>(sx)[i * 32 + lane] = pack2(g0, g1);
                 } else if (FWD) {
                     float z0 = fmaf(a0, dm.x, nzv[i]) + bs.x, z1 = fmaf(a1, dm.y, nzv[i]) + bs.y;

@@ -54,8 +54,9 @@ struct UpFirParams {
     void* x_hi; void* x_lo; void* xs_hi; void* xs_lo;
     float act_gain, act_clamp, act_slope;
     // forward, activation-backward variant (discriminator: gradient through blur + lrelu): when act_saved is set the
-    // epilogue is  y = FIR(T) * act_gain * (saved > 0 ? 1 : act_slope) * (|saved| < act_clamp)  -> x_hi
+    // epilogue is  y = FIR(T) * act_gain * (saved > 0 ? 1 : act_slope), 0 where saved is clamped (act.cuh)  -> x_hi
     const void* act_saved;                   // bf16 [B, OH, OW, C] saved activation output, or null
+    const void* act_saved_lo;                // its residual plane (split mode, sliding-window kernel), or null
     // backward: g_y [B, OH, OW, C] -> g_T
     const void* gy_hi; const void* gy_lo;
     void* gt_hi; void* gt_lo;

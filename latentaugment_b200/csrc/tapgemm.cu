@@ -7,6 +7,7 @@
 
 #include <type_traits>
 
+#include "act.cuh"
 #include "sm100.cuh"
 
 namespace la {
@@ -305,6 +306,7 @@ __device__ __forceinline__ void rowowner_warp_tile(const TapGemmParams& P, const
     float rgb0 = 0.f, rgb1 = 0.f, rgb2 = 0.f;
     const bool tk_valid = rc.valid && rc.pix < P.n_queries;
     const float clampv = P.act_clamp >= 0.f ? P.act_clamp : __int_as_float(0x7f800000);
+    const float saved_thr = act_saved_clamp(P.act_clamp, P.split && P.lin_saved_lo);
     // staged stores: the lane re-reads 16-byte piece (lane & 3) of rows 8j + (lane >> 2), j = 0..3, so that
     // every store instruction writes whole 64-byte row segments (row-owner stores write 32 scattered pieces)
     long long srow[4];
@@ -390,11 +392,19 @@ __device__ __forceinline__ void rowowner_warp_tile(const TapGemmParams& P, const
                 if (P.lin_out) store_bf16x32(P.lin_out, P.split ? P.lin_out_lo : nullptr, eoff, acc);
                 if (P.lin_gz || P.lin_rgb_w) {
                     load_bf16x32(P.lin_saved, eoff, t);
+                    if (P.split && P.lin_saved_lo) {      // hi + lo, eight values at a time (no second 32-register row)
+                        const uint4* s = reinterpret_cast<const uint4*>(reinterpret_cast<const __nv_bfloat16*>(P.lin_saved_lo) + eoff);
 #pragma unroll
-                    for (int j = 0; j < 32; ++j) {
-                        const float g = acc[j] * P.act_gain * (t[j] > 0.f ? 1.f : P.act_slope);
-                        acc[j] = fabsf(t[j]) < clampv ? g : 0.f;
+                        for (int q = 0; q < 4; ++q) {
+                            const uint4 a = __ldg(s + q);
+                            t[8 * q + 0] += bf16lo_f(a.x); t[8 * q + 1] += bf16hi_f(a.x);
+                            t[8 * q + 2] += bf16lo_f(a.y); t[8 * q + 3] += bf16hi_f(a.y);
+                            t[8 * q + 4] += bf16lo_f(a.z); t[8 * q + 5] += bf16hi_f(a.z);
+                            t[8 * q + 6] += bf16lo_f(a.w); t[8 * q + 7] += bf16hi_f(a.w);
+                        }
                     }
+#pragma unroll
+                    for (int j = 0; j < 32; ++j) acc[j] = act_grad(acc[j] * P.act_gain, t[j], P.act_slope, saved_thr);
                     if (P.lin_gz) store_bf16x32(P.lin_gz, P.split ? P.lin_gz_lo : nullptr, eoff, acc);
                     if (P.lin_rgb_w) {
                         const float4* w4 = reinterpret_cast<const float4*>(P.lin_rgb_w) + col0;
@@ -627,7 +637,7 @@ __device__ __forceinline__ void bwd_warp_tile(const TapGemmParams& P, const BwdT
     if (n_ok && nsteps > st.nsteps) st.nsteps = nsteps;
 
     const float inv_gain = 1.f / P.act_gain, inv_gain_slope = 1.f / (P.act_gain * P.act_slope);
-    const float clampv = P.act_clamp >= 0.f ? P.act_clamp : __int_as_float(0x7f800000);
+    const float saved_thr = act_saved_clamp(P.act_clamp, kSplit);
     const bool last = P.bwd_last != 0;        // x_{l-1} is the constant input: only red_s is wanted (coefficients stay 0, no store)
     const unsigned* soff = ws->off[buf] + half * 16;
     const float* snz = ws->nz[buf] + half * 16;
@@ -686,10 +696,7 @@ __device__ __forceinline__ void bwd_warp_tile(const TapGemmParams& P, const BwdT
             const float nz = snz[i];
             // activation backward of layer l-1 decided by its saved output; y recovered from it
             const bool p0 = x0 > 0.f, p1 = x1 > 0.f;
-            float gz0 = g0 * (p0 ? 1.f : P.act_slope);
-            float gz1 = g1 * (p1 ? 1.f : P.act_slope);
-            gz0 = fabsf(x0) < clampv ? gz0 : 0.f;
-            gz1 = fabsf(x1) < clampv ? gz1 : 0.f;
+            const float gz0 = act_grad(g0, x0, P.act_slope, saved_thr), gz1 = act_grad(g1, x1, P.act_slope, saved_thr);
             const float z0 = x0 * (p0 ? inv_gain : inv_gain_slope), z1 = x1 * (p1 ? inv_gain : inv_gain_slope);
             r[2] = fmaf(gz0, z0 - (nz + bs.x), r[2]);
             r[3] = fmaf(gz1, z1 - (nz + bs.y), r[3]);
@@ -1325,7 +1332,7 @@ __global__ void __launch_bounds__(256) seed_stream_kernel(const __grid_constant_
     rw0.x *= P.act_gain; rw0.y *= P.act_gain; rw0.z *= P.act_gain;
     rw1.x *= P.act_gain; rw1.y *= P.act_gain; rw1.z *= P.act_gain;
     const float inv_gain = 1.f / P.act_gain, inv_gain_slope = 1.f / (P.act_gain * P.act_slope);
-    const float clampv = P.act_clamp >= 0.f ? P.act_clamp : __int_as_float(0x7f800000);
+    const float saved_thr = act_saved_clamp(P.act_clamp, P.split);       // split: hi + lo read below
     const long long base = static_cast<long long>(n) * img_px;
     const unsigned* xh = reinterpret_cast<const unsigned*>(P.xp_hi) + base * half_n + (col >> 1);
     const unsigned* xl = P.split ? reinterpret_cast<const unsigned*>(P.xp_lo) + base * half_n + (col >> 1) : nullptr;
@@ -1362,9 +1369,7 @@ __global__ void __launch_bounds__(256) seed_stream_kernel(const __grid_constant_
             r[4] = fmaf(x0, g[u].y, r[4]); r[5] = fmaf(x1, g[u].y, r[5]);
             r[6] = fmaf(x0, g[u].z, r[6]); r[7] = fmaf(x1, g[u].z, r[7]);
             const bool q0 = x0 > 0.f, q1 = x1 > 0.f;
-            float gz0 = g0 * (q0 ? 1.f : P.act_slope), gz1 = g1 * (q1 ? 1.f : P.act_slope);
-            gz0 = fabsf(x0) < clampv ? gz0 : 0.f;
-            gz1 = fabsf(x1) < clampv ? gz1 : 0.f;
+            const float gz0 = act_grad(g0, x0, P.act_slope, saved_thr), gz1 = act_grad(g1, x1, P.act_slope, saved_thr);
             const float z0 = x0 * (q0 ? inv_gain : inv_gain_slope), z1 = x1 * (q1 ? inv_gain : inv_gain_slope);
             r[0] = fmaf(gz0, z0 - nz[u] - bs.x, r[0]);
             r[1] = fmaf(gz1, z1 - nz[u] - bs.y, r[1]);
@@ -1438,7 +1443,7 @@ __global__ void __launch_bounds__(128) seed_bulk_kernel(const __grid_constant__ 
     rw0.x *= P.act_gain; rw0.y *= P.act_gain; rw0.z *= P.act_gain;
     rw1.x *= P.act_gain; rw1.y *= P.act_gain; rw1.z *= P.act_gain;
     const float inv_gain = 1.f / P.act_gain, inv_gain_slope = 1.f / (P.act_gain * P.act_slope);
-    const float clampv = P.act_clamp >= 0.f ? P.act_clamp : __int_as_float(0x7f800000);
+    const float saved_thr = act_saved_clamp(P.act_clamp, false);         // hi plane only
     const float nscale = nzp ? P.noise_prev_scale : 0.f;
     float r[8];
 #pragma unroll
@@ -1464,9 +1469,7 @@ __global__ void __launch_bounds__(128) seed_bulk_kernel(const __grid_constant__ 
             r[4] = fmaf(x0, g.y, r[4]); r[5] = fmaf(x1, g.y, r[5]);
             r[6] = fmaf(x0, g.z, r[6]); r[7] = fmaf(x1, g.z, r[7]);
             const bool q0 = x0 > 0.f, q1 = x1 > 0.f;
-            float gz0 = g0 * (q0 ? 1.f : P.act_slope), gz1 = g1 * (q1 ? 1.f : P.act_slope);
-            gz0 = fabsf(x0) < clampv ? gz0 : 0.f;
-            gz1 = fabsf(x1) < clampv ? gz1 : 0.f;
+            const float gz0 = act_grad(g0, x0, P.act_slope, saved_thr), gz1 = act_grad(g1, x1, P.act_slope, saved_thr);
             const float z0 = x0 * (q0 ? inv_gain : inv_gain_slope), z1 = x1 * (q1 ? inv_gain : inv_gain_slope);
             r[0] = fmaf(gz0, z0 - nz - bs.x, r[0]);
             r[1] = fmaf(gz1, z1 - nz - bs.y, r[1]);

@@ -130,8 +130,9 @@ struct TapGemmParams {
     float lin_fir[16];                 // flipped 4x4 filter of lin_add_down
     void* lin_out;                     // bf16 r or null
     const void* lin_saved;             // bf16 saved activation output deciding the activation gradient, or null
-    void* lin_gz;                      // bf16 r * act_gain * (saved > 0 ? 1 : act_slope) * (|saved| < act_clamp), or null
+    void* lin_gz;                      // bf16 r * act_gain * (saved > 0 ? 1 : act_slope), 0 where saved is clamped (act.cuh), or null
     const void* lin_add_lo; const void* lin_add_down_lo; void* lin_out_lo; void* lin_gz_lo;   // residual planes when split
+    const void* lin_saved_lo;          // residual plane of lin_saved (split), or null: the clamp decision reads hi + lo
     const float* lin_rgb_w;            // [N][4] or null: fused 1x1 "fromrgb" backward -- the activation-gradient row (the lin_gz
     float4* lin_rgb_g;                 // value) is contracted with these weights and atomically added to lin_rgb_g[pixel].xyz
 

@@ -36,11 +36,12 @@ def _randn(shape, seed):
     return torch.randn(shape, generator=torch.Generator().manual_seed(seed))
 
 
-def make_workload(cfg, noise_strength=0.0, batch=None, with_img_bank=True):
-    """Returns dict(G, W [M,num_ws,w_dim], w0 [B,1,w_dim], X [Mi,C,res,res] or None)."""
+def make_workload(cfg, noise_strength=0.0, batch=None, with_img_bank=True, conv_clamp=256.0):
+    """Returns dict(G, W [M,num_ws,w_dim], w0 [B,1,w_dim], X [Mi,C,res,res] or None).  ``conv_clamp`` changes no drawn
+    tensor."""
     c = dict(CONFIGS[cfg]) if isinstance(cfg, str) else dict(cfg)
     B = batch if batch is not None else c['batch']
-    G = sg2.make_generator(seed=0, noise_strength=noise_strength, **generator_kwargs(c))
+    G = sg2.make_generator(seed=0, noise_strength=noise_strength, conv_clamp=conv_clamp, **generator_kwargs(c))
     with torch.no_grad():
         W = G.mapping(_randn([c['bank'], G.z_dim], 1), None)[:, :1].repeat(1, G.num_ws, 1).contiguous()
         w0 = G.mapping(_randn([B, G.z_dim], 2), None)[:, :1].contiguous()

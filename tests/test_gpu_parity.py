@@ -18,24 +18,31 @@ pytestmark = pytest.mark.gpu
 TOL = {'fp32_parity': 1e-3, 'bf16': 1e-2}
 
 
-def _engine(wl, precision, batch=None):
+def _engine(wl, precision, batch=None, conv_clamp=256.0):
     from latentaugment_b200.engine import SynthesisEngine
     G = wl['G']
     return SynthesisEngine(dict(G.state_dict()), img_resolution=G.img_resolution, img_channels=G.img_channels,
-                           w_dim=G.w_dim, z_dim=G.z_dim, batch=batch or wl['w0'].shape[0], precision=precision)
+                           w_dim=G.w_dim, z_dim=G.z_dim, conv_clamp=conv_clamp, batch=batch or wl['w0'].shape[0], precision=precision)
 
 
-def _workload(cfg, noise_strength=0.1):
+def _workload(cfg, noise_strength=0.1, conv_clamp=256.0):
     from oracle import synthetic
-    return synthetic.make_workload(cfg, noise_strength=noise_strength)
+    return synthetic.make_workload(cfg, noise_strength=noise_strength, conv_clamp=conv_clamp)
 
 
-@pytest.mark.parametrize('cfg', ['tiny', 'tiny128', 'small'])
+def with_clamps(cases, clamps=(None, 1.0, 0.7)):
+    """Parameters (case, conv_clamp): every case at the networks' default 256 under its plain id, then the clamp off (None)
+    and engaged (1.0 is bf16-exact, 0.7 is not; tests/test_gpu_act_clamp.py) -- ids ``<case>-clamp<value>``."""
+    out = [pytest.param(c, 256.0, id=str(c)) for c in cases]
+    return out + [pytest.param(c, v, id=f'{c}-clamp{v}') for v in clamps for c in cases]
+
+
+@pytest.mark.parametrize('cfg,conv_clamp', with_clamps(['tiny', 'tiny128', 'small'])[:3] + with_clamps(['tiny'])[1:])
 @pytest.mark.parametrize('precision', ['fp32_parity', 'bf16'])
-def test_synthesis_matches_oracle(cfg, precision):
-    wl = _workload(cfg)
+def test_synthesis_matches_oracle(cfg, precision, conv_clamp):
+    wl = _workload(cfg, conv_clamp=conv_clamp)
     G = wl['G']
-    eng = _engine(wl, precision)
+    eng = _engine(wl, precision, conv_clamp=conv_clamp)
     ws = wl['w0'].repeat(1, G.num_ws, 1)
     with torch.no_grad():
         ref_const = G.synthesis(ws, noise_mode='const')
@@ -44,7 +51,7 @@ def test_synthesis_matches_oracle(cfg, precision):
     out_none = eng.synthesis(ws, noise_mode='none').cpu()
     eng.debug_check()
     e1, e2 = rel_l2(out_const, ref_const), rel_l2(out_none, ref_none)
-    print(f'\n[synthesis {cfg} {precision}] rel_l2 const={e1:.3e} none={e2:.3e}')
+    print(f'\n[synthesis {cfg} {precision} conv_clamp={conv_clamp}] rel_l2 const={e1:.3e} none={e2:.3e}')
     tol = 1e-4 if precision == 'fp32_parity' else 1e-2
     assert e1 < tol and e2 < tol
     # distinct ws rows per layer (general G.synthesis(ws) call)
@@ -241,16 +248,16 @@ def test_plugin_api_end_to_end():
 
 
 @pytest.mark.parametrize('split_min_res', ['8', '100000'])
-@pytest.mark.parametrize('precision', ['fp32_parity', 'bf16'])
-def test_both_upconv_formulations(monkeypatch, split_min_res, precision):
+@pytest.mark.parametrize('precision,conv_clamp', with_clamps(['fp32_parity', 'bf16']))
+def test_both_upconv_formulations(monkeypatch, split_min_res, precision, conv_clamp):
     """x2 layers as transposed-conv GEMM + FIR pass (split) and with the FIR folded into 36 taps: both
     must match the oracle, at every resolution (LA_UPCONV_SPLIT_MIN_RES picks per layer)."""
     from oracle import latent_aug as ola
     monkeypatch.setenv('LA_UPCONV_SPLIT_MIN_RES', split_min_res)
     for cfg in ('tiny', 'small'):
-        wl = _workload(cfg)
+        wl = _workload(cfg, conv_clamp=conv_clamp)
         G = wl['G']
-        eng = _engine(wl, precision)
+        eng = _engine(wl, precision, conv_clamp=conv_clamp)
         eng.set_latent_bank(wl['W'])
         eng.set_image_bank(wl['X'])
         ws = wl['w0'].repeat(1, G.num_ws, 1)
@@ -265,7 +272,7 @@ def test_both_upconv_formulations(monkeypatch, split_min_res, precision):
         img, w_aug = eng.augment(wl['w0'], num_steps=2, final_noise_mode='const')
         eng.debug_check()
         ew, ei = rel_l2(w_aug.cpu(), w_ref[:, 0]), rel_l2(img.cpu(), img_ref)
-        print(f'\n[upconv split_min_res={split_min_res} {cfg} {precision}] synth={e0:.3e} rel_w={ew:.3e} rel_img={ei:.3e}')
+        print(f'\n[upconv split_min_res={split_min_res} {cfg} {precision} conv_clamp={conv_clamp}] synth={e0:.3e} rel_w={ew:.3e} rel_img={ei:.3e}')
         assert e0 < (1e-4 if precision == 'fp32_parity' else 1e-2)
         assert ew < TOL[precision] and ei < TOL[precision]
         # tensor-core path against the SIMT twin on this formulation
@@ -301,13 +308,22 @@ def test_ragged_batches(batch, precision):
 
 def test_single_channel_wide_generator():
     """1-channel images and 256-wide layers at 64^2 (BN = 256 path, TMA FIR passes, bulk seed kernel) against the oracle."""
+    _single_channel_wide(256.0)
+
+
+@pytest.mark.parametrize('conv_clamp', [None, 1.0, 0.7])
+def test_single_channel_wide_generator_clamped(conv_clamp):
+    _single_channel_wide(conv_clamp)
+
+
+def _single_channel_wide(conv_clamp):
     from oracle import latent_aug as ola
     from oracle import synthetic
     cfg = dict(img_resolution=64, img_channels=1, channel_base=16384, channel_max=256, batch=4, steps=2, bank=32, img_bank=4)
-    wl = synthetic.make_workload(cfg, noise_strength=0.1)
+    wl = synthetic.make_workload(cfg, noise_strength=0.1, conv_clamp=conv_clamp)
     G = wl['G']
     for precision in ('fp32_parity', 'bf16'):
-        eng = _engine(wl, precision)
+        eng = _engine(wl, precision, conv_clamp=conv_clamp)
         eng.set_latent_bank(wl['W'])
         eng.set_image_bank(wl['X'])
         orc = ola.LatentAugOracle(G, wl['W'], wl['X'], num_epochs=2, fused=True)
@@ -318,7 +334,7 @@ def test_single_channel_wide_generator():
         img, w_aug = eng.augment(wl['w0'], num_steps=2, final_noise_mode='const')
         eng.debug_check()
         ew, ei = rel_l2(w_aug.cpu(), w_ref[:, 0]), rel_l2(img.cpu(), img_ref)
-        print(f'\n[1-ch wide {precision}] rel_w={ew:.3e} rel_img={ei:.3e}')
+        print(f'\n[1-ch wide {precision} conv_clamp={conv_clamp}] rel_w={ew:.3e} rel_img={ei:.3e}')
         assert ew < TOL[precision] and ei < TOL[precision]
 
 
@@ -433,17 +449,17 @@ def test_micro_batches_and_lookahead_loop_match_plain_calls():
         assert rel_l2(img, r) < 1e-5
 
 
-@pytest.mark.parametrize('precision', ['fp32_parity', 'bf16'])
-def test_bn128_layers_match_oracle(precision):
+@pytest.mark.parametrize('precision,conv_clamp', with_clamps(['fp32_parity', 'bf16']))
+def test_bn128_layers_match_oracle(precision, conv_clamp):
     """128-channel layers on a grid with more than 74 M tiles select the BN = 128 kernels (two M tiles per unit sharing each
     weight tile; CTA-pair four-tile work items in the forward conv) -- the variant the 256x256 layers of config C2 run.
     64x64 with batch 4 reaches it at a size the oracle finishes in seconds."""
     from oracle import latent_aug as ola
     from oracle import synthetic
     cfg = dict(img_resolution=64, img_channels=3, channel_base=8192, channel_max=128, batch=4, steps=3, bank=32, img_bank=4)
-    wl = synthetic.make_workload(cfg, noise_strength=0.1)
+    wl = synthetic.make_workload(cfg, noise_strength=0.1, conv_clamp=conv_clamp)
     G = wl['G']
-    eng = _engine(wl, precision)
+    eng = _engine(wl, precision, conv_clamp=conv_clamp)
     eng.set_latent_bank(wl['W'])
     eng.set_image_bank(wl['X'])
     orc = ola.LatentAugOracle(G, wl['W'], wl['X'], num_epochs=3, fused=True)
@@ -455,5 +471,5 @@ def test_bn128_layers_match_oracle(precision):
     eng.debug_check()
     d = (w_aug.cpu() - w_ref[:, 0]).abs()
     ew, ei = rel_l2(w_aug.cpu(), w_ref[:, 0]), rel_l2(img.cpu(), img_ref)
-    print(f'\n[BN=128 layers {precision}] rel_w={ew:.3e} rel_img={ei:.3e} components off by > lr: {int((d > 0.01).sum())}/{d.numel()}')
+    print(f'\n[BN=128 layers {precision} conv_clamp={conv_clamp}] rel_w={ew:.3e} rel_img={ei:.3e} components off by > lr: {int((d > 0.01).sum())}/{d.numel()}')
     assert ew < TOL[precision] and ei < TOL[precision]

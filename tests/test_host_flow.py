@@ -280,3 +280,47 @@ def test_constructor_loads_the_reference_network_pickle_tree(fake_engine, tmp_pa
     os.makedirs(run.parent / '00003-duplicate')
     with pytest.raises(AssertionError):
         create_augment(opt)
+
+
+@pytest.mark.parametrize('with_kwargs', [True, False])
+def test_network_pickle_constructor_arguments_reach_the_engine(fake_engine, tmp_path, monkeypatch, with_kwargs):
+    """The pickled modules' own ``init_kwargs`` (``torch_utils/persistence.py``) decide the clamp and the minibatch-stddev
+    group, as they do when the reference runs the unpickled modules: a ``--cfg stylegan2`` G (``conv_clamp=None``) and a
+    ``paper256`` D (``mbstd_group_size=8``, ``conv_clamp=256``).  Modules without ``init_kwargs`` keep the defaults."""
+    import pickle
+
+    from latentaugment_b200.augments import create_augment
+    from latentaugment_b200.options.aug_options import AugOptions
+    from oracle import sg2, sg2_disc
+    cfg = dict(img_resolution=16, img_channels=2, channel_base=512, channel_max=32)
+    G = sg2.Generator(**cfg).eval()
+    D = sg2_disc.make_discriminator(**cfg)
+    if with_kwargs:
+        G.init_kwargs = dict(z_dim=512, c_dim=0, w_dim=512, img_resolution=16, img_channels=2, mapping_kwargs={},
+                             synthesis_kwargs=dict(channel_base=512, channel_max=32, num_fp16_res=0, conv_clamp=None))
+        D.init_kwargs = dict(c_dim=0, img_resolution=16, img_channels=2, channel_base=512, channel_max=32, num_fp16_res=0,
+                             conv_clamp=256, block_kwargs={}, mapping_kwargs={}, epilogue_kwargs=dict(mbstd_group_size=8))
+    run = tmp_path / 'models' / 'DS' / 'training-runs' / 'DSname' / 'm0,m1' / '00003-stylegan2-DS-gpus2'
+    os.makedirs(run)
+    with open(run / 'network-snapshot-005320.pkl', 'wb') as f:
+        pickle.dump({'G_ema': G, 'D': D}, f)
+    seen = {}
+    monkeypatch.setattr(fake_engine, 'set_discriminator', lambda self, state, **kw: seen.__setitem__('D', kw))
+    real_init = fake_engine.__init__
+
+    def init(self, state, **kw):
+        seen['G'] = kw
+        real_init(self, state, **kw)
+    monkeypatch.setattr(fake_engine, '__init__', init)
+    argv = ['--aug', 'latent', '--batch_size', '8', '--no_log', '--model_dir', str(tmp_path / 'models'), '--dataset_aug', 'DS',
+            '--dataset_name_aug', 'DSname', '--modalities_aug', 'm0,m1', '--img_resolution', '16', '--checkpoints_dir', str(tmp_path),
+            '--synthetic', '--synthetic_bank', '8', '--synthetic_img_bank', '3', '--synthetic_codes', '8',
+            '--synthetic_channel_base', '512', '--synthetic_channel_max', '32']
+    opt = AugOptions().parse(args={'p_thres': 0.0, 'init_w': 'inv', 'w_lpips': 0.0, 'w_disc': 1.0}, argv=argv)
+    create_augment(opt)
+    if with_kwargs:
+        assert 'conv_clamp' in seen['G'] and seen['G']['conv_clamp'] is None
+        assert seen['D'] == dict(conv_clamp=256, mbstd_group_size=8)
+    else:
+        assert seen['G']['conv_clamp'] == 256.0
+        assert seen['D'] == dict(conv_clamp=256.0, mbstd_group_size=4)
