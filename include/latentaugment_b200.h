@@ -21,6 +21,8 @@
  *                            realism term calc_loss_disc: softplus(-D(x, c=None)).mean() * w_disc   util_latent_aug.py:363-371
  *   la_pairwise_sqdist    <- l2_loss_vectorized(X, Y, compute_mean=False)         util_latent_aug.py:315-361
  *   la_nearest_codes      <- (north_star extension, SURVEY.md F3) argmin / top-k of that matrix
+ *   la_project            <- StyleGAN2-ADA projector.py::project, batched, producing the inverted codes of --init_w inv
+ *                            (DESIGN.md "Projection")
  */
 #ifndef LATENTAUGMENT_B200_H
 #define LATENTAUGMENT_B200_H
@@ -37,7 +39,7 @@ extern "C" {
 #define LA_MAX_MAPPING 8
 #define LA_MAX_STEPS 64            /* steps whose loss values are logged (the loop itself is not capped) */
 #define LA_LOSS_COLS 5             /* loss-log row: latent, pixel, total, discriminator, perceptual */
-#define LA_ABI_VERSION 201
+#define LA_ABI_VERSION 202
 
 typedef struct la_engine la_engine;
 typedef void* la_stream;          /* cudaStream_t */
@@ -142,6 +144,8 @@ typedef struct la_vgg_desc {
     const float* d_lin_weight[LA_VGG_TAPS];    /* [C_tap] (the 1x1 conv C -> 1 without bias), or null = tap not used */
     float mean[3], std[3];                     /* z-score of the replicated grey crop (networks.py:41-50) */
     int crop_size;                             /* crop_size_aug: 64 (power of two >= 64) */
+    int per_sample_targets;                    /* 1: also plan fp32 per-sample target features for la_set_projection_targets
+                                                  (crop_size must be min(res, 256), res <= 512); 0: bank mode only */
 } la_vgg_desc;
 
 const char* la_last_error(void);
@@ -174,6 +178,9 @@ int la_set_lpips(la_engine* e, const la_vgg_desc* v, void* d_workspace, size_t w
 int la_set_feature_bank(la_engine* e, const float* d_crops, int M, la_stream stream);
 int la_lpips_loss_grad(la_engine* e, const float* d_img, int crop_x, int crop_y, float w_lpips, int norm_mode, float* d_loss,
                        float* d_grad, la_stream stream);
+/* norm_mode 2 (needs la_set_projection_targets): the projection's distance of every sample to its OWN target over the whole
+ * image (crop_x = crop_y = 0; area-pooled 2x2 when res = 2 * crop_size), d_loss [batch] per sample (w_lpips is ignored),
+ * d_grad = d (sum of d_loss) / d img. */
 /* Test hook: normalised activations of used tap k (0-based among the used taps) from the last la_lpips_loss_grad /
  * la_augment step: fp32 [batch * img_channels, h, w, C] (NHWC); *count receives the element count (d_out may be null). */
 int la_lpips_tap(la_engine* e, int k, float* d_out, size_t* count, la_stream stream);
@@ -223,6 +230,18 @@ size_t la_noise_floats(const la_engine* e);
  * (latent, pixel, total, discriminator, perceptual) or NULL.  d_final_noise as in la_synthesis (may be NULL unless final_noise_mode == RANDOM). */
 int la_augment(la_engine* e, const float* d_w0, const la_augment_options* opt, const float* d_final_noise, float* d_img,
                float* d_w_aug, float* d_loss_log, la_stream stream);
+
+/* Projection of real images into W (StyleGAN2-ADA projector.py::project, batched; DESIGN.md "Projection").
+ * la_set_projection_targets: d_img [batch, C, res, res] fp32 in [-1, 1]; needs la_set_lpips with per_sample_targets = 1.
+ * la_project: num_steps Adam steps (betas 0.9 / 0.999, eps 1e-8) from d_w0 [batch, w_dim]; step t synthesises (const noise)
+ * from w_opt + d_sigma[t] * d_wnoise[t] (d_wnoise [num_steps, batch, w_dim] unit normal, or NULL for none), takes the
+ * summed per-sample LPIPS distance to the targets over all used taps, and steps with learning rate d_lr[t].
+ * d_lr, d_sigma: DEVICE arrays [num_steps].  Outputs: d_w_out [batch, w_dim] = w_opt after the last step (no noise);
+ * d_loss_log [num_steps] (or NULL) = the summed loss of every step.  All device arrays must stay alive until the call
+ * has completed on the stream. */
+int la_set_projection_targets(la_engine* e, const float* d_img, la_stream stream);
+int la_project(la_engine* e, const float* d_w0, int num_steps, const float* d_lr, const float* d_sigma, const float* d_wnoise,
+               float* d_w_out, float* d_loss_log, la_stream stream);
 
 /* D[j, i] = |Y_j|^2 + |X_i|^2 - 2 <Y_j, X_i>  ([bank, batch] orientation, fp32, the reference's
  * association order).  X [n, K], Y [m, K]. */

@@ -13,7 +13,7 @@ LA_MAX_MAPPING = 8
 LA_MAX_STEPS = 64
 LA_LOSS_COLS = 5
 LA_VGG_CONVS, LA_VGG_TAPS = 13, 5
-ABI_VERSION = 201          # == LA_ABI_VERSION of include/latentaugment_b200.h
+ABI_VERSION = 202          # == LA_ABI_VERSION of include/latentaugment_b200.h
 PRECISION = {'bf16': 0, 'fp32_parity': 1}
 NOISE = {'none': 0, 'const': 1, 'random': 2}
 
@@ -48,7 +48,7 @@ class AugmentOptions(C.Structure):
 
 class VggDesc(C.Structure):
     _fields_ = [('d_conv_weight', fptr * LA_VGG_CONVS), ('d_conv_bias', fptr * LA_VGG_CONVS), ('d_lin_weight', fptr * LA_VGG_TAPS),
-                ('mean', C.c_float * 3), ('std', C.c_float * 3), ('crop_size', C.c_int)]
+                ('mean', C.c_float * 3), ('std', C.c_float * 3), ('crop_size', C.c_int), ('per_sample_targets', C.c_int)]
 
 
 class DiscBlockParams(C.Structure):
@@ -88,6 +88,8 @@ SIGNATURES = {
     'la_set_feature_bank': (C.c_int, [C.c_void_p, fptr, C.c_int, C.c_void_p]),
     'la_lpips_loss_grad': (C.c_int, [C.c_void_p, fptr, C.c_int, C.c_int, C.c_float, C.c_int, fptr, fptr, C.c_void_p]),
     'la_lpips_tap': (C.c_int, [C.c_void_p, C.c_int, fptr, C.POINTER(C.c_size_t), C.c_void_p]),
+    'la_set_projection_targets': (C.c_int, [C.c_void_p, fptr, C.c_void_p]),
+    'la_project': (C.c_int, [C.c_void_p, fptr, C.c_int, fptr, fptr, fptr, fptr, fptr, C.c_void_p]),
     'la_filtered_lrelu': (C.c_int, [fptr, C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_float), C.c_int, C.POINTER(C.c_float), C.c_int,
                                     fptr, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_float, C.c_float, C.c_float, C.c_int,
                                     C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, fptr, C.c_void_p]),

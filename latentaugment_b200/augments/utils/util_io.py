@@ -11,6 +11,7 @@ import os
 import pickle
 import queue
 import threading
+import zipfile
 
 import numpy as np
 import torch
@@ -120,3 +121,41 @@ def augment_dataset(augment, dataset, outdir, n_iter=None, writer=None, verbose=
         if own_writer:
             writer.close()
     return n
+
+
+def invert_dataset(engine, img_zip, out_zip, *, split, modalities, num_steps=1000, seed=0, verbose=False, **project_kw):
+    """Projects every image of ``img_zip`` (``ImgDataset`` layout: one pickled dict of 0..255 slices per entry; entries of
+    ``split`` -- one name or a list, all written into the one zip --, channels = ``modalities`` in order) into W and writes
+    ``out_zip``: the same entry names, each a pickled
+    float32 ndarray ``[num_ws, w_dim]`` (the code broadcast to every layer) -- the ``{dataset_w_name}.zip`` that
+    ``LatentCodeDataset`` / ``banks_from_reference_layout`` read for ``--init_w inv``.
+
+    ``engine``: a ``SynthesisEngine`` with ``set_lpips(..., per_sample_targets=True)`` done.  Images are mapped to
+    ``x / 127.5 - 1`` and projected ``engine.batch`` at a time (batch i with ``seed + i``); the last batch is padded by
+    repeating its last image and the padded rows are dropped (rows are independent, so padding changes no code).
+    Returns the number of codes written."""
+    from .util_dataset import ImgDataset
+    splits = [split] if isinstance(split, str) else list(split)
+    B = engine.batch
+    os.makedirs(os.path.dirname(os.path.abspath(out_zip)), exist_ok=True)
+    tmp = out_zip + '.partial'
+    total, bi = 0, 0
+    with zipfile.ZipFile(tmp, 'w', zipfile.ZIP_STORED) as zf:
+        for sp in splits:
+            ds = ImgDataset(img_zip, split=sp, modalities=modalities, resolution=engine.img_resolution)
+            names = ds.fnames
+            for i0 in range(0, len(names), B):
+                rows = list(range(i0, min(i0 + B, len(names))))
+                x = np.stack([ds[r][0] for r in rows] + [ds[rows[-1]][0]] * (B - len(rows)))
+                engine.set_projection_targets(torch.from_numpy(x) / 127.5 - 1)
+                w = engine.project(num_steps=num_steps, seed=seed + bi, **project_kw)
+                w = w.detach().float().cpu().numpy()
+                for k, r in enumerate(rows):
+                    code = np.repeat(w[k:k + 1], engine.num_ws, axis=0).astype('float32')
+                    zf.writestr(names[r], pickle.dumps(code, protocol=pickle.HIGHEST_PROTOCOL))
+                bi += 1
+                if verbose:
+                    print(f'{sp}: projected {rows[-1] + 1} / {len(names)}')
+            total += len(names)
+    os.replace(tmp, out_zip)
+    return total

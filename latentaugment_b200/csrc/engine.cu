@@ -112,8 +112,13 @@ struct la_engine {
     la_disc* disc = nullptr;          // realism-term discriminator (optional)
     float* disc_loss = nullptr;
     la_lpips* lp = nullptr;           // perceptual term (optional)
-    float* lpips_loss = nullptr;
+    float* lpips_loss = nullptr;      // [batch]: the total in bank mode, the per-sample distances in projection
     float cur_w_lpips = -1.f;
+    // projection (la_project): perturbed code the style GEMMs read, the device-resident schedule
+    float* w_pert = nullptr;
+    ProjConsts* proj = nullptr;
+    int cur_project = 0;              // the captured step_graph is a projection step (it bakes the criterion launches)
+    bool proj_warmed = false;         // a projection step has run eagerly (its launches differ from the augmentation's)
 };
 
 namespace {
@@ -236,11 +241,13 @@ int plan(la_engine* e, char* ws, size_t* bytes_out) {
     e->step = bp.take<int>(1);
     e->err_flag = bp.take<int>(1);
     e->disc_loss = bp.take<float>(1);
-    e->lpips_loss = bp.take<float>(1);
+    e->lpips_loss = bp.take<float>(B);
+    e->proj = bp.take<ProjConsts>(1);
     e->dbg_clock = bp.take<unsigned long long>(64);
     const size_t wn = static_cast<size_t>(B) * g.w_dim;
     e->w_opt = bp.take<float>(wn); e->m = bp.take<float>(wn); e->v = bp.take<float>(wn);
     e->w0 = bp.take<float>(wn); e->w_aug = bp.take<float>(wn);
+    e->w_pert = bp.take<float>(wn);
     e->loss_log = bp.take<float>(LA_MAX_STEPS * LA_LOSS_COLS);
     const size_t mapn = static_cast<size_t>(B) * (g.w_dim > g.z_dim ? g.w_dim : g.z_dim);
     e->map_a = bp.take<float>(mapn); e->map_b = bp.take<float>(mapn);
@@ -563,25 +570,30 @@ int run_forward(la_engine* e, const float* ws, long long sn, long long si, int n
     return 0;
 }
 
-int run_backward(la_engine* e, const la_augment_options& opt, cudaStream_t s) {
+// project: the perceptual term alone, against the per-sample targets (la_project); opt is not read then
+int run_backward(la_engine* e, const la_augment_options& opt, bool project, cudaStream_t s) {
     const la_generator_desc& g = e->g;
     const int B = e->batch;
     const int L = static_cast<int>(e->conv.size());
     Rgb& top = e->rgb.back();
     int nparts = 0;
-    if (opt.w_pix > 0.f) {
+    if (project) {
+        CU(cudaMemsetAsync(top.g_img, 0, sizeof(float4) * static_cast<size_t>(B) * g.img_resolution * g.img_resolution, s));
+        if (lpips_forward(e->lp, top.img, 1, s, &e->launches) || lpips_backward(e->lp, top.g_img, 1, e->lpips_loss, 1, s, &e->launches))
+            return fail(-7, "lpips: %s", lpips_last_error());
+    } else if (opt.w_pix > 0.f) {
         LA(pix_loss(top.img, e->bank_mean, e->bank_m2, B, g.img_resolution, g.img_channels, e->crop_off, e->crop_size, e->cur_w_pix,
                     top.g_img, e->loss_parts, &nparts, s));
     } else {
         CU(cudaMemsetAsync(top.g_img, 0, sizeof(float4) * static_cast<size_t>(B) * g.img_resolution * g.img_resolution, s));
     }
     e->n_loss_parts = nparts;
-    if (opt.w_disc > 0.f) {          // realism term (util_latent_aug.py:363-371): + w_disc * mean softplus(-D(x))
+    if (!project && opt.w_disc > 0.f) {          // realism term (util_latent_aug.py:363-371): + w_disc * mean softplus(-D(x))
         if (disc_forward(e->disc, top.img, s, &e->launches) || disc_backward(e->disc, opt.w_disc, top.g_img, 1, e->disc_loss, s, &e->launches))
             return fail(-6, "discriminator: %s", disc_last_error());
     }
-    if (opt.w_lpips > 0.f) {         // perceptual term (util_latent_aug.py:387-424): - w_lpips * pair-normalised LPIPS distance to the bank
-        if (lpips_forward(e->lp, top.img, s, &e->launches) || lpips_backward(e->lp, top.g_img, 1, e->lpips_loss, s, &e->launches))
+    if (!project && opt.w_lpips > 0.f) {   // perceptual term (util_latent_aug.py:387-424): - w_lpips * pair-normalised LPIPS distance to the bank
+        if (lpips_forward(e->lp, top.img, 0, s, &e->launches) || lpips_backward(e->lp, top.g_img, 1, e->lpips_loss, 0, s, &e->launches))
             return fail(-7, "lpips: %s", lpips_last_error());
     }
     for (int b = g.num_blocks - 1; b >= 0; --b) {
@@ -608,12 +620,58 @@ int run_step(la_engine* e, const la_augment_options& opt, cudaStream_t s) {
     if (synth) {
         CU(cudaMemsetAsync(e->red_all, 0, e->red_bytes, s));
         LA(run_forward(e, e->w_opt, g.w_dim, 0, LA_NOISE_CONST, nullptr, nullptr, s));
-        LA(run_backward(e, opt, s));
+        LA(run_backward(e, opt, false, s));
     }
     LA(adam_step(e->partial, e->nchunks, synth ? 1 : 0, e->w_sum, e->lat_m2, e->consts, e->step, e->w_opt, e->m, e->v, B, g.w_dim,
                  e->loss_parts, synth ? e->n_loss_parts : 0, e->bank_m2, opt.n_modalities, e->crop_size, e->loss_log, LA_MAX_STEPS,
                  opt.w_disc > 0.f ? e->disc_loss : nullptr, opt.w_lpips > 0.f ? e->lpips_loss : nullptr, s));
     e->launches += 3;
+    return 0;
+}
+
+// one projection step: synthesis from the perturbed code, distance to the targets, scheduled Adam (which also writes the
+// next step's perturbed code)
+int run_project_step(la_engine* e, cudaStream_t s) {
+    const la_generator_desc& g = e->g;
+    la_augment_options unused{};
+    CU(cudaMemsetAsync(e->red_all, 0, e->red_bytes, s));
+    LA(run_forward(e, e->w_pert, g.w_dim, 0, LA_NOISE_CONST, nullptr, nullptr, s));
+    LA(run_backward(e, unused, true, s));
+    LA(adam_scheduled(e->partial, e->nchunks, e->proj, e->step, e->w_opt, e->m, e->v, e->w_pert, e->batch, g.w_dim, s));
+    e->launches += 2;
+    return 0;
+}
+
+// Runs num_steps of `step` on e->work: the first one ever eagerly (warm-up, flag `warmed`), the rest as replays of one
+// captured graph.  after(it) enqueues per-step work outside the graph.
+template <class Step, class After>
+int run_loop(la_engine* e, int num_steps, bool graphable, bool& warmed, Step step, After after) {
+    cudaStream_t w = e->work;
+    for (int it = 0; it < num_steps; ++it) {
+        if (!graphable || e->graph_disabled || !warmed) {
+            LA(step());
+            warmed = true;
+        } else {
+            if (!e->step_graph) {
+                cudaGraph_t graph = nullptr;
+                const long long before = e->launches;
+                CU(cudaStreamBeginCapture(w, cudaStreamCaptureModeThreadLocal));
+                int r = step();
+                cudaError_t ce = cudaStreamEndCapture(w, &graph);
+                e->launches_captured = e->launches - before;
+                e->launches = before;
+                if (r) { if (graph) cudaGraphDestroy(graph); return r; }
+                CU(ce);
+                e->graph_kernels = e->launches_captured;
+                ce = cudaGraphInstantiate(&e->step_graph, graph, 0);
+                cudaGraphDestroy(graph);
+                CU(ce);
+            }
+            CU(cudaGraphLaunch(e->step_graph, w));
+            e->launches += e->graph_kernels;
+        }
+        LA(after(it));
+    }
     return 0;
 }
 
@@ -792,45 +850,65 @@ LA_API int la_augment(la_engine* e, const float* d_w0, const la_augment_options*
         if (lpips_set_call(e->lp, opt->lpips_crop_x, opt->lpips_crop_y, opt->w_lpips, opt->lpips_norm_mode, w))
             return fail(-7, "lpips: %s", lpips_last_error());
     }
-    if ((e->cur_w_pix != opt->w_pix || e->cur_w_disc != opt->w_disc || (e->cur_w_lpips > 0.f) != (opt->w_lpips > 0.f)) &&
+    if ((e->cur_project || e->cur_w_pix != opt->w_pix || e->cur_w_disc != opt->w_disc || (e->cur_w_lpips > 0.f) != (opt->w_lpips > 0.f)) &&
         e->step_graph) {   // baked into the criterion launches
         cudaGraphExecDestroy(e->step_graph);
         e->step_graph = nullptr;
     }
+    e->cur_project = 0;
     e->cur_w_pix = opt->w_pix;
     e->cur_w_disc = opt->w_disc;
     e->cur_w_lpips = opt->w_lpips;
-    for (int it = 0; it < opt->num_steps; ++it) {
-        const bool synth = opt->w_pix > 0.f || opt->w_disc > 0.f || opt->w_lpips > 0.f;
-        if (!synth || e->graph_disabled || !e->warmed) {
-            LA(run_step(e, *opt, w));
-            e->warmed = true;
-            continue;
-        }
-        if (!e->step_graph) {
-            cudaGraph_t graph = nullptr;
-            const long long before = e->launches;
-            CU(cudaStreamBeginCapture(w, cudaStreamCaptureModeThreadLocal));
-            int r = run_step(e, *opt, w);
-            cudaError_t ce = cudaStreamEndCapture(w, &graph);
-            e->launches_captured = e->launches - before;
-            e->launches = before;
-            if (r) { if (graph) cudaGraphDestroy(graph); return r; }
-            CU(ce);
-            e->graph_kernels = e->launches_captured;
-            ce = cudaGraphInstantiate(&e->step_graph, graph, 0);
-            cudaGraphDestroy(graph);
-            CU(ce);
-        }
-        CU(cudaGraphLaunch(e->step_graph, w));
-        e->launches += e->graph_kernels;
-    }
+    const bool synth = opt->w_pix > 0.f || opt->w_disc > 0.f || opt->w_lpips > 0.f;
+    LA(run_loop(e, opt->num_steps, synth, e->warmed, [&] { return run_step(e, *opt, w); }, [](int) { return 0; }));
     LA(finalize_w(e->w_opt, e->w0, opt->alpha, opt->soft_aug, B, g.w_dim, e->w_aug, w));
     LA(run_forward(e, e->w_aug, g.w_dim, 0, opt->final_noise_mode, d_final_noise, d_img, w));
     CU(cudaMemcpyAsync(d_w_aug, e->w_aug, wbytes, cudaMemcpyDeviceToDevice, w));
     if (d_loss_log && opt->num_steps > 0)
         CU(cudaMemcpyAsync(d_loss_log, e->loss_log, sizeof(float) * LA_LOSS_COLS * (opt->num_steps < LA_MAX_STEPS ? opt->num_steps : LA_MAX_STEPS),
                            cudaMemcpyDeviceToDevice, w));
+    LA(bridge_out(e, s));
+    return 0;
+}
+
+LA_API int la_set_projection_targets(la_engine* e, const float* d_img, la_stream stream) {
+    if (!e || !d_img) return fail(-2, "bad arguments");
+    if (!e->lp) return fail(-2, "la_set_projection_targets needs la_set_lpips (with per_sample_targets = 1)");
+    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    Rgb& top = e->rgb.back();
+    LA(bridge_in(e, s));
+    LA(nchw_to_f4(d_img, e->batch, e->g.img_channels, e->g.img_resolution, top.img, e->work));
+    if (lpips_set_targets(e->lp, top.img, e->work, &e->launches)) return fail(-7, "lpips: %s", lpips_last_error());
+    LA(bridge_out(e, s));
+    return 0;
+}
+
+LA_API int la_project(la_engine* e, const float* d_w0, int num_steps, const float* d_lr, const float* d_sigma, const float* d_wnoise,
+                      float* d_w_out, float* d_loss_log, la_stream stream) {
+    if (!e || !d_w0 || !d_w_out || num_steps < 0 || (num_steps > 0 && (!d_lr || !d_sigma))) return fail(-2, "bad arguments");
+    if (!e->lp || !lpips_has_targets(e->lp)) return fail(-2, "la_project needs la_set_lpips and la_set_projection_targets");
+    const int B = e->batch, wd = e->g.w_dim;
+    const size_t wbytes = sizeof(float) * B * wd;
+    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    cudaStream_t w = e->work;
+    LA(bridge_in(e, s));
+    const ProjConsts hc{d_lr, d_sigma, d_wnoise, num_steps};
+    CU(cudaMemcpyAsync(e->proj, &hc, sizeof hc, cudaMemcpyHostToDevice, w));
+    if (lpips_set_call(e->lp, 0, 0, 1.f, 1, w)) return fail(-7, "lpips: %s", lpips_last_error());      // whole-image window
+    CU(cudaMemcpyAsync(e->w_opt, d_w0, wbytes, cudaMemcpyDeviceToDevice, w));
+    CU(cudaMemsetAsync(e->m, 0, wbytes, w));
+    CU(cudaMemsetAsync(e->v, 0, wbytes, w));
+    CU(cudaMemsetAsync(e->step, 0, sizeof(int), w));
+    LA(perturb_first(e->w_opt, e->proj, e->w_pert, B, wd, w));
+    if (!e->cur_project && e->step_graph) {       // never replay an augmentation step here (nor the reverse, la_augment)
+        cudaGraphExecDestroy(e->step_graph);
+        e->step_graph = nullptr;
+    }
+    e->cur_project = 1;
+    e->cur_w_pix = e->cur_w_disc = e->cur_w_lpips = -1.f;
+    LA(run_loop(e, num_steps, true, e->proj_warmed, [&] { return run_project_step(e, w); },
+                [&](int it) { return d_loss_log ? sum_floats(e->lpips_loss, B, d_loss_log + it, w) : 0; }));
+    CU(cudaMemcpyAsync(d_w_out, e->w_opt, wbytes, cudaMemcpyDeviceToDevice, w));
     LA(bridge_out(e, s));
     return 0;
 }
@@ -911,9 +989,19 @@ LA_API int la_lpips_loss_grad(la_engine* e, const float* d_img, int crop_x, int 
     Rgb& top = e->rgb.back();
     LA(bridge_in(e, s));
     LA(nchw_to_f4(d_img, e->batch, e->g.img_channels, e->g.img_resolution, top.img, e->work));
+    if (norm_mode == 2) {             // the projection's per-sample distance to the targets: the window is the whole image
+        if (crop_x != 0 || crop_y != 0) return fail(-2, "norm_mode 2 (per-sample targets) uses the whole image: crop_x = crop_y = 0");
+        if (lpips_set_call(e->lp, 0, 0, 1.f, 1, e->work) || lpips_forward(e->lp, top.img, 1, e->work, &e->launches) ||
+            lpips_backward(e->lp, top.g_img, 0, e->lpips_loss, 1, e->work, &e->launches))
+            return fail(-7, "lpips: %s", lpips_last_error());
+        LA(f4_to_nchw(top.g_img, e->batch, e->g.img_channels, e->g.img_resolution, d_grad, e->work));
+        CU(cudaMemcpyAsync(d_loss, e->lpips_loss, sizeof(float) * e->batch, cudaMemcpyDeviceToDevice, e->work));
+        LA(bridge_out(e, s));
+        return 0;
+    }
     // (the term enters the objective with a minus sign; the stand-alone call returns d loss / d img, hence -w)
     if (lpips_set_call(e->lp, crop_x, crop_y, -w_lpips, norm_mode, e->work) ||
-        lpips_forward(e->lp, top.img, e->work, &e->launches) || lpips_backward(e->lp, top.g_img, 0, e->lpips_loss, e->work, &e->launches))
+        lpips_forward(e->lp, top.img, 0, e->work, &e->launches) || lpips_backward(e->lp, top.g_img, 0, e->lpips_loss, 0, e->work, &e->launches))
         return fail(-7, "lpips: %s", lpips_last_error());
     LA(f4_to_nchw(top.g_img, e->batch, e->g.img_channels, e->g.img_resolution, d_grad, e->work));
     LA(prep_scale(e->lpips_loss, -1.f, e->lpips_loss, 1, e->work));

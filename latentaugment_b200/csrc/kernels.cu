@@ -876,6 +876,40 @@ __global__ void adam_kernel(const float* __restrict__ partial, int nchunks, int 
 }
 __global__ void step_inc_kernel(int* step_counter) { *step_counter += 1; }
 
+// projection: the same update with the learning rate of step t from the schedule table (projector.py::project)
+__global__ void adam_sched_kernel(const float* __restrict__ partial, int nchunks, const ProjConsts* pc, const int* step_counter, float* w, float* m,
+                                  float* v, float* w_pert, int batch, int w_dim) {
+    const int e = blockIdx.x * blockDim.x + threadIdx.x;
+    const int n = batch * w_dim;
+    if (e >= n) return;
+    float g = 0.f;
+    for (int c = 0; c < nchunks; ++c) g += partial[static_cast<long long>(c) * n + e];
+    const int t = *step_counter;
+    const float b1 = 0.9f, b2 = 0.999f;
+    const float mm = b1 * m[e] + (1.f - b1) * g;
+    const float vv = b2 * v[e] + (1.f - b2) * g * g;
+    m[e] = mm;
+    v[e] = vv;
+    const float bc1 = 1.f - powf(b1, static_cast<float>(t + 1));
+    const float bc2 = 1.f - powf(b2, static_cast<float>(t + 1));
+    const float denom = sqrtf(vv) / sqrtf(bc2) + 1e-8f;
+    const float wn = w[e] - (pc->lr[t] / bc1) * (mm / denom);
+    w[e] = wn;
+    const int next = t + 1;
+    w_pert[e] = (pc->noise && next < pc->num_steps) ? fmaf(pc->sigma[next], pc->noise[static_cast<long long>(next) * n + e], wn) : wn;
+}
+__global__ void perturb_first_kernel(const float* __restrict__ w, const ProjConsts* pc, float* w_pert, int n) {
+    const int e = blockIdx.x * blockDim.x + threadIdx.x;
+    if (e >= n) return;
+    w_pert[e] = (pc->noise && pc->num_steps > 0) ? fmaf(pc->sigma[0], pc->noise[e], w[e]) : w[e];
+}
+__global__ void sum_floats_kernel(const float* __restrict__ x, int n, float* out) {
+    double acc = 0.0;
+    for (int i = threadIdx.x; i < n; i += 32) acc += x[i];
+    acc = warp_sum_d(acc);
+    if (threadIdx.x == 0) out[0] = static_cast<float>(acc);
+}
+
 __global__ void finalize_w_kernel(const float* __restrict__ w_opt, const float* __restrict__ w0, float alpha, int soft, int n,
                                   float* w_aug) {
     const int e = blockIdx.x * blockDim.x + threadIdx.x;
@@ -1160,6 +1194,20 @@ int adam_step(const float* partial, int nchunks, int use_partial, const float* w
                                         crop_size, loss_log, max_steps, disc_loss, lpips_loss);
     adam_kernel<<<cdiv(batch * w_dim, 256), 256, 0, s>>>(partial, nchunks, use_partial, w_sum_bank, consts, step_counter, w, m, v, batch, w_dim);
     step_inc_kernel<<<1, 1, 0, s>>>(step_counter);
+    return last_err();
+}
+int adam_scheduled(const float* partial, int nchunks, const ProjConsts* pc, int* step_counter, float* w, float* m, float* v,
+                   float* w_pert, int batch, int w_dim, cudaStream_t s) {
+    adam_sched_kernel<<<cdiv(batch * w_dim, 256), 256, 0, s>>>(partial, nchunks, pc, step_counter, w, m, v, w_pert, batch, w_dim);
+    step_inc_kernel<<<1, 1, 0, s>>>(step_counter);
+    return last_err();
+}
+int perturb_first(const float* w, const ProjConsts* pc, float* w_pert, int batch, int w_dim, cudaStream_t s) {
+    perturb_first_kernel<<<cdiv(batch * w_dim, 256), 256, 0, s>>>(w, pc, w_pert, batch * w_dim);
+    return last_err();
+}
+int sum_floats(const float* x, int n, float* out, cudaStream_t s) {
+    sum_floats_kernel<<<1, 32, 0, s>>>(x, n, out);
     return last_err();
 }
 int finalize_w(const float* w_opt, const float* w0, float alpha, int soft, int batch, int w_dim, float* w_aug, cudaStream_t s) {

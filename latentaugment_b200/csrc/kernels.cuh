@@ -95,6 +95,21 @@ int adam_step(const float* partial, int nchunks, int use_partial, const float* w
               float* w, float* m, float* v, int batch, int w_dim, const float* pix_parts, int n_pix_parts, const float* bank_m2,
               int img_c, int crop_size, float* loss_log, int max_steps, const float* disc_loss /*or null*/, const float* lpips_loss /*or null*/,
               cudaStream_t s);
+// Projection (la_project): the per-step schedule, device-resident so one captured graph serves every call.
+struct ProjConsts {
+    const float* lr;          // [num_steps]
+    const float* sigma;       // [num_steps] absolute w-noise scale
+    const float* noise;       // [num_steps, batch, w_dim] unit normal, or null
+    int num_steps;
+};
+// Adam step with lr = lr[t] (t = *step_counter), then w_pert = w + sigma[t+1] * noise[t+1] (the code the next step's style
+// GEMMs read; the gradient wrt the perturbed code is the gradient wrt w), then ++*step_counter.
+int adam_scheduled(const float* partial, int nchunks, const ProjConsts* pc, int* step_counter, float* w, float* m, float* v,
+                   float* w_pert, int batch, int w_dim, cudaStream_t s);
+// w_pert = w + sigma[0] * noise[0]  (the code of step 0)
+int perturb_first(const float* w, const ProjConsts* pc, float* w_pert, int batch, int w_dim, cudaStream_t s);
+// out[0] = sum of x[0..n)
+int sum_floats(const float* x, int n, float* out, cudaStream_t s);
 constexpr int kLossCols = 5;      // loss-log row: latent, pixel, total, discriminator, perceptual (== LA_LOSS_COLS)
 int finalize_w(const float* w_opt, const float* w0, float alpha, int soft, int batch, int w_dim, float* w_aug, cudaStream_t s);
 

@@ -116,8 +116,10 @@ __global__ void fill_kernel(float* p, float v, long long n) {
 // x_in [crop = b*imgc + c][y][x][64]: channels 0..2 = (img[b, cy+y, cx+x].c - mean_k) / std_k, 3..63 = 0.
 // src_nchw != null: bank path, crops come as fp32 [n, imgc, cs, cs] (n_valid crops, the rest of the chunk is zero).
 struct ZScore { float mean[3], inv_std[3]; };
+// f > 0: whole-image window of a per-sample-target call (origin 0, 0; res = f * cs), area-downsampled f x f (the mean of each
+// f x f block).  f == 0: the crop window at the call's origin (bank mode).
 __global__ void lpips_crop_kernel(const float4* __restrict__ img, const float* __restrict__ src_nchw, int n_valid, const CallConsts* cc, int res,
-                                  int imgc, int cs, int ncrops, ZScore z, bf16* x_hi, bf16* x_lo) {
+                                  int imgc, int cs, int ncrops, ZScore z, int f, bf16* x_hi, bf16* x_lo) {
     const long long idx = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x;
     if (idx >= static_cast<long long>(ncrops) * cs * cs) return;
     const int x = static_cast<int>(idx % cs), y = static_cast<int>((idx / cs) % cs), crop = static_cast<int>(idx / (static_cast<long long>(cs) * cs));
@@ -128,8 +130,13 @@ __global__ void lpips_crop_kernel(const float4* __restrict__ img, const float* _
         valid = b < n_valid;
         if (valid) v = __ldg(src_nchw + (static_cast<long long>(crop) * cs + y) * cs + x);
     } else {
-        const float4 p = __ldg(img + (static_cast<long long>(b) * res + cc->crop_y + y) * res + cc->crop_x + x);
-        v = c == 0 ? p.x : (c == 1 ? p.y : p.z);
+        const int oy = f ? 0 : cc->crop_y, ox = f ? 0 : cc->crop_x, k = f ? f : 1;
+        for (int dy = 0; dy < k; ++dy)
+            for (int dx = 0; dx < k; ++dx) {
+                const float4 p = __ldg(img + (static_cast<long long>(b) * res + oy + k * y + dy) * res + ox + k * x + dx);
+                v += c == 0 ? p.x : (c == 1 ? p.y : p.z);
+            }
+        if (k > 1) v *= 1.f / static_cast<float>(k * k);
     }
     float ch[4] = {0.f, 0.f, 0.f, 0.f};
     if (valid) {
@@ -149,9 +156,10 @@ __global__ void lpips_crop_kernel(const float4* __restrict__ img, const float* _
         for (int j = 1; j < 8; ++j) dl[j] = zero;
     }
 }
-// g_img[b, cy+y, cx+x].c += sum_k g_in[crop, y, x, k] / std_k
+// g_img[b, cy+y, cx+x].c += sum_k g_in[crop, y, x, k] / std_k   (f as in lpips_crop_kernel; f > 1: / f^2 to each pixel of the
+// f x f block, the pool's adjoint)
 __global__ void lpips_crop_bwd_kernel(const bf16* __restrict__ g_hi, const bf16* __restrict__ g_lo, const CallConsts* cc, int res, int imgc, int cs,
-                                      int ncrops, ZScore z, float4* g_img) {
+                                      int ncrops, ZScore z, int f, float4* g_img) {
     const long long idx = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x;
     if (idx >= static_cast<long long>(ncrops) * cs * cs) return;
     const int x = static_cast<int>(idx % cs), y = static_cast<int>((idx / cs) % cs), crop = static_cast<int>(idx / (static_cast<long long>(cs) * cs));
@@ -163,8 +171,13 @@ __global__ void lpips_crop_bwd_kernel(const bf16* __restrict__ g_hi, const bf16*
         if (g_lo) v += __bfloat162float(g_lo[idx * 64 + k]);
         g = fmaf(v, z.inv_std[k], g);
     }
-    float* dst = reinterpret_cast<float*>(g_img + (static_cast<long long>(b) * res + cc->crop_y + y) * res + cc->crop_x + x) + c;
-    *dst += g;
+    const int oy = f ? 0 : cc->crop_y, ox = f ? 0 : cc->crop_x, k = f ? f : 1;
+    if (k > 1) g *= 1.f / static_cast<float>(k * k);
+    for (int dy = 0; dy < k; ++dy)
+        for (int dx = 0; dx < k; ++dx) {
+            float* dst = reinterpret_cast<float*>(g_img + (static_cast<long long>(b) * res + oy + k * y + dy) * res + ox + k * x + dx) + c;
+            *dst += g;
+        }
 }
 
 // ------------------------------------------------------------------------- 2x2 max-pool and its adjoint (+ tap gradient + ReLU mask)
@@ -232,7 +245,10 @@ __global__ void pool_bwd_kernel(const unsigned* __restrict__ gp_hi, const unsign
 //        -> out (masked by x > 0 when `mask`: the tap is the last layer, its ReLU gradient is applied here)
 //   mode 1 (bank):  b_bar += n^ / M,  M2 += sum_ch w n^2 / (P M)   for the valid crops
 //   mode 2 (test hook):  n^ -> fp32 out
-template <int MODE>
+// TGT (per-sample targets; bank_mean is then [crop][P][C], one target per crop):
+//   mode 1 stores n^ of the target crop;  mode 0:  S[sample] += sum_ch w (n^ - t)^2 / P,  g_n = (2 / P) w (n^ - t)
+//   (the projection minimises the distance, so the sign is the opposite of the bank term's)
+template <int MODE, bool TGT = false>
 __global__ void __launch_bounds__(256) lpips_tap_kernel(const unsigned* __restrict__ x_hi, const unsigned* __restrict__ x_lo, int ncrops, int imgc, int P,
                                                         int C, const float* __restrict__ lin_w, float* bank_mean, const CallConsts* cc, int n_valid_crops,
                                                         float inv_m, double* S, float* m2, int mask, unsigned* out_hi, unsigned* out_lo, float* out_f32) {
@@ -240,6 +256,11 @@ __global__ void __launch_bounds__(256) lpips_tap_kernel(const unsigned* __restri
     const long long total_px = static_cast<long long>(ncrops) * P;
     float s_block = 0.f;             // this warp's loss partial over all its pixels (grid-stride walk: few, long-lived blocks, so
                                      // the loss needs one double atomic per block instead of one per 8 pixels)
+    extern __shared__ float s_part[];      // TGT mode 0: this block's loss partial per sample [batch] (dynamic shared memory)
+    if (MODE == 0 && TGT) {
+        for (int i = threadIdx.x; i < ncrops / imgc; i += blockDim.x) s_part[i] = 0.f;
+        __syncthreads();
+    }
     for (long long pix = blockIdx.x * static_cast<long long>(warps) + (threadIdx.x >> 5); pix < total_px;
          pix += static_cast<long long>(gridDim.x) * warps) {
     float s_acc = 0.f;
@@ -262,6 +283,11 @@ __global__ void __launch_bounds__(256) lpips_tap_kernel(const unsigned* __restri
 #pragma unroll
             for (int j = 0; j < 8; ++j)
                 if (j < npair) reinterpret_cast<float2*>(out_f32)[pix * hc + j * 32 + lane] = make_float2(x[j].x * inv, x[j].y * inv);
+        } else if (MODE == 1 && TGT) {
+            float* bm = bank_mean + (static_cast<long long>(crop) * P + p) * C;
+#pragma unroll
+            for (int j = 0; j < 8; ++j)
+                if (j < npair) reinterpret_cast<float2*>(bm)[j * 32 + lane] = make_float2(__fmul_rn(x[j].x, inv), __fmul_rn(x[j].y, inv));
         } else if (MODE == 1) {
             if (crop < n_valid_crops) {
                 float* bm = bank_mean + (static_cast<long long>(mod) * P + p) * C;
@@ -279,8 +305,8 @@ __global__ void __launch_bounds__(256) lpips_tap_kernel(const unsigned* __restri
                 if (lane == 0) atomicAdd(m2 + mod, s_acc * inv_m / P);
             }
         } else {
-            const float* bm = bank_mean + (static_cast<long long>(mod) * P + p) * C;
-            const float coef = -(cc->w_lpips / imgc) * cc->norm * 2.f / P;
+            const float* bm = bank_mean + (static_cast<long long>(TGT ? crop : mod) * P + p) * C;
+            const float coef = TGT ? 2.f / P : -(cc->w_lpips / imgc) * cc->norm * 2.f / P;
             float2 g[8];
             float dot = 0.f;
 #pragma unroll
@@ -289,8 +315,11 @@ __global__ void __launch_bounds__(256) lpips_tap_kernel(const unsigned* __restri
                     const int ch = 2 * (j * 32 + lane);
                     const float2 w = __ldg(reinterpret_cast<const float2*>(lin_w + ch));
                     const float2 b = __ldg(reinterpret_cast<const float2*>(bm + ch));
-                    const float n0 = x[j].x * inv, n1 = x[j].y * inv;
-                    s_acc = fmaf(w.x * n0, n0 - 2.f * b.x, fmaf(w.y * n1, n1 - 2.f * b.y, s_acc));
+                    // TGT: n^ rounded exactly as the target pass stored it (no FMA contraction into n^ - t), so an image
+                    // equal to its target gives exactly zero loss and gradient
+                    const float n0 = TGT ? __fmul_rn(x[j].x, inv) : x[j].x * inv, n1 = TGT ? __fmul_rn(x[j].y, inv) : x[j].y * inv;
+                    if (TGT) s_acc = fmaf(w.x * (n0 - b.x), n0 - b.x, fmaf(w.y * (n1 - b.y), n1 - b.y, s_acc));
+                    else s_acc = fmaf(w.x * n0, n0 - 2.f * b.x, fmaf(w.y * n1, n1 - 2.f * b.y, s_acc));
                     g[j].x = coef * w.x * (n0 - b.x);
                     g[j].y = coef * w.y * (n1 - b.y);
                     dot = fmaf(g[j].x, x[j].x, fmaf(g[j].y, x[j].y, dot));
@@ -305,11 +334,19 @@ __global__ void __launch_bounds__(256) lpips_tap_kernel(const unsigned* __restri
                     st_sp2(out_hi, out_lo, pix * hc + j * 32 + lane, o0, o1);
                 }
             s_acc = warp_sum(s_acc) / P;
-            s_block += s_acc;
+            if (TGT) {
+                if (lane == 0) atomicAdd(s_part + crop / imgc, s_acc);
+            } else {
+                s_block += s_acc;
+            }
         }
     }
     }
-    if (MODE == 0) {       // one double atomic per block
+    if (MODE == 0 && TGT) {       // one double atomic per (block, sample it touched)
+        __syncthreads();
+        for (int i = threadIdx.x; i < ncrops / imgc; i += blockDim.x)
+            if (s_part[i] != 0.f) atomicAdd(S + i, static_cast<double>(s_part[i]));
+    } else if (MODE == 0) {       // one double atomic per block
         __shared__ float sm[8];
         if (lane == 0) sm[threadIdx.x >> 5] = s_block;
         __syncthreads();
@@ -325,6 +362,10 @@ __global__ void lpips_loss_kernel(const double* S, const float* m2, int imgc, in
     double m = 0.0;
     for (int c = 0; c < imgc; ++c) m += m2[c];
     loss[0] = static_cast<float>((cc->w_lpips / imgc) * cc->norm * (S[0] + batch * m));
+}
+// per-sample targets: loss[b] = sum over modalities and taps of the distance of sample b to its own target
+__global__ void lpips_target_loss_kernel(const double* S, int batch, float* loss) {
+    for (int b = threadIdx.x; b < batch; b += blockDim.x) loss[b] = static_cast<float>(S[b]);
 }
 
 struct Bump {
@@ -349,6 +390,7 @@ struct TapL {
     int used, conv, C, R;
     const float* lin_w;
     float* bank_mean;           // [imgc][R*R][C]
+    float* target;              // [ncrops][R*R][C] normalised activations of the per-sample targets (when planned)
     Pl tg;                      // gradient wrt the tap tensor (before its ReLU mask); unused for the last tap
 };
 
@@ -357,12 +399,13 @@ struct TapL {
 struct la_lpips {
     la_vgg_desc d;
     int batch, imgc, res, split, num_sms, ncrops, cs, last_conv, ntaps_used, has_bank;
+    int has_targets, pool_f;    // per-sample targets set; area-pool factor res / crop of the whole-image window
     Conv conv[kNConv];
     TapL tap[LA_VGG_TAPS];
     Pl x_in, g_in, pool[4], gp, gz[2];
     float* ones;
     float* m2;                  // [4] per-modality bank constant
-    double* S;
+    double* S;                  // [batch] (loss partials; one per sample in target mode)
     CallConsts* cc;
     int* err_flag;
     ZScore z;
@@ -442,10 +485,11 @@ int plan_lpips(la_lpips* L, char* ws, size_t* bytes_out) {
         if (!T.used) continue;
         T.bank_mean = bp.take<float>(static_cast<size_t>(L->imgc) * T.R * T.R * T.C);
         if (T.conv != L->last_conv) T.tg = take_pl(n * T.R * T.R * T.C);
+        T.target = d.per_sample_targets ? bp.take<float>(n * T.R * T.R * T.C) : nullptr;    // fp32, ~32 MB per crop at a 256 window
     }
     L->ones = bp.take<float>(n * 512);
     L->m2 = bp.take<float>(4);
-    L->S = bp.take<double>(1);
+    L->S = bp.take<double>(L->batch);
     L->cc = bp.take<CallConsts>(1);
     L->err_flag = bp.take<int>(1);
     bp.take<char>(1024);
@@ -514,7 +558,7 @@ int prepare_lpips(la_lpips* L, cudaStream_t s) {
     LCU(cudaGetLastError());
     LCU(cudaMemsetAsync(L->err_flag, 0, sizeof(int), s));
     LCU(cudaMemsetAsync(L->m2, 0, 4 * sizeof(float), s));
-    LCU(cudaMemsetAsync(L->S, 0, sizeof(double), s));
+    LCU(cudaMemsetAsync(L->S, 0, sizeof(double) * L->batch, s));
     LCU(cudaMemsetAsync(L->cc, 0, sizeof(CallConsts), s));
     LCU(cudaStreamSynchronize(s));
     return 0;
@@ -564,6 +608,15 @@ int lpips_create(const la_vgg_desc& d, int batch, int img_channels, int img_reso
         if (!(d.std[k] > 0.f)) { delete L; return lfail(-2, "lpips: std[%d] must be positive", k); }
         L->z.mean[k] = d.mean[k]; L->z.inv_std[k] = 1.f / d.std[k];
     }
+    L->pool_f = 1;
+    if (d.per_sample_targets) {       // whole-image window: crop == res, or res / 2 with a 2x2 area pool (512 -> 256)
+        if (img_resolution > 512 || (d.crop_size != img_resolution && 2 * d.crop_size != img_resolution) ||
+            d.crop_size != (img_resolution < 256 ? img_resolution : 256)) {
+            delete L;
+            return lfail(-2, "lpips: per-sample targets need crop_size == min(res, 256) and res <= 512 (crop %d, res %d)", d.crop_size, img_resolution);
+        }
+        L->pool_f = img_resolution / d.crop_size;
+    }
     size_t need = 0;
     int r = plan_lpips(L, static_cast<char*>(ws), &need);
     if (!r && need > bytes) r = lfail(-2, "lpips workspace too small: %zu < %zu", bytes, need);
@@ -596,7 +649,7 @@ int lpips_set_bank(la_lpips* L, const float* d_crops, int M, cudaStream_t s, lon
     for (int m0 = 0; m0 < M; m0 += L->batch) {
         const int nv = M - m0 < L->batch ? M - m0 : L->batch;
         lpips_crop_kernel<<<cdiv(npx, 256), 256, 0, s>>>(nullptr, d_crops + static_cast<long long>(m0) * L->imgc * L->cs * L->cs, nv, L->cc, L->res,
-                                                        L->imgc, L->cs, L->ncrops, L->z, L->x_in.hi, L->x_in.lo);
+                                                        L->imgc, L->cs, L->ncrops, L->z, 0, L->x_in.hi, L->x_in.lo);
         LCU(cudaGetLastError());
         LLA(run_network(L, s, launches));
         for (int t = 0; t < LA_VGG_TAPS; ++t) {
@@ -613,17 +666,41 @@ int lpips_set_bank(la_lpips* L, const float* d_crops, int M, cudaStream_t s, lon
     return 0;
 }
 
-int lpips_forward(la_lpips* L, const float4* img, cudaStream_t s, long long* launches) {
+int lpips_forward(la_lpips* L, const float4* img, int targets, cudaStream_t s, long long* launches) {
     const long long npx = static_cast<long long>(L->ncrops) * L->cs * L->cs;
-    lpips_crop_kernel<<<cdiv(npx, 256), 256, 0, s>>>(img, nullptr, L->batch, L->cc, L->res, L->imgc, L->cs, L->ncrops, L->z, L->x_in.hi, L->x_in.lo);
+    lpips_crop_kernel<<<cdiv(npx, 256), 256, 0, s>>>(img, nullptr, L->batch, L->cc, L->res, L->imgc, L->cs, L->ncrops, L->z, targets ? L->pool_f : 0,
+                                                    L->x_in.hi, L->x_in.lo);
     LCU(cudaGetLastError());
     if (launches) ++*launches;
     return run_network(L, s, launches);
 }
 
-int lpips_backward(la_lpips* L, float4* g_img, int accumulate, float* d_loss, cudaStream_t s, long long* launches) {
-    if (!L->has_bank) return lfail(-2, "lpips: no feature bank (la_set_feature_bank)");
-    LCU(cudaMemsetAsync(L->S, 0, sizeof(double), s));
+int lpips_has_targets(const la_lpips* L) { return L->has_targets; }
+
+int lpips_set_targets(la_lpips* L, const float4* img, cudaStream_t s, long long* launches) {
+    bool planned = false;
+    for (int t = 0; t < LA_VGG_TAPS; ++t) planned = planned || L->tap[t].target;
+    if (!planned) return lfail(-2, "lpips: per-sample targets were not planned (la_vgg_desc.per_sample_targets = 0)");
+    LLA(lpips_set_call(L, 0, 0, 1.f, 1, s));
+    LLA(lpips_forward(L, img, 1, s, launches));
+    for (int t = 0; t < LA_VGG_TAPS; ++t) {
+        TapL& T = L->tap[t];
+        if (!T.used) continue;
+        const Conv& c = L->conv[T.conv];
+        const long long pixels = static_cast<long long>(L->ncrops) * T.R * T.R;
+        lpips_tap_kernel<1, true><<<tap_grid(pixels, L->num_sms), 256, 0, s>>>(CU32(c.x.hi), CU32(c.x.lo), L->ncrops, L->imgc, T.R * T.R, T.C, T.lin_w,
+                                                                          T.target, L->cc, L->ncrops, 0.f, nullptr, nullptr, 0, nullptr, nullptr, nullptr);
+        LCU(cudaGetLastError());
+        if (launches) ++*launches;
+    }
+    L->has_targets = 1;
+    return 0;
+}
+
+int lpips_backward(la_lpips* L, float4* g_img, int accumulate, float* d_loss, int targets, cudaStream_t s, long long* launches) {
+    if (targets && !L->has_targets) return lfail(-2, "lpips: no per-sample targets (la_set_projection_targets)");
+    if (!targets && !L->has_bank) return lfail(-2, "lpips: no feature bank (la_set_feature_bank)");
+    LCU(cudaMemsetAsync(L->S, 0, sizeof(double) * (targets ? L->batch : 1), s));
     if (!accumulate) LCU(cudaMemsetAsync(g_img, 0, sizeof(float4) * static_cast<size_t>(L->batch) * L->res * L->res, s));
     for (int t = 0; t < LA_VGG_TAPS; ++t) {
         TapL& T = L->tap[t];
@@ -632,8 +709,12 @@ int lpips_backward(la_lpips* L, float4* g_img, int accumulate, float* d_loss, cu
         const bool last = T.conv == L->last_conv;
         const Pl& out = last ? L->gz[T.conv & 1] : T.tg;
         const long long pixels = static_cast<long long>(L->ncrops) * T.R * T.R;
-        lpips_tap_kernel<0><<<tap_grid(pixels, L->num_sms), 256, 0, s>>>(CU32(c.x.hi), CU32(c.x.lo), L->ncrops, L->imgc, T.R * T.R, T.C, T.lin_w, T.bank_mean, L->cc,
-                                                          L->ncrops, 0.f, L->S, nullptr, last ? 1 : 0, U32(out.hi), U32(out.lo), nullptr);
+        if (targets)
+            lpips_tap_kernel<0, true><<<tap_grid(pixels, L->num_sms), 256, sizeof(float) * L->batch, s>>>(CU32(c.x.hi), CU32(c.x.lo), L->ncrops, L->imgc, T.R * T.R, T.C, T.lin_w, T.target,
+                                                                              L->cc, L->ncrops, 0.f, L->S, nullptr, last ? 1 : 0, U32(out.hi), U32(out.lo), nullptr);
+        else
+            lpips_tap_kernel<0><<<tap_grid(pixels, L->num_sms), 256, 0, s>>>(CU32(c.x.hi), CU32(c.x.lo), L->ncrops, L->imgc, T.R * T.R, T.C, T.lin_w, T.bank_mean, L->cc,
+                                                              L->ncrops, 0.f, L->S, nullptr, last ? 1 : 0, U32(out.hi), U32(out.lo), nullptr);
         LCU(cudaGetLastError());
         if (launches) ++*launches;
     }
@@ -656,9 +737,11 @@ int lpips_backward(la_lpips* L, float4* g_img, int accumulate, float* d_loss, cu
         }
     }
     const long long npx = static_cast<long long>(L->ncrops) * L->cs * L->cs;
-    lpips_crop_bwd_kernel<<<cdiv(npx, 256), 256, 0, s>>>(L->g_in.hi, L->g_in.lo, L->cc, L->res, L->imgc, L->cs, L->ncrops, L->z, g_img);
+    lpips_crop_bwd_kernel<<<cdiv(npx, 256), 256, 0, s>>>(L->g_in.hi, L->g_in.lo, L->cc, L->res, L->imgc, L->cs, L->ncrops, L->z,
+                                                        targets ? L->pool_f : 0, g_img);
     LCU(cudaGetLastError());
-    lpips_loss_kernel<<<1, 1, 0, s>>>(L->S, L->m2, L->imgc, L->batch, L->cc, d_loss);
+    if (targets) lpips_target_loss_kernel<<<1, 128, 0, s>>>(L->S, L->batch, d_loss);
+    else lpips_loss_kernel<<<1, 1, 0, s>>>(L->S, L->m2, L->imgc, L->batch, L->cc, d_loss);
     LCU(cudaGetLastError());
     if (launches) *launches += 2;
     return 0;

@@ -27,11 +27,19 @@ int lpips_has_bank(const la_lpips* L);
 // form; 1: sum over samples of the bank mean -- the forward_tr form).  Asynchronous on s.
 int lpips_set_call(la_lpips* L, int crop_x, int crop_y, float w_lpips, int norm_mode, cudaStream_t s);
 
-// img: float4 per pixel [B, R, R].  Crops, z-scores and runs VGG16 up to the last tap.
-int lpips_forward(la_lpips* L, const float4* img, cudaStream_t s, long long* launches);
+// img: float4 per pixel [B, R, R].  Crops, z-scores and runs VGG16 up to the last tap.  targets != 0: the window is the whole
+// image (crop origin 0, 0), area-pooled 2x2 when the image is twice the crop (per-sample-target mode).
+int lpips_forward(la_lpips* L, const float4* img, int targets, cudaStream_t s, long long* launches);
 // (after lpips_forward) loss value = w_lpips * mean over modalities of the pair-normalised LPIPS distance -> d_loss[0];
 // g_img[pix] (+)= d(-loss)/d img  (the term enters the objective with a minus sign, util_latent_aug.py:270).
-int lpips_backward(la_lpips* L, float4* g_img, int accumulate, float* d_loss, cudaStream_t s, long long* launches);
+// targets != 0 (projection): d_loss[b] = sum over modalities and taps of sample b's distance to its own target,
+// g_img (+)= d (sum_b d_loss[b]) / d img  (minimised, so no sign flip and no w_lpips / pair normaliser).
+int lpips_backward(la_lpips* L, float4* g_img, int accumulate, float* d_loss, int targets, cudaStream_t s, long long* launches);
+
+// Per-sample targets of the projection: img float4 [B, R, R] -> normalised activations per (sample, modality, tap), fp32.
+// Needs la_vgg_desc.per_sample_targets (the storage is planned in the workspace).  Sets the call constants to the whole window.
+int lpips_set_targets(la_lpips* L, const float4* img, cudaStream_t s, long long* launches);
+int lpips_has_targets(const la_lpips* L);
 
 // Test hook: normalised activations of tap k of the crops computed by the last lpips_forward -> fp32 [n_crops, h, w, C] (NHWC).
 int lpips_copy_tap(la_lpips* L, int k, float* d_out, size_t* count, cudaStream_t s);

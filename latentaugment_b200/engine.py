@@ -8,6 +8,7 @@ import math
 import torch
 
 from . import _lib
+from . import projection as _proj
 
 _PARAM_ORDER_DOC = 'parameter names follow the reference contract models/stylegan3/legacy.py:171-203'
 
@@ -204,10 +205,12 @@ class SynthesisEngine:
     VGG_TAP_LAYERS = (4, 9, 16, 23, 30)                                  # 1-based layer indices of networks.py:52-64
     VGG_TAP_CHANNELS = (64, 128, 256, 512, 512)
 
-    def set_lpips(self, state, taps=(16, 23, 30), crop_size=64, mean=(-.030, -.088, -.188), std=(.458, .448, .450)):
+    def set_lpips(self, state, taps=(16, 23, 30), crop_size=64, mean=(-.030, -.088, -.188), std=(.458, .448, .450),
+                  per_sample_targets=False):
         """``state``: torchvision names ``features.{i}.{weight,bias}`` + LPIPS lin layers ``lin.{k}.weight`` ([1, C, 1, 1] or
         [C]; k counts the used ``taps`` in order; criteria/lpips/networks.py:22-32).  ``taps``: 1-based layer indices as in
-        ``VGG16.target_layers`` (networks.py:94)."""
+        ``VGG16.target_layers`` (networks.py:94).  ``per_sample_targets``: also plan the target features of the projection
+        (``set_projection_targets``; needs ``crop_size == min(img_resolution, 256)``)."""
         keep = self._lpips_keep = []
 
         def dev(t):
@@ -227,6 +230,7 @@ class SynthesisEngine:
         for k in range(3):
             d.mean[k], d.std[k] = float(mean[k]), float(std[k])
         d.crop_size = int(crop_size)
+        d.per_sample_targets = int(bool(per_sample_targets))
         nbytes = C.c_size_t(0)
         _lib.check(self.lib.la_lpips_workspace_bytes(C.byref(d), self.batch, self.img_channels, _lib.PRECISION[self.precision], C.byref(nbytes)))
         self.lpips_workspace = torch.empty(nbytes.value + 1024, dtype=torch.uint8, device=self.device)
@@ -277,6 +281,68 @@ class SynthesisEngine:
         ch = self.VGG_TAP_CHANNELS[slot]
         hw = int(round((n.value // (self.batch * self.img_channels * ch)) ** 0.5))
         return out.reshape(self.batch * self.img_channels, hw, hw, ch)
+
+    # ---- projection of real images into W (projector.py::project, batched; DESIGN.md "Projection")
+    def set_projection_targets(self, img):
+        """Targets [batch, C, res, res] in [-1, 1] (``x / 127.5 - 1`` of the 0..255 images).  Needs ``set_lpips(...,
+        per_sample_targets=True)``."""
+        img = img.detach().to(self.device, torch.float32).contiguous()
+        assert img.shape == (self.batch, self.img_channels, self.img_resolution, self.img_resolution), img.shape
+        with torch.cuda.device(self.device):
+            _lib.check(self.lib.la_set_projection_targets(self.handle, _ptr(img), _stream_ptr(self.device)))
+        torch.cuda.current_stream(self.device).synchronize()
+
+    def projection_loss_grad(self, img):
+        """(per-sample distance [batch] of ``img`` to the projection targets, d sum / d img): the projection's loss alone."""
+        img = img.detach().to(self.device, torch.float32).contiguous()
+        loss = torch.empty([self.batch], device=self.device)
+        grad = torch.empty_like(img)
+        with torch.cuda.device(self.device):
+            _lib.check(self.lib.la_lpips_loss_grad(self.handle, _ptr(img), 0, 0, 1.0, 2, _ptr(loss), _ptr(grad), _stream_ptr(self.device)))
+        return loss, grad
+
+    def w_stats(self):
+        """(w_avg [w_dim], w_std) of 10 000 mapped ``z`` (``RandomState(123)``, psi = 1, row 0), float64 on the host; cached."""
+        if getattr(self, '_w_stats', None) is None:
+            if self.desc.mapping_layers < 1:
+                raise _lib.LatentAugmentError('projection needs the mapping network (w_avg / w_std); this generator has none')
+            z = torch.from_numpy(_proj.w_avg_z(self.z_dim)).float().to(self.device)
+            w = torch.empty([z.shape[0], self.w_dim], device=self.device)
+            with torch.cuda.device(self.device):
+                for i in range(0, z.shape[0], self.batch):
+                    j = min(z.shape[0], i + self.batch)
+                    _lib.check(self.lib.la_mapping(self.handle, _ptr(z[i:j]), j - i, 1.0, _ptr(w[i:j]), _stream_ptr(self.device)))
+            self._w_stats = _proj.w_stats_from_samples(w.cpu().double().numpy())
+        return self._w_stats
+
+    def project(self, w0=None, *, num_steps=_proj.NUM_STEPS, initial_lr=_proj.INITIAL_LR, initial_noise_factor=_proj.INITIAL_NOISE_FACTOR,
+                lr_rampdown_length=_proj.LR_RAMPDOWN_LENGTH, lr_rampup_length=_proj.LR_RAMPUP_LENGTH,
+                noise_ramp_length=_proj.NOISE_RAMP_LENGTH, w_noise=None, seed=0, return_losses=False):
+        """Projects the targets of ``set_projection_targets`` into W: ``num_steps`` Adam steps on one code per sample from
+        ``w0`` [batch, w_dim] (default ``w_avg``).  ``w_noise`` [T, batch, w_dim] unit normal draws of the w noise (default: drawn
+        on the CPU from ``torch.Generator().manual_seed(seed)``).  Returns w [batch, w_dim] (and the summed loss of every step)."""
+        T, B = int(num_steps), self.batch
+        w_avg, w_std = self.w_stats()
+        if w0 is None:
+            w0 = torch.from_numpy(w_avg).float().unsqueeze(0).repeat(B, 1)
+        w0 = w0.detach().to(self.device, torch.float32).reshape(B, self.w_dim).contiguous()
+        lr, sigma = _proj.projection_schedule(T, initial_lr=initial_lr, initial_noise_factor=initial_noise_factor,
+                                              lr_rampdown_length=lr_rampdown_length, lr_rampup_length=lr_rampup_length,
+                                              noise_ramp_length=noise_ramp_length)
+        lr = torch.from_numpy(lr).float().to(self.device)
+        sigma = torch.from_numpy(sigma * w_std).float().to(self.device)
+        if w_noise is None:
+            w_noise = torch.randn([T, B, self.w_dim], generator=torch.Generator().manual_seed(int(seed)))
+        w_noise = w_noise.detach().to(self.device, torch.float32).contiguous()
+        assert w_noise.shape == (T, B, self.w_dim), w_noise.shape
+        w = torch.empty([B, self.w_dim], device=self.device)
+        losses = torch.zeros([max(T, 1)], device=self.device) if return_losses else None
+        with torch.cuda.device(self.device):
+            _lib.check(self.lib.la_project(self.handle, _ptr(w0), T, _ptr(lr), _ptr(sigma), _ptr(w_noise), _ptr(w), _ptr(losses),
+                                           _stream_ptr(self.device)))
+        if return_losses:
+            return w, losses[:T]
+        return w
 
     # ---- network
     def mapping(self, z, truncation_psi=1.0):
