@@ -266,6 +266,25 @@ int la_merge_topk(const float* d_dist, const long long* d_idx, int shards, int n
 int la_merge_topk_strided(const float* d_dist, const long long* d_idx, int shards, int n, int k, long long dist_shard_stride,
                           long long idx_shard_stride, float* d_out_dist, long long* d_out_idx, la_stream stream);
 
+/* Precision / recall of feature sets (StyleGAN3 compute_pr; DESIGN.md §12).  The manifold Y [m, K] and the queries hold
+ * fp16-valued fp32 features; d2 is the distance above.  la_pr_manifold_prepare fills d_planes [2, m, K] bf16 (hi | lo: an fp16
+ * value is exactly hi + lo) and d_sqnorm [m + 1] (squared norms followed by their maximum).  Candidates are scored by three
+ * bf16 tensor-core passes over the planes, (hi,hi) + (lo,hi) + (hi,lo); exact rechecks make both results exact for any data.
+ *   la_pr_radii:  d_r2[i] = the (nhood + 1)-th smallest d2(X_i, Y_j) over all j (a point of the manifold counts itself and
+ *                 duplicates count).  X [n, K] are the rows whose radii are wanted (normally rows of Y).  1 <= nhood <= 7,
+ *                 m >= nhood + 1.
+ *   la_pr_member: d_member[i] = 1 when, for some j, h(d2(X_i, Y_j)) <= h(d_r2[j]) with h(v) = fp16(sqrt(max(v, 0)))
+ *                 (round to nearest even, saturating to +inf), else 0.  X [n, K] are the probes.
+ * Each adds to *d_fallback (device int, the caller zeroes it; NULL = not counted) the number of queries that were scanned
+ * exhaustively because their candidate list overflowed.  K must be a multiple of 64; workspaces 1024-byte aligned. */
+int la_pr_manifold_prepare(const float* d_Y, int m, int K, void* d_planes, float* d_sqnorm, la_stream stream);
+int la_pr_radii_workspace_bytes(int n, int m, int K, int nhood, size_t* bytes);
+int la_pr_radii(const float* d_X, int n, const float* d_Y, const void* d_planes, const float* d_sqnorm, int m, int K, int nhood,
+                void* d_workspace, size_t workspace_bytes, float* d_r2, int* d_fallback, la_stream stream);
+int la_pr_member_workspace_bytes(int n, int m, int K, size_t* bytes);
+int la_pr_member(const float* d_X, int n, const float* d_Y, const void* d_planes, const float* d_sqnorm, const float* d_r2, int m, int K,
+                 void* d_workspace, size_t workspace_bytes, unsigned char* d_member, int* d_fallback, la_stream stream);
+
 /* Test hooks: run every tap-GEMM of the engine once through the SIMT twin as well and report
  * the largest deviation (debug cross-check of the tensor-core path; not a product path). */
 int la_debug_set_simt(la_engine* e, int use_simt);

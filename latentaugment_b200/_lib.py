@@ -101,7 +101,14 @@ SIGNATURES = {
     'la_merge_topk': (C.c_int, [fptr, C.c_void_p, C.c_int, C.c_int, C.c_int, fptr, C.c_void_p, C.c_void_p]),
     'la_merge_topk_strided': (C.c_int, [fptr, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_longlong, C.c_longlong, fptr, C.c_void_p,
                                         C.c_void_p]),
-    'la_debug_set_simt': (C.c_int, [C.c_void_p, C.c_int]),
+    'la_pr_manifold_prepare': (C.c_int, [fptr, C.c_int, C.c_int, C.c_void_p, fptr, C.c_void_p]),
+    'la_pr_radii_workspace_bytes': (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_size_t)]),
+    'la_pr_radii': (C.c_int, [fptr, C.c_int, fptr, C.c_void_p, fptr, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_size_t, fptr,
+                              C.c_void_p, C.c_void_p]),
+    'la_pr_member_workspace_bytes': (C.c_int, [C.c_int, C.c_int, C.c_int, C.POINTER(C.c_size_t)]),
+    'la_pr_member': (C.c_int, [fptr, C.c_int, fptr, C.c_void_p, fptr, fptr, C.c_int, C.c_int, C.c_void_p, C.c_size_t, C.c_void_p,
+                               C.c_void_p, C.c_void_p]),
+    'la_debug_set_simt':(C.c_int, [C.c_void_p, C.c_int]),
     'la_debug_launch_count': (C.c_longlong, [C.c_void_p]),
     'la_debug_get': (C.c_int, [C.c_void_p, C.c_int, fptr, C.POINTER(C.c_size_t), C.c_void_p]),
     'la_debug_check': (C.c_int, [C.c_void_p, C.c_void_p]),

@@ -440,6 +440,37 @@ __device__ __forceinline__ void rowowner_warp_tile(const TapGemmParams& P, const
                 *reinterpret_cast<float2*>(P.cand_score + base) = make_float2(m1, m2);
                 *reinterpret_cast<int2*>(P.cand_idx + base) = make_int2(i1, i2);
             }
+        } else if constexpr (EPI == kEpiMember) {
+            // d = s^ - (T_j - |x|^2) with s^ = |y|^2 - 2<x,y>: d <= -margin is a definite hit, |d| <= margin ambiguous (the
+            // exact recheck decides), anything else a definite miss.  T_j = +inf gives d = -inf: a hit.
+            if (tk_valid) {
+                const float xi = __ldg(P.query_sqnorm + rc.pix);
+                const float ymax = __ldg(P.code_sqnorm + P.n_codes);
+                const float eps = P.member_eps * sqrtf(xi) * sqrtf(ymax) + 6e-7f * (xi + ymax);
+                bool hit = false;
+                unsigned amb = 0u;
+#pragma unroll
+                for (int j = 0; j < 32; ++j) {
+                    const int code = col0 + j;
+                    if (code < P.n_codes) {
+                        const float4 t = __ldg(P.member_tab + code);
+                        const float d = fmaf(-2.f, acc[j], t.x) - (t.y - xi);
+                        const float mg = eps + t.z;
+                        hit |= d <= -mg;
+                        amb |= (d <= mg ? 1u : 0u) << j;
+                    }
+                }
+                if (hit) {
+                    P.member_hit[rc.pix] = 1;
+                } else if (amb) {
+                    int slot = atomicAdd(P.member_cnt + rc.pix, __popc(amb));
+                    int* lst = P.member_list + rc.pix * P.member_cap;
+                    while (amb && slot < P.member_cap) {
+                        lst[slot++] = col0 + __ffs(amb) - 1;
+                        amb &= amb - 1;
+                    }
+                }
+            }
         } else if constexpr (EPI == kEpiFwd) {
             if (kStaged) {
                 // staged path (one sample per tile): coefficients come from the warp group's shared-memory table
@@ -1264,7 +1295,7 @@ __global__ void __launch_bounds__(kEpiThreads) tapgemm_simt_kernel(const __grid_
 #pragma unroll
         for (int j = 0; j < 32; ++j) v[j] = 0.f;
         if (!(ni < P.nb && n < P.batch)) return;
-        const int rows_total = EPI == kEpiTopK ? P.n_codes : P.n_total;
+        const int rows_total = (EPI == kEpiTopK || EPI == kEpiMember) ? P.n_codes : P.n_total;
         const int jmax = rows_total - (tc.nblk * BN + ch * 32);
         for (int ti = 0; ti < pr.ntaps; ++ti) {
             const Tap tap = P.taps[pr.tap_begin + ti];
@@ -1567,6 +1598,7 @@ int launch_bn(const TapGemmParams& p, int num_sms, cudaStream_t stream) {
         case kEpiFwd: return launch_bn_epi<BN, kEpiFwd>(p, num_sms, stream);
         case kEpiBwd: return launch_bn_epi<BN, kEpiBwd>(p, num_sms, stream);
         case kEpiTopK: return launch_bn_epi<BN, kEpiTopK>(p, num_sms, stream);
+        case kEpiMember: return launch_bn_epi<BN, kEpiMember>(p, num_sms, stream);
         case kEpiStoreBf16: return launch_bn_epi<BN, kEpiStoreBf16>(p, num_sms, stream);
         case kEpiLinear: return launch_bn_epi<BN, kEpiLinear>(p, num_sms, stream);
         default: return static_cast<int>(cudaErrorInvalidValue);
@@ -1589,6 +1621,7 @@ int launch_simt_bn(const TapGemmParams& p, const TapSimtOperands& ops, cudaStrea
         case kEpiFwd: return launch_simt_bn_epi<BN, kEpiFwd>(p, ops, stream);
         case kEpiBwd: return launch_simt_bn_epi<BN, kEpiBwd>(p, ops, stream);
         case kEpiTopK: return launch_simt_bn_epi<BN, kEpiTopK>(p, ops, stream);
+        case kEpiMember: return launch_simt_bn_epi<BN, kEpiMember>(p, ops, stream);
         case kEpiStoreBf16: return launch_simt_bn_epi<BN, kEpiStoreBf16>(p, ops, stream);
         case kEpiLinear: return launch_simt_bn_epi<BN, kEpiLinear>(p, ops, stream);
         default: return static_cast<int>(cudaErrorInvalidValue);

@@ -57,6 +57,8 @@ enum TapEpilogue : int {
     kEpiStoreBf16 = 4, // store accumulators as bf16 (hi [+ lo]) into x_hi / x_lo [pixel][n_total]
     kEpiLinear = 5,    // plain (unmodulated) layers of the discriminator: r = acc (+ lin_add) -> lin_out;
                        // r * act'(lin_saved) -> lin_gz   (bf16 [pixel][n_total] tensors, each optional)
+    kEpiMember = 6,    // rows = probes, columns = manifold points: |y|^2 - 2<x,y> against T_j - |x|^2 -> definite-hit flag
+                       // per row, ambiguous columns appended to a bounded per-row list (precision / recall, DESIGN.md §12)
 };
 
 struct TapGemmParams {
@@ -141,6 +143,15 @@ struct TapGemmParams {
     int n_codes, n_queries, topk;      // topk = 2
     float* cand_score;                 // [n_queries][n_blocks * BN / 32][2]  ascending per 32-code chunk
     int* cand_idx;                     // [n_queries][n_blocks * BN / 32][2]  (-1 = empty)
+
+    // ---- kEpiMember: acc[probe, point] = <x, y>  (n_codes / n_queries as above)
+    const float4* member_tab;          // [n_codes] {|y_j|^2, T_j, per-column margin, 0}
+    const float* query_sqnorm;         // [n_queries] |x_i|^2
+    float member_eps;                  // per-row margin = member_eps * |x_i| * max_j |y_j| + 6e-7 (|x_i|^2 + max_j |y_j|^2)
+    int* member_hit;                   // [n_queries] set to 1 on a definite hit
+    int* member_cnt;                   // [n_queries] ambiguous columns seen (may exceed member_cap: the row overflowed)
+    int* member_list;                  // [n_queries][member_cap]
+    int member_cap;
 
     int* err_flag;
     unsigned long long* dbg_clock;     // optional [64]: CTA 0 cycles, nanoseconds and MMA-thread timeline stamps (LA_DBG_CLK experiments)

@@ -485,6 +485,67 @@ class LatentBank:
         return dist, idx
 
 
+class FeatureManifold:
+    """Device-resident feature manifold of the precision / recall metric (DESIGN.md §12): the features rounded to fp16
+    (held as fp32), their hi | lo bf16 planes and squared norms.  ``fallback`` is a device int32 counter to which every
+    call adds the queries that were scanned exhaustively."""
+
+    ROWS_PER_CALL = 8192          # bounds the per-call workspace (candidate lists, query planes): ~0.2 GB at 50 000 x 4096
+
+    def __init__(self, Y):
+        self.lib = _lib.load()
+        m = Y.shape[0]
+        self.Y = Y.detach().reshape(m, -1).to(torch.float16).float().contiguous()
+        self.m, self.K = m, self.Y.shape[1]
+        dev = self.Y.device
+        self.planes = torch.empty([2, m, self.K], dtype=torch.bfloat16, device=dev)
+        self.sqnorm = torch.empty([m + 1], device=dev)
+        self.fallback = torch.zeros([1], dtype=torch.int32, device=dev)
+        self._ws = None
+        with torch.cuda.device(dev):
+            _lib.check(self.lib.la_pr_manifold_prepare(_ptr(self.Y), m, self.K, _ptr(self.planes), _ptr(self.sqnorm), _stream_ptr(dev)))
+
+    def _workspace(self, nbytes):
+        if self._ws is None or self._ws.numel() < nbytes + 1024:
+            self._ws = torch.empty(nbytes + 1024, dtype=torch.uint8, device=self.Y.device)
+        return C.c_void_p((self._ws.data_ptr() + 1023) // 1024 * 1024)
+
+    def radii(self, begin=0, end=None, nhood_size=3):
+        """r2 [end - begin]: the (nhood+1)-th smallest squared distance of manifold rows [begin, end) over the manifold."""
+        end = self.m if end is None else end
+        dev = self.Y.device
+        r2 = torch.empty([end - begin], device=dev)
+        with torch.cuda.device(dev):
+            for b in range(begin, end, self.ROWS_PER_CALL):
+                n = min(self.ROWS_PER_CALL, end - b)
+                nbytes = C.c_size_t(0)
+                _lib.check(self.lib.la_pr_radii_workspace_bytes(n, self.m, self.K, nhood_size, C.byref(nbytes)))
+                ws = self._workspace(nbytes.value)
+                _lib.check(self.lib.la_pr_radii(C.c_void_p(self.Y.data_ptr() + b * self.K * 4), n, _ptr(self.Y), _ptr(self.planes),
+                                                _ptr(self.sqnorm), self.m, self.K, nhood_size, ws, nbytes.value,
+                                                C.c_void_p(r2.data_ptr() + (b - begin) * 4), _ptr(self.fallback), _stream_ptr(dev)))
+        return r2
+
+    def member(self, X, r2):
+        """uint8 [n]: 1 where probe i lies in some manifold ball, h(d2(x_i, y_j)) <= h(r2_j); r2 [m] from ``radii``."""
+        n = X.shape[0]
+        X = X.detach().reshape(n, -1).to(torch.float16).float().contiguous()
+        r2 = r2.float().contiguous()
+        assert X.shape[1] == self.K and r2.shape == (self.m,)
+        dev = self.Y.device
+        out = torch.empty([n], dtype=torch.uint8, device=dev)
+        with torch.cuda.device(dev):
+            for b in range(0, n, self.ROWS_PER_CALL):
+                c = min(self.ROWS_PER_CALL, n - b)
+                nbytes = C.c_size_t(0)
+                _lib.check(self.lib.la_pr_member_workspace_bytes(c, self.m, self.K, C.byref(nbytes)))
+                ws = self._workspace(nbytes.value)
+                _lib.check(self.lib.la_pr_member(C.c_void_p(X.data_ptr() + b * self.K * 4), c, _ptr(self.Y), _ptr(self.planes),
+                                                 _ptr(self.sqnorm), _ptr(r2), self.m, self.K, ws, nbytes.value,
+                                                 C.c_void_p(out.data_ptr() + b), _ptr(self.fallback), _stream_ptr(dev)))
+        return out
+
+
 def merge_topk(dist, idx):
     """[shards, n, k] -> [n, k] global k best (ties to the lowest index)."""
     lib = _lib.load()
