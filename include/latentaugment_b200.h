@@ -23,6 +23,8 @@
  *   la_nearest_codes      <- (north_star extension, SURVEY.md F3) argmin / top-k of that matrix
  *   la_project            <- StyleGAN2-ADA projector.py::project, batched, producing the inverted codes of --init_w inv
  *                            (DESIGN.md "Projection")
+ *   la_detector_features  <- the VGG16 fc7 embedding StyleGAN3's precision / recall feeds to compute_pr (pinned to
+ *                            torchvision's vgg16; DESIGN.md §13)
  */
 #ifndef LATENTAUGMENT_B200_H
 #define LATENTAUGMENT_B200_H
@@ -39,9 +41,10 @@ extern "C" {
 #define LA_MAX_MAPPING 8
 #define LA_MAX_STEPS 64            /* steps whose loss values are logged (the loop itself is not capped) */
 #define LA_LOSS_COLS 5             /* loss-log row: latent, pixel, total, discriminator, perceptual */
-#define LA_ABI_VERSION 202
+#define LA_ABI_VERSION 203
 
 typedef struct la_engine la_engine;
+typedef struct la_detector la_detector;
 typedef void* la_stream;          /* cudaStream_t */
 
 enum la_precision {
@@ -148,10 +151,22 @@ typedef struct la_vgg_desc {
                                                   (crop_size must be min(res, 256), res <= 512); 0: bank mode only */
 } la_vgg_desc;
 
+/* VGG16 detector of precision / recall (DESIGN.md §13): torchvision vgg16 `features` (same parameters as la_vgg_desc), the
+ * NCHW flatten, classifier.0 (fc6) + ReLU and classifier.3 (fc7) + ReLU. */
+typedef struct la_detector_desc {
+    const float* d_conv_weight[LA_VGG_CONVS];  /* [cout, cin, 3, 3] */
+    const float* d_conv_bias[LA_VGG_CONVS];    /* [cout] */
+    const float* d_fc6_weight;                 /* [4096, 25088] (input index c * 49 + h * 7 + w) */
+    const float* d_fc6_bias;                   /* [4096] */
+    const float* d_fc7_weight;                 /* [4096, 4096] */
+    const float* d_fc7_bias;                   /* [4096] */
+    float mean[3], std[3];                     /* per-channel normalisation of the 0..255 input: (v - mean) / std */
+} la_detector_desc;
+
 const char* la_last_error(void);
 /* ABI version (LA_ABI_VERSION) and sizeof of the structs passed by pointer, in the order la_generator_desc,
- * la_augment_options, la_disc_desc, la_conv_params, la_torgb_params, la_disc_block_params, la_vgg_desc (returns how many were
- * written, at most `max`): a binding checks both before the first call. */
+ * la_augment_options, la_disc_desc, la_conv_params, la_torgb_params, la_disc_block_params, la_vgg_desc, la_detector_desc
+ * (returns how many were written, at most `max`): a binding checks both before the first call. */
 int la_version(void);
 int la_struct_sizes(size_t* out, int max);
 
@@ -284,6 +299,18 @@ int la_pr_radii(const float* d_X, int n, const float* d_Y, const void* d_planes,
 int la_pr_member_workspace_bytes(int n, int m, int K, size_t* bytes);
 int la_pr_member(const float* d_X, int n, const float* d_Y, const void* d_planes, const float* d_sqnorm, const float* d_r2, int m, int K,
                  void* d_workspace, size_t workspace_bytes, unsigned char* d_member, int* d_fallback, la_stream stream);
+
+/* VGG16 detector embeddings (DESIGN.md §13).  A detector is independent of any engine: it owns a caller-provided workspace
+ * (1024-byte aligned) planned for at most `batch` images per call in `precision`; creation prepares the weights on `stream`
+ * (the weight tensors are not referenced afterwards; the bias tensors are read in place and must stay alive).
+ * la_detector_features: d_img [n, C, res, res] fp32 in [-1, 1], 1 <= n <= batch, 16 <= res <= 1024; per image, channel
+ * `modality` is quantised to 0..255 as StyleGAN3 saves images (clamp(x * 127.5 + 128, 0, 255) truncated), replicated to three
+ * channels, area-resized to 224^2, normalised, and embedded -> d_out [n, 4096] fp32 (the ReLU of fc7). */
+int la_detector_workspace_bytes(const la_detector_desc* d, int batch, int precision, size_t* bytes);
+int la_detector_create(const la_detector_desc* d, int batch, int precision, void* d_workspace, size_t workspace_bytes, la_stream stream,
+                       la_detector** out);
+void la_detector_destroy(la_detector* det);
+int la_detector_features(la_detector* det, const float* d_img, int n, int C, int res, int modality, float* d_out, la_stream stream);
 
 /* Test hooks: run every tap-GEMM of the engine once through the SIMT twin as well and report
  * the largest deviation (debug cross-check of the tensor-core path; not a product path). */

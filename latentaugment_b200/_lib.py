@@ -13,7 +13,7 @@ LA_MAX_MAPPING = 8
 LA_MAX_STEPS = 64
 LA_LOSS_COLS = 5
 LA_VGG_CONVS, LA_VGG_TAPS = 13, 5
-ABI_VERSION = 202          # == LA_ABI_VERSION of include/latentaugment_b200.h
+ABI_VERSION = 203          # == LA_ABI_VERSION of include/latentaugment_b200.h
 PRECISION = {'bf16': 0, 'fp32_parity': 1}
 NOISE = {'none': 0, 'const': 1, 'random': 2}
 
@@ -49,6 +49,11 @@ class AugmentOptions(C.Structure):
 class VggDesc(C.Structure):
     _fields_ = [('d_conv_weight', fptr * LA_VGG_CONVS), ('d_conv_bias', fptr * LA_VGG_CONVS), ('d_lin_weight', fptr * LA_VGG_TAPS),
                 ('mean', C.c_float * 3), ('std', C.c_float * 3), ('crop_size', C.c_int), ('per_sample_targets', C.c_int)]
+
+
+class DetectorDesc(C.Structure):
+    _fields_ = [('d_conv_weight', fptr * LA_VGG_CONVS), ('d_conv_bias', fptr * LA_VGG_CONVS), ('d_fc6_weight', fptr), ('d_fc6_bias', fptr),
+                ('d_fc7_weight', fptr), ('d_fc7_bias', fptr), ('mean', C.c_float * 3), ('std', C.c_float * 3)]
 
 
 class DiscBlockParams(C.Structure):
@@ -108,6 +113,10 @@ SIGNATURES = {
     'la_pr_member_workspace_bytes': (C.c_int, [C.c_int, C.c_int, C.c_int, C.POINTER(C.c_size_t)]),
     'la_pr_member': (C.c_int, [fptr, C.c_int, fptr, C.c_void_p, fptr, fptr, C.c_int, C.c_int, C.c_void_p, C.c_size_t, C.c_void_p,
                                C.c_void_p, C.c_void_p]),
+    'la_detector_workspace_bytes': (C.c_int, [C.POINTER(DetectorDesc), C.c_int, C.c_int, C.POINTER(C.c_size_t)]),
+    'la_detector_create': (C.c_int, [C.POINTER(DetectorDesc), C.c_int, C.c_int, C.c_void_p, C.c_size_t, C.c_void_p, C.POINTER(C.c_void_p)]),
+    'la_detector_destroy': (None, [C.c_void_p]),
+    'la_detector_features': (C.c_int, [C.c_void_p, fptr, C.c_int, C.c_int, C.c_int, C.c_int, fptr, C.c_void_p]),
     'la_debug_set_simt':(C.c_int, [C.c_void_p, C.c_int]),
     'la_debug_launch_count': (C.c_longlong, [C.c_void_p]),
     'la_debug_get': (C.c_int, [C.c_void_p, C.c_int, fptr, C.POINTER(C.c_size_t), C.c_void_p]),
@@ -145,7 +154,7 @@ def load():
                                  'rebuild with `python -m latentaugment_b200._build --force`')
     sizes = (C.c_size_t * 8)()
     n = lib.la_struct_sizes(sizes, 8)
-    mine = [C.sizeof(t) for t in (GeneratorDesc, AugmentOptions, DiscDesc, ConvParams, ToRgbParams, DiscBlockParams, VggDesc)]
+    mine = [C.sizeof(t) for t in (GeneratorDesc, AugmentOptions, DiscDesc, ConvParams, ToRgbParams, DiscBlockParams, VggDesc, DetectorDesc)]
     if n < len(mine) or list(sizes)[:len(mine)] != mine:
         raise LatentAugmentError(f'struct layout mismatch between {path} {list(sizes)[:n]} and the ctypes binding {mine}')
     _lib = lib

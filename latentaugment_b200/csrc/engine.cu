@@ -696,7 +696,8 @@ LA_API int la_version(void) { return LA_ABI_VERSION; }
 LA_API int la_struct_sizes(size_t* out, int max) {
     static_assert(kLossCols == LA_LOSS_COLS, "loss-log row width");
     const size_t v[] = {sizeof(la_generator_desc), sizeof(la_augment_options), sizeof(la_disc_desc), sizeof(la_conv_params),
-                        sizeof(la_torgb_params), sizeof(la_disc_block_params), sizeof(la_vgg_desc)};
+                        sizeof(la_torgb_params), sizeof(la_disc_block_params), sizeof(la_vgg_desc),
+                        sizeof(la_detector_desc)};
     int n = 0;
     for (; out && n < max && n < static_cast<int>(sizeof v / sizeof v[0]); ++n) out[n] = v[n];
     return n;

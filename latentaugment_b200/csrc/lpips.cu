@@ -23,6 +23,7 @@
 
 #include "plan.cuh"
 #include "tapgemm.cuh"
+#include "vgg.cuh"
 
 using namespace la;
 
@@ -53,10 +54,7 @@ int lfail(int code, const char* fmt, ...) {
 
 inline int cdiv(long long a, long long b) { return static_cast<int>((a + b - 1) / b); }
 
-constexpr int kNConv = LA_VGG_CONVS;
-const int kCout[kNConv] = {64, 64, 128, 128, 256, 256, 256, 512, 512, 512, 512, 512, 512};
-const int kCin[kNConv] = {3, 64, 64, 128, 128, 256, 256, 256, 512, 512, 512, 512, 512};
-const int kShift[kNConv] = {0, 0, 1, 1, 2, 2, 2, 3, 3, 3, 4, 4, 4};       // resolution = crop >> shift
+static_assert(kNConv == LA_VGG_CONVS, "VGG16 has 13 convolutions");
 const int kTapConv[LA_VGG_TAPS] = {1, 3, 6, 9, 12};                        // conv whose ReLU output is tap t (a pool follows 1, 3, 6, 9)
 
 __device__ __forceinline__ float warp_sum(float v) {
@@ -95,7 +93,8 @@ struct CallConsts {
 };
 
 // ------------------------------------------------------------------------- weights
-// w [cout, cin, 3, 3] fp32 -> wf [9][cout][cin_pad] and wb [9][cin_pad][cout] (zero padded); split: residual planes follow
+// w [cout, cin, 3, 3] fp32 -> wf [9][cout][cin_pad] and wb [9][cin_pad][cout] (zero padded; wb may be null); split: residual
+// planes follow
 __global__ void prep_vgg_weights_kernel(const float* __restrict__ w, int cout, int cin, int cin_pad, int split, bf16* wf, bf16* wb) {
     const long long idx = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x;
     const long long total = 9LL * cout * cin_pad;
@@ -105,7 +104,7 @@ __global__ void prep_vgg_weights_kernel(const float* __restrict__ w, int cout, i
     const int t = static_cast<int>(idx / (static_cast<long long>(cin_pad) * cout));
     const float v = i < cin ? w[(static_cast<long long>(o) * cin + i) * 9 + t] : 0.f;
     st_sp(wf, split ? wf + total : nullptr, idx, v);
-    st_sp(wb, split ? wb + total : nullptr, (static_cast<long long>(t) * cin_pad + i) * cout + o, v);
+    if (wb) st_sp(wb, split ? wb + total : nullptr, (static_cast<long long>(t) * cin_pad + i) * cout + o, v);
 }
 __global__ void fill_kernel(float* p, float v, long long n) {
     const long long i = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x;
@@ -379,7 +378,6 @@ struct Bump {
         return p;
     }
 };
-struct Pl { bf16* hi = nullptr; bf16* lo = nullptr; };
 struct Conv {
     int R, cin, cin_pad, cout;
     bf16 *wf, *wb;
@@ -421,18 +419,18 @@ inline int tap_grid(long long pixels, int num_sms) {
     return static_cast<int>(want < cap ? want : cap);
 }
 
-int dense_maps(const la_lpips* L, TapGemmParams& P, const Pl& t, int C, int R) {
+int dense_maps(int n, int split, TapGemmParams& P, const Pl& t, int C, int R) {
     const long long sW = C, sH = static_cast<long long>(R) * C, sN = sH * R;
-    if (make_a_map(&P.a_map[0], t.hi, C, R, R, L->ncrops, sW, sH, sN, P.tw, P.th + P.halo, P.nb)) return -1;
-    if (L->split && make_a_map(&P.a_map[1], t.lo, C, R, R, L->ncrops, sW, sH, sN, P.tw, P.th + P.halo, P.nb)) return -1;
+    if (make_a_map(&P.a_map[0], t.hi, C, R, R, n, sW, sH, sN, P.tw, P.th + P.halo, P.nb)) return -1;
+    if (split && make_a_map(&P.a_map[1], t.lo, C, R, R, n, sW, sH, sN, P.tw, P.th + P.halo, P.nb)) return -1;
     return 0;
 }
-int conv_taps(const la_lpips* L, TapGemmParams& P, bool flipped) {
+int conv_taps(int split, TapGemmParams& P, bool flipped) {
     int nt = 0;
     P.prob[0].tap_begin = 0;
     for (int t = 0; t < 9; ++t) {
         const int dy = t / 3 - 1, dx = t % 3 - 1;
-        add_tap(P, nt, flipped ? -dy : dy, flipped ? -dx : dx, t, 0, 1, 9, L->split);
+        add_tap(P, nt, flipped ? -dy : dy, flipped ? -dx : dx, t, 0, 1, 9, split);
     }
     P.prob[0].ntaps = nt;
     return tapgemm_finalize(P);
@@ -505,29 +503,12 @@ int build_lpips(la_lpips* L) {
         int pk = -1;
         for (int k = 0; k < 4; ++k) if (kTapConv[k] + 1 == i) { pooled_in = true; pk = k; }
         const Pl& in = i == 0 ? L->x_in : (pooled_in ? L->pool[pk] : L->conv[i - 1].x);
-        {   // forward: in -> x (ReLU)
-            TapGemmParams& P = c.F;
-            memset(&P, 0, sizeof P);
-            set_grid(P, c.R, L->ncrops, 1);
-            LLA(dense_maps(L, P, in, c.cin_pad, c.R));
-            const int bn = choose_bn(c.cout, P.m_tiles);
-            LLA(make_b_map(P, c.wf, c.cin_pad, c.cout, 9 * wm, bn));
-            P.kchunks = c.cin_pad / 64;
-            P.epilogue = kEpiFwd;
-            P.n_total = c.cout; P.n_blocks = c.cout / bn;
-            P.OH = P.OW = c.R; P.osy = P.osx = 1; P.split = split;
-            P.act_gain = 1.f; P.act_clamp = -1.f; P.act_slope = 0.f;           // ReLU
-            P.demod = L->ones; P.bias = L->d.d_conv_bias[i];
-            P.x_hi = c.x.hi; P.x_lo = c.x.lo;
-            P.staged = P.nb == 1 && !split && !getenv("LA_NO_STAGED");
-            P.err_flag = L->err_flag;
-            LLA(conv_taps(L, P, false));
-        }
+        LLA(vgg_conv_fwd_plan(c.F, c.R, L->ncrops, c.cin_pad, c.cout, in, c.wf, split, L->d.d_conv_bias[i], L->ones, c.x, L->err_flag));
         {   // data gradient: g_z (wrt this conv's pre-activation) -> gradient wrt its input
             TapGemmParams& P = c.B;
             memset(&P, 0, sizeof P);
             set_grid(P, c.R, L->ncrops, 1);
-            LLA(dense_maps(L, P, L->gz[i & 1], c.cout, c.R));
+            LLA(dense_maps(L->ncrops, split, P, L->gz[i & 1], c.cout, c.R));
             const int bn = choose_bn(c.cin_pad, P.m_tiles);
             LLA(make_b_map(P, c.wb, c.cout, c.cin_pad, 9 * wm, bn));
             P.kchunks = c.cout / 64;
@@ -539,7 +520,7 @@ int build_lpips(la_lpips* L) {
             else if (pooled_in) { P.lin_out = L->gp.hi; P.lin_out_lo = L->gp.lo; }
             else { P.lin_saved = L->conv[i - 1].x.hi; P.lin_gz = L->gz[(i - 1) & 1].hi; P.lin_gz_lo = L->gz[(i - 1) & 1].lo; }
             P.err_flag = L->err_flag;
-            LLA(conv_taps(L, P, true));
+            LLA(conv_taps(split, P, true));
         }
     }
     return 0;
@@ -549,9 +530,7 @@ int prepare_lpips(la_lpips* L, cudaStream_t s) {
     for (int i = 0; i <= L->last_conv; ++i) {
         Conv& c = L->conv[i];
         if (!L->d.d_conv_weight[i] || !L->d.d_conv_bias[i]) return lfail(-2, "lpips: missing parameters of conv %d", i);
-        const long long total = 9LL * c.cout * c.cin_pad;
-        prep_vgg_weights_kernel<<<cdiv(total, 256), 256, 0, s>>>(L->d.d_conv_weight[i], c.cout, c.cin, c.cin_pad, L->split, c.wf, c.wb);
-        LCU(cudaGetLastError());
+        LLA(vgg_prep_weights(L->d.d_conv_weight[i], c.cout, c.cin, c.cin_pad, L->split, c.wf, c.wb, s));
     }
     const long long n_ones = static_cast<long long>(L->ncrops) * 512;
     fill_kernel<<<cdiv(n_ones, 256), 256, 0, s>>>(L->ones, 1.f, n_ones);
@@ -575,9 +554,7 @@ int run_network(la_lpips* L, cudaStream_t s, long long* launches) {
         if (launches) ++*launches;
         for (int k = 0; k < 4; ++k)
             if (kTapConv[k] == i && i + 1 <= L->last_conv) {
-                const long long total = static_cast<long long>(L->ncrops) * (c.R / 2) * (c.R / 2) * (c.cout / 2);
-                pool_fwd_kernel<<<cdiv(total, 256), 256, 0, s>>>(CU32(c.x.hi), CU32(c.x.lo), L->ncrops, c.R, c.cout, U32(L->pool[k].hi), U32(L->pool[k].lo));
-                LCU(cudaGetLastError());
+                LLA(vgg_pool_fwd(c.x, L->ncrops, c.R, c.cout, L->pool[k], s));
                 if (launches) ++*launches;
             }
     }
@@ -589,6 +566,41 @@ int run_network(la_lpips* L, cudaStream_t s, long long* launches) {
 namespace la {
 
 const char* lpips_last_error() { return g_lerr.c_str(); }
+
+int vgg_prep_weights(const float* w, int cout, int cin, int cin_pad, int split, bf16* wf, bf16* wb, cudaStream_t s) {
+    const long long total = 9LL * cout * cin_pad;
+    prep_vgg_weights_kernel<<<cdiv(total, 256), 256, 0, s>>>(w, cout, cin, cin_pad, split, wf, wb);
+    LCU(cudaGetLastError());
+    return 0;
+}
+
+int vgg_conv_fwd_plan(TapGemmParams& P, int R, int n, int cin_pad, int cout, const Pl& in, const bf16* wf, int split, const float* bias,
+                      const float* ones, const Pl& out, int* err_flag) {
+    const int wm = split ? 2 : 1;
+    memset(&P, 0, sizeof P);
+    set_grid(P, R, n, 1);
+    LLA(dense_maps(n, split, P, in, cin_pad, R));
+    const int bn = choose_bn(cout, P.m_tiles);
+    LLA(make_b_map(P, wf, cin_pad, cout, 9 * wm, bn));
+    P.kchunks = cin_pad / 64;
+    P.epilogue = kEpiFwd;
+    P.n_total = cout; P.n_blocks = cout / bn;
+    P.OH = P.OW = R; P.osy = P.osx = 1; P.split = split;
+    P.act_gain = 1.f; P.act_clamp = -1.f; P.act_slope = 0.f;           // ReLU
+    P.demod = ones; P.bias = bias;
+    P.x_hi = out.hi; P.x_lo = out.lo;
+    P.staged = P.nb == 1 && !split && !getenv("LA_NO_STAGED");
+    P.err_flag = err_flag;
+    LLA(conv_taps(split, P, false));
+    return 0;
+}
+
+int vgg_pool_fwd(const Pl& x, int n, int R, int C, const Pl& out, cudaStream_t s) {
+    const long long total = static_cast<long long>(n) * (R / 2) * (R / 2) * (C / 2);
+    pool_fwd_kernel<<<cdiv(total, 256), 256, 0, s>>>(CU32(x.hi), CU32(x.lo), n, R, C, U32(out.hi), U32(out.lo));
+    LCU(cudaGetLastError());
+    return 0;
+}
 int lpips_has_bank(const la_lpips* L) { return L->has_bank; }
 int lpips_num_taps(const la_lpips* L) { return L->ntaps_used; }
 

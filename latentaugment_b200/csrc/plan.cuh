@@ -8,9 +8,10 @@
 namespace la {
 
 // M tile of a grid of resolution g: 16 rows x 8 pixels with a 2-row halo (the three vertical taps share
-// one TMA box) from 16^2 up; whole small images below that.
+// one TMA box) from 9^2 up (below 16^2 and at sizes that are not multiples of the tile the overhang is masked,
+// e.g. the 14^2 conv5 stage of a 224^2 VGG16); whole small images below that.
 inline void tile_geometry(int g, int& th, int& tw, int& nb, int& halo) {
-    if (g >= 16) { th = 16; tw = 8; nb = 1; halo = 2; }
+    if (g >= 9) { th = 16; tw = 8; nb = 1; halo = 2; }
     else if (g == 8) { th = 8; tw = 8; nb = 2; halo = 0; }
     else { th = g; tw = g; nb = 128 / (g * g); halo = 0; }
 }

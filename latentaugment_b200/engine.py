@@ -546,6 +546,75 @@ class FeatureManifold:
         return out
 
 
+IMAGENET_MEAN = tuple(255.0 * v for v in (0.485, 0.456, 0.406))     # torchvision's normalisation, in the 0..255 domain
+IMAGENET_STD = tuple(255.0 * v for v in (0.229, 0.224, 0.225))
+
+
+class FeatureDetector:
+    """VGG16 detector of precision / recall (DESIGN.md §13): torchvision ``vgg16`` up to the ReLU of fc7 on the GPU.
+
+    ``state``: torchvision names ``features.{i}.{weight,bias}`` and ``classifier.{0,3}.{weight,bias}`` (e.g.
+    ``torchvision.models.vgg16(...).state_dict()``).  ``batch``: images per call of the native detector (its workspace is
+    planned for that many); ``features`` walks any number of images in chunks of ``batch``.  ``mean`` / ``std``: per-channel
+    normalisation of the 0..255 input (default torchvision's ImageNet constants x 255)."""
+
+    VGG_CONV_IDX = SynthesisEngine.VGG_CONV_IDX
+    DIM = 4096
+
+    def __init__(self, state, batch=256, precision='bf16', mean=IMAGENET_MEAN, std=IMAGENET_STD, device=None):
+        self.lib = _lib.load()
+        self.device = torch.device(device) if device is not None else torch.device('cuda', torch.cuda.current_device())
+        self.batch, self.precision = int(batch), precision
+        keep = self._params = []
+
+        def dev(t):
+            t = torch.as_tensor(t).detach().to(self.device, torch.float32).contiguous()
+            keep.append(t)
+            return _ptr(t)
+        d = _lib.DetectorDesc()
+        for j, i in enumerate(self.VGG_CONV_IDX):
+            d.d_conv_weight[j] = dev(state[f'features.{i}.weight'])
+            d.d_conv_bias[j] = dev(state[f'features.{i}.bias'])
+        assert tuple(state['classifier.0.weight'].shape) == (4096, 25088) and tuple(state['classifier.3.weight'].shape) == (4096, 4096)
+        d.d_fc6_weight, d.d_fc6_bias = dev(state['classifier.0.weight']), dev(state['classifier.0.bias'])
+        d.d_fc7_weight, d.d_fc7_bias = dev(state['classifier.3.weight']), dev(state['classifier.3.bias'])
+        for k in range(3):
+            d.mean[k], d.std[k] = float(mean[k]), float(std[k])
+        prec = _lib.PRECISION[precision]
+        nbytes = C.c_size_t(0)
+        _lib.check(self.lib.la_detector_workspace_bytes(C.byref(d), self.batch, prec, C.byref(nbytes)))
+        self.workspace = torch.empty(nbytes.value + 1024, dtype=torch.uint8, device=self.device)
+        base = (self.workspace.data_ptr() + 1023) // 1024 * 1024
+        h = C.c_void_p()
+        with torch.cuda.device(self.device):
+            _lib.check(self.lib.la_detector_create(C.byref(d), self.batch, prec, C.c_void_p(base), nbytes.value, _stream_ptr(self.device),
+                                                   C.byref(h)))
+        self.handle = h
+        # only the biases are read in place; the prepared operands of the weights live in the workspace
+        self._params = [t for t in keep if t.dim() == 1]
+
+    def __del__(self):
+        h = getattr(self, 'handle', None)
+        if h:
+            torch.cuda.synchronize(self.device)
+            self.lib.la_detector_destroy(h)
+            self.handle = None
+
+    def features(self, img, modality=0):
+        """fp32 [n, 4096] on the detector's GPU: fc7 embeddings of channel ``modality`` of ``img`` [n, C, H, W] (H == W,
+        values in [-1, 1], on any device)."""
+        n, c, hh, ww = img.shape
+        assert hh == ww, img.shape
+        out = torch.empty([n, self.DIM], device=self.device)
+        with torch.cuda.device(self.device):
+            for b in range(0, n, self.batch):
+                e = min(n, b + self.batch)
+                x = img[b:e].detach().to(self.device, torch.float32).contiguous()
+                _lib.check(self.lib.la_detector_features(self.handle, _ptr(x), e - b, c, hh, int(modality), _ptr(out[b:e]),
+                                                         _stream_ptr(self.device)))
+        return out
+
+
 def merge_topk(dist, idx):
     """[shards, n, k] -> [n, k] global k best (ties to the lowest index)."""
     lib = _lib.load()

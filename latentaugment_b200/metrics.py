@@ -4,6 +4,8 @@
 fp16 as the reference rounds them; a manifold point's radius is its (nhood+1)-th smallest squared distance over the
 manifold (itself included); a probe counts when some manifold ball holds it under the reference's comparison of fp16
 distances.  Precision uses the real features as the manifold and the generated ones as probes; recall the reverse.
+``precision_recall_images`` takes images instead and embeds them with the VGG16 detector (``engine.FeatureDetector``,
+DESIGN.md §13) first.
 """
 import torch
 import torch.distributed as dist
@@ -54,3 +56,32 @@ def precision_recall(real_features, gen_features, nhood_size=3, group=None, stat
     if stats is not None:
         stats.update(fallback_precision=counts[2], fallback_recall=counts[3])
     return counts[0] / gen_features.shape[0], counts[1] / real_features.shape[0]
+
+
+def _embed(detector, images, modality, rank, world, group):
+    """[N, 4096] features of all ``images`` on every rank: each rank embeds its ``shard_range`` and one
+    all_gather_into_tensor of equal-sized pieces makes them whole."""
+    n = images.shape[0]
+    b, e = shard_range(n, rank, world)
+    f = detector.features(images[b:e], modality)
+    if world == 1:
+        return f
+    per = -(-n // world)
+    piece = torch.zeros([per, f.shape[1]], dtype=f.dtype, device=f.device)
+    piece[:e - b] = f
+    whole = torch.empty([world * per, f.shape[1]], dtype=f.dtype, device=f.device)
+    dist.all_gather_into_tensor(whole, piece, group=group)
+    return torch.cat([whole[k * per:k * per + shard_range(n, k, world)[1] - shard_range(n, k, world)[0]] for k in range(world)])
+
+
+def precision_recall_images(detector, real_img, gen_img, nhood_size=3, modality=0, group=None, stats=None):
+    """(precision, recall) of generated images against real images [N, C, H, W] in [-1, 1] (any device): channel
+    ``modality`` of both sets is embedded by ``detector`` (an ``engine.FeatureDetector``) and the features go to
+    ``precision_recall``.  With a process group each rank embeds its ``parallel.shard_range`` of each set and the features
+    are all-gathered (one collective per set) before the metric, which shards its own work as usual."""
+    distributed = group is not None or (dist.is_available() and dist.is_initialized())
+    world = dist.get_world_size(group) if distributed else 1
+    rank = dist.get_rank(group) if distributed else 0
+    real = _embed(detector, real_img, modality, rank, world, group)
+    gen = _embed(detector, gen_img, modality, rank, world, group)
+    return precision_recall(real, gen, nhood_size, group=group, stats=stats)
