@@ -10,59 +10,25 @@
 // torchvision's NCHW flatten order at preparation time.  fc7 stores raw fp32 accumulators and a small kernel adds the bias
 // and applies the ReLU, so the embedding is never rounded to bf16.
 #include <cuda_bf16.h>
-#include <stdarg.h>
-#include <stdio.h>
 #include <string.h>
 
 #include "../../include/latentaugment_b200.h"
-#include "lpips.cuh"
+#include "common.cuh"
+#include "kernels.cuh"
 #include "plan.cuh"
 #include "tapgemm.cuh"
 #include "vgg.cuh"
-
-int la_fail_msg(int code, const char* msg);   // engine.cu
 
 using namespace la;
 
 namespace {
 
+constexpr char kModule[] = "detector";
 typedef __nv_bfloat16 bf16;
 
 constexpr int kIn = 224;                  // detector input resolution
 constexpr int kPool5 = 7 * 7 * 512;       // fc6 fan-in
 constexpr int kFc = 4096;
-
-int dfail(int code, const char* fmt, ...) {
-    char buf[512];
-    va_list ap;
-    va_start(ap, fmt);
-    vsnprintf(buf, sizeof buf, fmt, ap);
-    va_end(ap);
-    return la_fail_msg(code ? code : -1, buf);
-}
-#define TCU(x)                                                                                               \
-    do {                                                                                                     \
-        cudaError_t e_ = (x);                                                                                \
-        if (e_ != cudaSuccess) return dfail(static_cast<int>(e_), "detector: %s: %s", #x, cudaGetErrorString(e_)); \
-    } while (0)
-#define TVGG(x)                                                                                              \
-    do {                                                                                                     \
-        int r_ = (x);                                                                                        \
-        if (r_) return dfail(r_, "detector: %s", lpips_last_error());                                        \
-    } while (0)
-#define TLA(x)                                                                                               \
-    do {                                                                                                     \
-        int r_ = (x);                                                                                        \
-        if (r_) return dfail(r_, "detector: %s failed (%d)", #x, r_);                                        \
-    } while (0)
-
-inline int cdiv(long long a, long long b) { return static_cast<int>((a + b - 1) / b); }
-
-__device__ __forceinline__ unsigned pack2(float a, float b) {
-    __nv_bfloat162 v = __floats2bfloat162_rn(a, b);
-    return *reinterpret_cast<unsigned*>(&v);
-}
-__device__ __forceinline__ float rnd(float v) { return __bfloat162float(__float2bfloat16_rn(v)); }
 
 struct Norm { float mean[3], std[3]; };
 
@@ -123,22 +89,6 @@ __global__ void bias_relu_kernel(const float* __restrict__ raw, const float* __r
     const long long i = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x;
     if (i < total) out[i] = fmaxf(raw[i] + __ldg(bias + i % N), 0.f);
 }
-__global__ void fill_ones_kernel(float* p, long long n) {
-    const long long i = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x;
-    if (i < n) p[i] = 1.f;
-}
-
-struct Bump {
-    char* base = nullptr;
-    size_t off = 0;
-    template <class T>
-    T* take(size_t count) {
-        off = (off + 1023) & ~size_t(1023);
-        T* p = base ? reinterpret_cast<T*>(base + off) : nullptr;
-        off += count * sizeof(T);
-        return p;
-    }
-};
 
 }  // namespace
 
@@ -158,13 +108,13 @@ struct la_detector {
 namespace {
 
 int validate(const la_detector_desc* d, int batch, int precision) {
-    if (!d || batch < 1) return dfail(-2, "detector: bad arguments");
-    if (precision != LA_PRECISION_BF16 && precision != LA_PRECISION_FP32_PARITY) return dfail(-2, "detector: unknown precision %d", precision);
+    if (!d || batch < 1) return fail(-2, "detector: bad arguments");
+    if (precision != LA_PRECISION_BF16 && precision != LA_PRECISION_FP32_PARITY) return fail(-2, "detector: unknown precision %d", precision);
     for (int i = 0; i < kNConv; ++i)
-        if (!d->d_conv_weight[i] || !d->d_conv_bias[i]) return dfail(-2, "detector: missing parameters of conv %d", i);
-    if (!d->d_fc6_weight || !d->d_fc6_bias || !d->d_fc7_weight || !d->d_fc7_bias) return dfail(-2, "detector: missing fc6 / fc7 parameters");
+        if (!d->d_conv_weight[i] || !d->d_conv_bias[i]) return fail(-2, "detector: missing parameters of conv %d", i);
+    if (!d->d_fc6_weight || !d->d_fc6_bias || !d->d_fc7_weight || !d->d_fc7_bias) return fail(-2, "detector: missing fc6 / fc7 parameters");
     for (int k = 0; k < 3; ++k)
-        if (!(d->std[k] > 0.f)) return dfail(-2, "detector: std[%d] must be positive", k);
+        if (!(d->std[k] > 0.f)) return fail(-2, "detector: std[%d] must be positive", k);
     return 0;
 }
 
@@ -212,7 +162,7 @@ int build_detector(la_detector* D) {
     int cur = 1;
     for (int i = 0; i < kNConv; ++i) {
         const int R = kIn >> kShift[i];
-        TVGG(vgg_conv_fwd_plan(D->conv[i], R, D->batch, (kCin[i] + 63) / 64 * 64, kCout[i], D->buf[cur], D->wconv[i], D->split, D->d.d_conv_bias[i],
+        LA(vgg_conv_fwd_plan(D->conv[i], R, D->batch, (kCin[i] + 63) / 64 * 64, kCout[i], D->buf[cur], D->wconv[i], D->split, D->d.d_conv_bias[i],
                                D->ones, D->buf[cur ^ 1], D->err_flag));
         cur ^= 1;
         for (int k = 0; k < 5; ++k) if (kPoolConv[k] == i) cur ^= 1;
@@ -220,14 +170,14 @@ int build_detector(la_detector* D) {
     D->pool5 = cur;
     {   // fc6 + ReLU -> h6 (bf16, the A operand of fc7)
         TapGemmParams& P = D->fc6;
-        TLA(dense_layer(D, P, D->buf[cur], kPool5, D->w6));
+        LA(dense_layer(D, P, D->buf[cur], kPool5, D->w6));
         P.epilogue = kEpiFwd;
         P.demod = D->ones; P.bias = D->d.d_fc6_bias;
         P.x_hi = D->h6.hi; P.x_lo = D->h6.lo;
     }
     {   // fc7 -> raw fp32 accumulators (bias + ReLU follow)
         TapGemmParams& P = D->fc7;
-        TLA(dense_layer(D, P, D->h6, kFc, D->w7));
+        LA(dense_layer(D, P, D->h6, kFc, D->w7));
         P.epilogue = kEpiRawF32;
         P.raw_out = D->raw7;
     }
@@ -236,16 +186,15 @@ int build_detector(la_detector* D) {
 
 int prepare_detector(la_detector* D, cudaStream_t s) {
     for (int i = 0; i < kNConv; ++i)
-        TVGG(vgg_prep_weights(D->d.d_conv_weight[i], kCout[i], kCin[i], (kCin[i] + 63) / 64 * 64, D->split, D->wconv[i], nullptr, s));
+        LA(vgg_prep_weights(D->d.d_conv_weight[i], kCout[i], kCin[i], (kCin[i] + 63) / 64 * 64, D->split, D->wconv[i], nullptr, s));
     prep_dense_kernel<<<cdiv(static_cast<long long>(kFc) * kPool5, 256), 256, 0, s>>>(D->d.d_fc6_weight, kFc, kPool5, 512, D->split, D->w6);
-    TCU(cudaGetLastError());
+    CU(cudaGetLastError());
     prep_dense_kernel<<<cdiv(static_cast<long long>(kFc) * kFc, 256), 256, 0, s>>>(D->d.d_fc7_weight, kFc, kFc, 0, D->split, D->w7);
-    TCU(cudaGetLastError());
+    CU(cudaGetLastError());
     const long long n_ones = static_cast<long long>(D->batch) * kFc;
-    fill_ones_kernel<<<cdiv(n_ones, 256), 256, 0, s>>>(D->ones, n_ones);
-    TCU(cudaGetLastError());
-    TCU(cudaMemsetAsync(D->err_flag, 0, sizeof(int), s));
-    TCU(cudaStreamSynchronize(s));
+    LA(fill(D->ones, 1.f, n_ones, s));
+    CU(cudaMemsetAsync(D->err_flag, 0, sizeof(int), s));
+    CU(cudaStreamSynchronize(s));
     return 0;
 }
 
@@ -255,7 +204,7 @@ int prepare_detector(la_detector* D, cudaStream_t s) {
 extern "C" {
 
 LA_API int la_detector_workspace_bytes(const la_detector_desc* d, int batch, int precision, size_t* bytes) {
-    if (!bytes) return dfail(-2, "detector: bad arguments");
+    if (!bytes) return fail(-2, "detector: bad arguments");
     if (int r = validate(d, batch, precision)) return r;
     la_detector* tmp = new la_detector{};
     tmp->batch = batch; tmp->split = precision == LA_PRECISION_FP32_PARITY;
@@ -266,20 +215,16 @@ LA_API int la_detector_workspace_bytes(const la_detector_desc* d, int batch, int
 
 LA_API int la_detector_create(const la_detector_desc* d, int batch, int precision, void* d_workspace, size_t workspace_bytes, la_stream stream,
                               la_detector** out) {
-    if (!out || !d_workspace) return dfail(-2, "detector: bad arguments");
+    if (!out || !d_workspace) return fail(-2, "detector: bad arguments");
     if (int r = validate(d, batch, precision)) return r;
-    if (reinterpret_cast<uintptr_t>(d_workspace) & 1023) return dfail(-2, "detector: workspace must be 1024-byte aligned");
     la_detector* D = new la_detector{};
     D->d = *d; D->batch = batch; D->split = precision == LA_PRECISION_FP32_PARITY;
     const size_t need = plan_detector(D, static_cast<char*>(d_workspace));
-    if (workspace_bytes < need) {
-        delete D;
-        return dfail(-2, "detector: workspace too small: %zu < %zu", workspace_bytes, need);
-    }
+    if (int r = check_workspace(kModule, need, workspace_bytes, d_workspace)) { delete D; return r; }
     int dev = 0;
     int r = static_cast<int>(cudaGetDevice(&dev));
     if (!r) r = static_cast<int>(cudaDeviceGetAttribute(&D->num_sms, cudaDevAttrMultiProcessorCount, dev));
-    if (r) { delete D; return dfail(r, "detector: %s", cudaGetErrorString(static_cast<cudaError_t>(r))); }
+    if (r) { delete D; return fail(r, "detector: %s", cudaGetErrorString(static_cast<cudaError_t>(r))); }
     r = build_detector(D);
     if (!r) r = prepare_detector(D, static_cast<cudaStream_t>(stream));
     if (r) { delete D; return r; }
@@ -290,31 +235,31 @@ LA_API int la_detector_create(const la_detector_desc* d, int batch, int precisio
 LA_API void la_detector_destroy(la_detector* det) { delete det; }
 
 LA_API int la_detector_features(la_detector* D, const float* d_img, int n, int C, int res, int modality, float* d_out, la_stream stream) {
-    if (!D || !d_img || !d_out) return dfail(-2, "detector: bad arguments");
-    if (n < 1 || n > D->batch) return dfail(-2, "detector: n = %d outside 1..%d (the planned batch)", n, D->batch);
-    if (C < 1 || modality < 0 || modality >= C) return dfail(-2, "detector: modality %d outside 0..%d", modality, C - 1);
-    if (res < 16 || res > 1024) return dfail(-2, "detector: resolution %d outside 16..1024", res);
+    if (!D || !d_img || !d_out) return fail(-2, "detector: bad arguments");
+    if (n < 1 || n > D->batch) return fail(-2, "detector: n = %d outside 1..%d (the planned batch)", n, D->batch);
+    if (C < 1 || modality < 0 || modality >= C) return fail(-2, "detector: modality %d outside 0..%d", modality, C - 1);
+    if (res < 16 || res > 1024) return fail(-2, "detector: resolution %d outside 16..1024", res);
     cudaStream_t s = static_cast<cudaStream_t>(stream);
     Norm z;
     for (int k = 0; k < 3; ++k) { z.mean[k] = D->d.mean[k]; z.std[k] = D->d.std[k]; }
     const long long npx = static_cast<long long>(n) * kIn * kIn;
     detector_input_kernel<<<cdiv(npx, 256), 256, 0, s>>>(d_img, n, C, res, modality, z, D->buf[1].hi, D->buf[1].lo);
-    TCU(cudaGetLastError());
+    CU(cudaGetLastError());
     int cur = 1;
     for (int i = 0; i < kNConv; ++i) {
-        TLA(launch_tapgemm(D->conv[i], D->num_sms, s));
+        LA(launch_tapgemm(D->conv[i], D->num_sms, s));
         cur ^= 1;
         for (int k = 0; k < 5; ++k)
             if (kPoolConv[k] == i) {
-                TVGG(vgg_pool_fwd(D->buf[cur], n, kIn >> kShift[i], kCout[i], D->buf[cur ^ 1], s));
+                LA(vgg_pool_fwd(D->buf[cur], n, kIn >> kShift[i], kCout[i], D->buf[cur ^ 1], s));
                 cur ^= 1;
             }
     }
-    TLA(launch_tapgemm(D->fc6, D->num_sms, s));
-    TLA(launch_tapgemm(D->fc7, D->num_sms, s));
+    LA(launch_tapgemm(D->fc6, D->num_sms, s));
+    LA(launch_tapgemm(D->fc7, D->num_sms, s));
     const long long total = static_cast<long long>(n) * kFc;
     bias_relu_kernel<<<cdiv(total, 256), 256, 0, s>>>(D->raw7, D->d.d_fc7_bias, total, kFc, d_out);
-    TCU(cudaGetLastError());
+    CU(cudaGetLastError());
     return 0;
 }
 

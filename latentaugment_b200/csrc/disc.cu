@@ -14,14 +14,12 @@
 
 #include <cuda_bf16.h>
 #include <math.h>
-#include <stdarg.h>
-#include <stdio.h>
 #include <string.h>
 
-#include <string>
 #include <vector>
 
 #include "act.cuh"
+#include "common.cuh"
 #include "kernels.cuh"
 #include "plan.cuh"
 #include "tapgemm.cuh"
@@ -30,78 +28,15 @@ using namespace la;
 
 namespace {
 
+constexpr char kModule[] = "discriminator";
 typedef __nv_bfloat16 bf16;
-thread_local std::string g_derr;
 
-int dfail(int code, const char* fmt, ...) {
-    char buf[512];
-    va_list ap;
-    va_start(ap, fmt);
-    vsnprintf(buf, sizeof buf, fmt, ap);
-    va_end(ap);
-    g_derr = buf;
-    return code ? code : -1;
-}
-#define DCU(x)                                                                                               \
-    do {                                                                                                     \
-        cudaError_t e_ = (x);                                                                                \
-        if (e_ != cudaSuccess) return dfail(static_cast<int>(e_), "%s: %s (%s:%d)", #x, cudaGetErrorString(e_), __FILE__, __LINE__); \
-    } while (0)
-#define DLA(x)                                                                                               \
-    do {                                                                                                     \
-        int r_ = (x);                                                                                        \
-        if (r_) return dfail(r_, "%s failed (%d) (%s:%d)", #x, r_, __FILE__, __LINE__);                      \
-    } while (0)
-
-inline int cdiv(long long a, long long b) { return static_cast<int>((a + b - 1) / b); }
-
-__device__ __forceinline__ float warp_sum(float v) {
-#pragma unroll
-    for (int o = 16; o >= 1; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-    return v;
-}
-__device__ __forceinline__ unsigned pack2(float a, float b) {
-    __nv_bfloat162 v = __floats2bfloat162_rn(a, b);
-    return *reinterpret_cast<unsigned*>(&v);
-}
-__device__ __forceinline__ float lo_f(unsigned u) { return __uint_as_float(u << 16); }
-__device__ __forceinline__ float hi_f(unsigned u) { return __uint_as_float(u & 0xffff0000u); }
-// value of element i of a (hi [, lo]) bf16 pair / pair store
-__device__ __forceinline__ float ld_sp(const bf16* hi, const bf16* lo, long long i) {
-    float v = __bfloat162float(hi[i]);
-    if (lo) v += __bfloat162float(lo[i]);
-    return v;
-}
-__device__ __forceinline__ void st_sp(bf16* hi, bf16* lo, long long i, float v) {
-    const bf16 h = __float2bfloat16_rn(v);
-    hi[i] = h;
-    if (lo) lo[i] = __float2bfloat16_rn(v - __bfloat162float(h));
-}
-__device__ __forceinline__ void st_sp2(unsigned* hi, unsigned* lo, long long i, float a, float b) {
-    hi[i] = pack2(a, b);
-    if (lo) lo[i] = pack2(a - __bfloat162float(__float2bfloat16_rn(a)), b - __bfloat162float(__float2bfloat16_rn(b)));
-}
 __device__ __forceinline__ float act_fwd(float z, float gain, float slope, float clamp) {
     z = (z > 0.f ? z : z * slope) * gain;
     return clamp >= 0.f ? fminf(fmaxf(z, -clamp), clamp) : z;
 }
 
 // ------------------------------------------------------------------------- weight preparation
-// w [cout, cin, k, k] fp32 -> wf [k*k][cout][cin_pad] and wb [k*k][cin_pad][cout], both * scale, zero padded;
-// with split the bf16 residual planes follow as a second stack of k*k matrices
-__global__ void prep_plain_weights_kernel(const float* __restrict__ w, int cout, int cin, int k2, float scale, int cin_pad, int split,
-                                          bf16* wf, bf16* wb) {
-    const long long idx = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x;
-    const long long total = static_cast<long long>(k2) * cout * cin_pad;
-    if (idx >= total) return;
-    const int i = static_cast<int>(idx % cin_pad);
-    const int o = static_cast<int>((idx / cin_pad) % cout);
-    const int t = static_cast<int>(idx / (static_cast<long long>(cin_pad) * cout));
-    const float v = i < cin ? w[(static_cast<long long>(o) * cin + i) * k2 + t] * scale : 0.f;
-    const long long bidx = (static_cast<long long>(t) * cin_pad + i) * cout + o;
-    st_sp(wf, split ? wf + total : nullptr, idx, v);
-    st_sp(wb, split ? wb + total : nullptr, bidx, v);
-}
 // dense [C, 16*C] over the NCHW flatten (index c*16 + hw) -> wf [16][C(o)][C(c)], wb [16*C (hw, c)][C(o)]
 __global__ void prep_fc_weights_kernel(const float* __restrict__ w, int C, float scale, int split, bf16* wf, bf16* wb) {
     const long long idx = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x;
@@ -121,10 +56,6 @@ __global__ void prep_rgb_w4_kernel(const float* __restrict__ w, int C, int imgc,
     w4[4 * c + 1] = imgc > 1 ? w[c * imgc + 1] * wg : 0.f;
     w4[4 * c + 2] = imgc > 2 ? w[c * imgc + 2] * wg : 0.f;
     w4[4 * c + 3] = 0.f;
-}
-__global__ void fill_kernel(float* p, float v, long long n) {
-    const long long i = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x;
-    if (i < n) p[i] = v;
 }
 
 // ------------------------------------------------------------------------- image layout
@@ -337,23 +268,6 @@ __global__ void out_bwd_kernel(const float* __restrict__ gl, const float* __rest
     st_sp(gz6, gz6_lo, idx, act_grad(gl[n] * w[c] * wg * gain, __bfloat162float(x6[idx]), slope, act_saved_clamp(-1.f, false)));
 }
 
-struct Bump {
-    char* base = nullptr;
-    size_t off = 0;
-    template <class T>
-    T* take(size_t count) {
-        off = (off + 1023) & ~size_t(1023);
-        T* p = base ? reinterpret_cast<T*>(base + off) : nullptr;
-        off += count * sizeof(T);
-        return p;
-    }
-};
-
-struct Pl {                 // a bf16 tensor as (hi [, lo]) planes; lo only in split (fp32_parity) precision
-    bf16* hi = nullptr;
-    bf16* lo = nullptr;
-};
-
 struct Block {
     int R, C, Cn;
     la_disc_block_params p;
@@ -403,25 +317,16 @@ void lin_epi(TapGemmParams& P, const la_disc* D, int n_total, int bn, int oh, in
     P.OH = oh; P.OW = ow; P.osy = P.osx = 1; P.split = D->split;
     P.act_gain = 1.f; P.act_clamp = -1.f; P.act_slope = 0.2f;
 }
-int choose_bn(int n, long long m_tiles) { return n % 128 ? 64 : pick_bn(n, m_tiles); }
-
-// A map(s) of a dense NHWC tensor [B, H, W, C]: map `slot` = hi plane, `slot + lo_slot` = lo plane
-int dense_maps(const la_disc* D, TapGemmParams& P, int slot, int lo_slot, const Pl& t, int C, int W, int H, int tw, int th, int nb) {
-    const long long sW = C, sH = static_cast<long long>(W) * C, sN = sH * H;
-    if (make_a_map(&P.a_map[slot], t.hi, C, W, H, D->batch, sW, sH, sN, tw, th, nb)) return -1;
-    if (D->split && make_a_map(&P.a_map[slot + lo_slot], t.lo, C, W, H, D->batch, sW, sH, sN, tw, th, nb)) return -1;
-    return 0;
-}
 
 int plan_disc(la_disc* D, char* ws, size_t* bytes_out) {
     const la_disc_desc& d = D->d;
     const int B = D->batch, split = D->split;
     if (d.num_blocks < 1 || d.num_blocks + 1 > LA_MAX_BLOCKS || (8 << (d.num_blocks - 1)) != d.img_resolution)
-        return dfail(-2, "discriminator: img_resolution %d does not match num_blocks %d", d.img_resolution, d.num_blocks);
-    if (d.img_channels < 1 || d.img_channels > 3) return dfail(-2, "discriminator: img_channels must be 1..3");
-    if (d.mbstd_group_size < 1 || d.mbstd_group_size > 8) return dfail(-2, "discriminator: mbstd_group_size must be 1..8");
+        return fail(-2, "discriminator: img_resolution %d does not match num_blocks %d", d.img_resolution, d.num_blocks);
+    if (d.img_channels < 1 || d.img_channels > 3) return fail(-2, "discriminator: img_channels must be 1..3");
+    if (d.mbstd_group_size < 1 || d.mbstd_group_size > 8) return fail(-2, "discriminator: mbstd_group_size must be 1..8");
     for (int b = 0; b <= d.num_blocks; ++b)
-        if (d.channels[b] % 64 || d.channels[b] < 64 || d.channels[b] > 1024) return dfail(-2, "discriminator: channels[%d]=%d unsupported", b, d.channels[b]);
+        if (d.channels[b] % 64 || d.channels[b] < 64 || d.channels[b] > 1024) return fail(-2, "discriminator: channels[%d]=%d unsupported", b, d.channels[b]);
     Bump bp;
     bp.base = ws;
     auto take_pl = [&](size_t n) { Pl t; t.hi = bp.take<bf16>(n); t.lo = split ? bp.take<bf16>(n) : nullptr; return t; };
@@ -502,13 +407,13 @@ int build_disc(la_disc* D) {
             TapGemmParams& P = k.F0;
             memset(&P, 0, sizeof P);
             set_grid(P, R, B, 1);
-            DLA(dense_maps(D, P, 0, 1, k.x_in, C, R, R, P.tw, P.th + P.halo, P.nb));
+            LA(dense_maps(P, k.x_in, D->batch, C, R, R, P.tw, P.th + P.halo, P.nb, D->split));
             const int bn = choose_bn(C, P.m_tiles);
-            DLA(make_b_map(P, k.w0f, C, C, 9 * wm, bn));
+            LA(make_b_map(P, k.w0f, C, C, 9 * wm, bn));
             P.kchunks = C / 64;
             fwd_epi(P, D, k.p.d_conv0_bias, k.x0, kSqrt2, clamp, C, bn, R);
             P.err_flag = D->err_flag;
-            DLA(conv_taps(D, P, false));
+            LA(conv_taps(D, P, false));
         }
         // ---- blur (pad 2): x0 -> yb, and its adjoint fused with conv0's activation gradient: g_yb -> g_z0
         {
@@ -541,7 +446,7 @@ int build_disc(la_disc* D) {
                 r |= encode_tmap_bf16(&U.fwd_out_x, D->g_z0.hi, 4, ydims, ystr, sbox, 0);
                 r |= encode_tmap_bf16(&U.bwd_in, k.x0.hi, 4, ydims, ystr, lbox, 0);
                 r |= encode_tmap_bf16(&U.bwd_out, D->yb.hi, 4, tdims, tstr, sbox, 0);
-                if (r) return dfail(-5, "tensor map encoding failed (discriminator blur)");
+                if (r) return fail(-5, "tensor map encoding failed (discriminator blur)");
                 U.use_tma = 1;
             }
         }
@@ -555,8 +460,8 @@ int build_disc(la_disc* D) {
                 const int py = ph / 2, px = ph % 2;
                 const int ph_h = Ro + (py == 0), ph_w = Ro + (px == 0);
                 const long long off = (static_cast<long long>(py) * TWp + px) * C;
-                DLA(make_a_map(&P.a_map[ph], D->yb.hi + off, C, ph_w, ph_h, B, gW, gH, gN, P.tw, P.th + P.halo, P.nb));
-                if (split) DLA(make_a_map(&P.a_map[4 + ph], D->yb.lo + off, C, ph_w, ph_h, B, gW, gH, gN, P.tw, P.th + P.halo, P.nb));
+                LA(make_a_map(&P.a_map[ph], D->yb.hi + off, C, ph_w, ph_h, B, gW, gH, gN, P.tw, P.th + P.halo, P.nb));
+                if (split) LA(make_a_map(&P.a_map[4 + ph], D->yb.lo + off, C, ph_w, ph_h, B, gW, gH, gN, P.tw, P.th + P.halo, P.nb));
             }
             int nt = 0;
             for (int a = 0; a < 3; ++a)
@@ -566,39 +471,39 @@ int build_disc(la_disc* D) {
                 }
             P.prob[0].tap_begin = 0; P.prob[0].ntaps = nt;
             const int bn = choose_bn(Cn, P.m_tiles);
-            DLA(make_b_map(P, k.w1f, C, Cn, 9 * wm, bn));
+            LA(make_b_map(P, k.w1f, C, Cn, 9 * wm, bn));
             P.kchunks = C / 64;
             fwd_epi(P, D, k.p.d_conv1_bias, k.y1, kSqrt2 * kSqrtHalf, clamp >= 0.f ? clamp * kSqrtHalf : clamp, Cn, bn, Ro);
             P.err_flag = D->err_flag;
-            DLA(tapgemm_finalize(P));
+            LA(tapgemm_finalize(P));
         }
         // ---- skip forward: 1x1 on the decimated blur, + y1 -> y
         {
             TapGemmParams& P = k.FS;
             memset(&P, 0, sizeof P);
             set_grid(P, Ro, B, 1);
-            DLA(dense_maps(D, P, 0, 1, D->ys, C, Ro, Ro, P.tw, P.th + P.halo, P.nb));
+            LA(dense_maps(P, D->ys, D->batch, C, Ro, Ro, P.tw, P.th + P.halo, P.nb, D->split));
             const int bn = choose_bn(Cn, P.m_tiles);
-            DLA(make_b_map(P, k.wsf, C, Cn, wm, bn));
+            LA(make_b_map(P, k.wsf, C, Cn, wm, bn));
             P.kchunks = C / 64;
             lin_epi(P, D, Cn, bn, Ro, Ro);
             P.lin_add = k.y1.hi; P.lin_add_lo = k.y1.lo; P.lin_out = k.y.hi; P.lin_out_lo = k.y.lo;
             P.err_flag = D->err_flag;
-            DLA(one_tap(D, P));
+            LA(one_tap(D, P));
         }
         // ---- skip backward: g_ys = Ws^T g_y
         {
             TapGemmParams& P = k.BS;
             memset(&P, 0, sizeof P);
             set_grid(P, Ro, B, 1);
-            DLA(dense_maps(D, P, 0, 1, k.g_y, Cn, Ro, Ro, P.tw, P.th + P.halo, P.nb));
+            LA(dense_maps(P, k.g_y, D->batch, Cn, Ro, Ro, P.tw, P.th + P.halo, P.nb, D->split));
             const int bn = choose_bn(C, P.m_tiles);
-            DLA(make_b_map(P, k.wsb, Cn, C, wm, bn));
+            LA(make_b_map(P, k.wsb, Cn, C, wm, bn));
             P.kchunks = Cn / 64;
             lin_epi(P, D, C, bn, Ro, Ro);
             P.lin_out = D->g_ys.hi; P.lin_out_lo = D->g_ys.lo;
             P.err_flag = D->err_flag;
-            DLA(one_tap(D, P));
+            LA(one_tap(D, P));
         }
         // ---- conv1 backward: transposed stride-2 convolution, g_z1 -> g_yb (four output phases)
         {
@@ -606,7 +511,7 @@ int build_disc(la_disc* D) {
             memset(&P, 0, sizeof P);
             const int gh[4] = {Ro + 1, Ro + 1, Ro, Ro}, gw[4] = {Ro + 1, Ro, Ro + 1, Ro};
             set_grid(P, Ro, B, 4, gh, gw);
-            DLA(dense_maps(D, P, 0, 1, k.g_z1, Cn, Ro, Ro, P.tw, P.th + P.halo, P.nb));
+            LA(dense_maps(P, k.g_z1, D->batch, Cn, Ro, Ro, P.tw, P.th + P.halo, P.nb, D->split));
             int nt = 0;
             for (int ph = 0; ph < 4; ++ph) {
                 P.prob[ph].tap_begin = nt;
@@ -616,22 +521,22 @@ int build_disc(la_disc* D) {
                 P.prob[ph].oy0 = ph / 2; P.prob[ph].ox0 = ph % 2;
             }
             const int bn = choose_bn(C, P.m_tiles);
-            DLA(make_b_map(P, k.w1b, Cn, C, 9 * wm, bn));
+            LA(make_b_map(P, k.w1b, Cn, C, 9 * wm, bn));
             P.kchunks = Cn / 64; P.n_total = C; P.n_blocks = C / bn;
             P.epilogue = kEpiStoreBf16; P.OH = TH; P.OW = TWp; P.osy = P.osx = 2; P.split = split;
             P.x_hi = D->g_yb.hi; P.x_lo = D->g_yb.lo;
             P.staged = P.nb == 1 && !split && !getenv("LA_NO_STAGED");
             P.err_flag = D->err_flag;
-            DLA(tapgemm_finalize(P));
+            LA(tapgemm_finalize(P));
         }
         // ---- conv0 backward: g_z0 -> (+ skip-branch gradient) -> gradient wrt the block input, raw and through the producer's activation
         {
             TapGemmParams& P = k.B0;
             memset(&P, 0, sizeof P);
             set_grid(P, R, B, 1);
-            DLA(dense_maps(D, P, 0, 1, D->g_z0, C, R, R, P.tw, P.th + P.halo, P.nb));
+            LA(dense_maps(P, D->g_z0, D->batch, C, R, R, P.tw, P.th + P.halo, P.nb, D->split));
             const int bn = choose_bn(C, P.m_tiles);
-            DLA(make_b_map(P, k.w0b, C, C, 9 * wm, bn));
+            LA(make_b_map(P, k.w0b, C, C, 9 * wm, bn));
             P.kchunks = C / 64;
             lin_epi(P, D, C, bn, R, R);
             P.lin_add_down = D->g_ys.hi; P.lin_add_down_lo = D->g_ys.lo;      // FIRdown^T(g_ys) is evaluated inside the epilogue
@@ -645,7 +550,7 @@ int build_disc(la_disc* D) {
                 P.act_gain = kSqrt2 * kSqrtHalf; P.act_clamp = clamp >= 0.f ? clamp * kSqrtHalf : clamp;
             }
             P.err_flag = D->err_flag;
-            DLA(conv_taps(D, P, true));
+            LA(conv_taps(D, P, true));
         }
     }
     // ------------------------------------------------------------------ 4x4 epilogue
@@ -654,13 +559,13 @@ int build_disc(la_disc* D) {
         TapGemmParams& P = D->FE;
         memset(&P, 0, sizeof P);
         set_grid(P, 4, B, 1);
-        DLA(dense_maps(D, P, 0, 1, D->x4p, Cp, 4, 4, P.tw, P.th + P.halo, P.nb));
+        LA(dense_maps(P, D->x4p, D->batch, Cp, 4, 4, P.tw, P.th + P.halo, P.nb, D->split));
         const int bn = choose_bn(C4, P.m_tiles);
-        DLA(make_b_map(P, D->wef, Cp, C4, 9 * wm, bn));
+        LA(make_b_map(P, D->wef, Cp, C4, 9 * wm, bn));
         P.kchunks = Cp / 64;
         fwd_epi(P, D, d.d_b4_conv_bias, D->x5, kSqrt2, d.conv_clamp, C4, bn, 4);
         P.err_flag = D->err_flag;
-        DLA(conv_taps(D, P, false));
+        LA(conv_taps(D, P, false));
     }
     auto sample_rows = [&](TapGemmParams& P) {        // M rows = samples: 128 samples x one pixel per tile
         P.th = 1; P.tw = 1; P.nb = 128; P.halo = 0;
@@ -672,44 +577,44 @@ int build_disc(la_disc* D) {
         TapGemmParams& P = D->FF;
         memset(&P, 0, sizeof P);
         sample_rows(P);
-        DLA(dense_maps(D, P, 0, 1, D->x5, C4, 4, 4, 1, 1, 128));
+        LA(dense_maps(P, D->x5, D->batch, C4, 4, 4, 1, 1, 128, D->split));
         int nt = 0;
         for (int hw = 0; hw < 16; ++hw) add_tap(P, nt, hw / 4, hw % 4, hw, 0, 1, 16, split);
         P.prob[0].tap_begin = 0; P.prob[0].ntaps = nt;
         const int bn = 64;
-        DLA(make_b_map(P, D->wff, C4, C4, 16 * wm, bn));
+        LA(make_b_map(P, D->wff, C4, C4, 16 * wm, bn));
         P.kchunks = C4 / 64;
         fwd_epi(P, D, d.d_b4_fc_bias, D->x6, kSqrt2, -1.f, C4, bn, 1);
         P.staged = 0;
         P.err_flag = D->err_flag;
-        DLA(tapgemm_finalize(P));
+        LA(tapgemm_finalize(P));
     }
     {   // dense backward: gz6 [B, C4] -> gradient wrt x5 (all 16 positions as columns), through conv's activation -> gz5
         TapGemmParams& P = D->BF;
         memset(&P, 0, sizeof P);
         sample_rows(P);
-        DLA(dense_maps(D, P, 0, 1, D->gz6, C4, 1, 1, 1, 1, 128));
+        LA(dense_maps(P, D->gz6, D->batch, C4, 1, 1, 1, 1, 128, D->split));
         const int bn = 64;
-        DLA(make_b_map(P, D->wfb, C4, 16 * C4, wm, bn));
+        LA(make_b_map(P, D->wfb, C4, 16 * C4, wm, bn));
         P.kchunks = C4 / 64;
         lin_epi(P, D, 16 * C4, bn, 1, 1);
         P.lin_saved = D->x5.hi; P.lin_saved_lo = D->x5.lo; P.lin_gz = D->gz5.hi; P.lin_gz_lo = D->gz5.lo;
         P.act_gain = kSqrt2; P.act_clamp = d.conv_clamp;
         P.err_flag = D->err_flag;
-        DLA(one_tap(D, P));
+        LA(one_tap(D, P));
     }
     {   // 3x3 conv backward: gz5 -> gradient wrt [x | stddev]
         TapGemmParams& P = D->BE;
         memset(&P, 0, sizeof P);
         set_grid(P, 4, B, 1);
-        DLA(dense_maps(D, P, 0, 1, D->gz5, C4, 4, 4, P.tw, P.th + P.halo, P.nb));
+        LA(dense_maps(P, D->gz5, D->batch, C4, 4, 4, P.tw, P.th + P.halo, P.nb, D->split));
         const int bn = 64;
-        DLA(make_b_map(P, D->web, C4, Cp, 9 * wm, bn));
+        LA(make_b_map(P, D->web, C4, Cp, 9 * wm, bn));
         P.kchunks = C4 / 64;
         lin_epi(P, D, Cp, bn, 4, 4);
         P.lin_out = D->gx4p.hi; P.lin_out_lo = D->gx4p.lo;
         P.err_flag = D->err_flag;
-        DLA(conv_taps(D, P, true));
+        LA(conv_taps(D, P, true));
     }
     return 0;
 }
@@ -717,35 +622,29 @@ int build_disc(la_disc* D) {
 int prepare_disc(la_disc* D, cudaStream_t s) {
     const la_disc_desc& d = D->d;
     const int split = D->split;
-    auto prep = [&](const float* w, int cout, int cin, int k2, float scale, int cin_pad, bf16* wf, bf16* wb) -> int {
-        const long long total = static_cast<long long>(k2) * cout * cin_pad;
-        prep_plain_weights_kernel<<<cdiv(total, 256), 256, 0, s>>>(w, cout, cin, k2, scale, cin_pad, split, wf, wb);
-        return static_cast<int>(cudaGetLastError());
-    };
     for (Block& k : D->blk) {
         if (!k.p.d_conv0_weight || !k.p.d_conv0_bias || !k.p.d_conv1_weight || !k.p.d_conv1_bias || !k.p.d_skip_weight)
-            return dfail(-2, "discriminator: missing block parameters at resolution %d", k.R);
-        DLA(prep(k.p.d_conv0_weight, k.C, k.C, 9, 1.f / sqrtf(9.f * k.C), k.C, k.w0f, k.w0b));
-        DLA(prep(k.p.d_conv1_weight, k.Cn, k.C, 9, 1.f / sqrtf(9.f * k.C), k.C, k.w1f, k.w1b));
-        DLA(prep(k.p.d_skip_weight, k.Cn, k.C, 1, kSqrtHalf / sqrtf(static_cast<float>(k.C)), k.C, k.wsf, k.wsb));
+            return fail(-2, "discriminator: missing block parameters at resolution %d", k.R);
+        LA(prep_plain_weights(k.p.d_conv0_weight, k.C, k.C, 9, 1.f / sqrtf(9.f * k.C), k.C, split, k.w0f, k.w0b, s));
+        LA(prep_plain_weights(k.p.d_conv1_weight, k.Cn, k.C, 9, 1.f / sqrtf(9.f * k.C), k.C, split, k.w1f, k.w1b, s));
+        LA(prep_plain_weights(k.p.d_skip_weight, k.Cn, k.C, 1, kSqrtHalf / sqrtf(static_cast<float>(k.C)), k.C, split, k.wsf, k.wsb, s));
     }
-    if (!D->blk[0].p.d_fromrgb_weight || !D->blk[0].p.d_fromrgb_bias) return dfail(-2, "discriminator: missing fromrgb parameters");
+    if (!D->blk[0].p.d_fromrgb_weight || !D->blk[0].p.d_fromrgb_bias) return fail(-2, "discriminator: missing fromrgb parameters");
     if (!d.d_b4_conv_weight || !d.d_b4_conv_bias || !d.d_b4_fc_weight || !d.d_b4_fc_bias || !d.d_b4_out_weight || !d.d_b4_out_bias)
-        return dfail(-2, "discriminator: missing epilogue parameters");
+        return fail(-2, "discriminator: missing epilogue parameters");
     prep_rgb_w4_kernel<<<cdiv(D->blk[0].C, 128), 128, 0, s>>>(D->blk[0].p.d_fromrgb_weight, D->blk[0].C, d.img_channels,
                                                              1.f / sqrtf(static_cast<float>(d.img_channels)), D->rgb_w4);
-    DCU(cudaGetLastError());
+    CU(cudaGetLastError());
     const int C4 = D->C4, Cp = D->Cp;
-    DLA(prep(d.d_b4_conv_weight, C4, C4 + 1, 9, 1.f / sqrtf(9.f * (C4 + 1)), Cp, D->wef, D->web));
+    LA(prep_plain_weights(d.d_b4_conv_weight, C4, C4 + 1, 9, 1.f / sqrtf(9.f * (C4 + 1)), Cp, split, D->wef, D->web, s));
     prep_fc_weights_kernel<<<cdiv(16LL * C4 * C4, 256), 256, 0, s>>>(d.d_b4_fc_weight, C4, 1.f / sqrtf(16.f * C4), split, D->wff, D->wfb);
-    DCU(cudaGetLastError());
+    CU(cudaGetLastError());
     size_t cmax = 16 * static_cast<size_t>(C4);
     for (const Block& k : D->blk) { cmax = k.C > static_cast<int>(cmax) ? k.C : cmax; cmax = k.Cn > static_cast<int>(cmax) ? k.Cn : cmax; }
     const long long n_ones = static_cast<long long>(D->batch) * cmax;
-    fill_kernel<<<cdiv(n_ones, 256), 256, 0, s>>>(D->ones, 1.f, n_ones);
-    DCU(cudaGetLastError());
-    DCU(cudaMemsetAsync(D->err_flag, 0, sizeof(int), s));
-    DCU(cudaStreamSynchronize(s));
+    LA(fill(D->ones, 1.f, n_ones, s));
+    CU(cudaMemsetAsync(D->err_flag, 0, sizeof(int), s));
+    CU(cudaStreamSynchronize(s));
     return 0;
 }
 
@@ -760,7 +659,6 @@ inline const unsigned* CU32(const bf16* p) { return reinterpret_cast<const unsig
 
 namespace la {
 
-const char* disc_last_error() { return g_derr.c_str(); }
 const float* disc_logits(const la_disc* D) { return D->logits; }
 int disc_batch(const la_disc* D) { return D->batch; }
 int disc_resolution(const la_disc* D) { return D->d.img_resolution; }
@@ -788,13 +686,12 @@ int disc_create(const la_disc_desc& d, int batch, int split, int num_sms, void* 
     D->d = d; D->batch = batch; D->num_sms = num_sms; D->split = split;
     size_t need = 0;
     int r = plan_disc(D, static_cast<char*>(ws), &need);
-    if (!r && need > bytes) r = dfail(-2, "discriminator workspace too small: %zu < %zu", bytes, need);
-    if (!r && (reinterpret_cast<uintptr_t>(ws) & 1023)) r = dfail(-2, "discriminator workspace must be 1024-byte aligned");
+    if (!r) r = check_workspace(kModule, need, bytes, ws);
     if (!r) {
         float f[16];
         cudaError_t ce = cudaMemcpyAsync(f, d.d_resample_filter, sizeof f, cudaMemcpyDeviceToHost, s);
         if (ce == cudaSuccess) ce = cudaStreamSynchronize(s);
-        if (ce != cudaSuccess) r = dfail(static_cast<int>(ce), "reading the resample filter: %s", cudaGetErrorString(ce));
+        if (ce != cudaSuccess) r = fail(static_cast<int>(ce), "discriminator: reading the resample filter: %s", cudaGetErrorString(ce));
         for (int jy = 0; jy < 4; ++jy)
             for (int jx = 0; jx < 4; ++jx) D->fir[jy * 4 + jx] = f[(3 - jy) * 4 + (3 - jx)];      // true convolution, gain 1
     }
@@ -819,32 +716,32 @@ int disc_forward(la_disc* D, const float4* img, cudaStream_t s, long long* launc
         fromrgb_fwd_kernel<<<dim3(cdiv(npix, kRgbPixels), hc / cpb), 256, 0, s>>>(img, k.p.d_fromrgb_weight, k.p.d_fromrgb_bias, npix, k.C, d.img_channels,
                                                                                 1.f / sqrtf(static_cast<float>(d.img_channels)), kSqrt2, 0.2f, d.conv_clamp,
                                                                                 U32(k.x_in.hi), U32(k.x_in.lo));
-        DCU(cudaGetLastError());
+        CU(cudaGetLastError());
         if (launches) ++*launches;
     }
     for (Block& k : D->blk) {
-        DLA(gemm(D, k.F0, s, launches));
-        DLA(upfir_backward(k.blur, s));                               // blur: x0 -> yb
-        DLA(gemm(D, k.F1, s, launches));
+        LA(gemm(D, k.F0, s, launches));
+        LA(upfir_backward(k.blur, s));                               // blur: x0 -> yb
+        LA(gemm(D, k.F1, s, launches));
         firdown_fwd_kernel<<<dim3(cdiv((k.R / 2) * (k.C / 2), 256), k.R / 2, B), 256, 0, s>>>(CU32(k.x_in.hi), CU32(k.x_in.lo), B, k.R, k.C, f,
                                                                                            U32(D->ys.hi), U32(D->ys.lo));
-        DCU(cudaGetLastError());
-        DLA(gemm(D, k.FS, s, launches));
+        CU(cudaGetLastError());
+        LA(gemm(D, k.FS, s, launches));
         if (launches) *launches += 2;
     }
     const Block& last = D->blk.back();
     const int G = d.mbstd_group_size < B ? d.mbstd_group_size : B;
-    if (B % G) return dfail(-2, "discriminator: batch %d is not a multiple of the minibatch-stddev group %d", B, G);
+    if (B % G) return fail(-2, "discriminator: batch %d is not a multiple of the minibatch-stddev group %d", B, G);
     const int M = B / G;
     mbstd_stat_kernel<<<M, 256, 0, s>>>(last.y.hi, last.y.lo, B, G, D->C4, D->feat);
     mbstd_concat_kernel<<<cdiv(static_cast<long long>(B) * 16 * D->Cp, 256), 256, 0, s>>>(last.y.hi, last.y.lo, D->feat, B, M, D->C4, D->Cp, D->x4p.hi,
                                                                                       D->x4p.lo);
-    DCU(cudaGetLastError());
-    DLA(gemm(D, D->FE, s, launches));
-    DLA(gemm(D, D->FF, s, launches));
+    CU(cudaGetLastError());
+    LA(gemm(D, D->FE, s, launches));
+    LA(gemm(D, D->FF, s, launches));
     out_fwd_kernel<<<cdiv(B, 8), 256, 0, s>>>(D->x6.hi, D->x6.lo, d.d_b4_out_weight, d.d_b4_out_bias, B, D->C4, 1.f / sqrtf(static_cast<float>(D->C4)),
                                               D->logits);
-    DCU(cudaGetLastError());
+    CU(cudaGetLastError());
     if (launches) *launches += 3;
     return 0;
 }
@@ -858,27 +755,27 @@ int disc_backward(la_disc* D, float w_disc, float4* g_img, int accumulate, float
     disc_loss_kernel<<<1, 256, 0, s>>>(D->logits, B, w_disc, d_loss, D->gl);
     out_bwd_kernel<<<cdiv(static_cast<long long>(B) * C4, 256), 256, 0, s>>>(D->gl, d.d_b4_out_weight, D->x6.hi, B, C4, 1.f / sqrtf(static_cast<float>(C4)),
                                                                          kSqrt2, 0.2f, D->gz6.hi, D->gz6.lo);
-    DCU(cudaGetLastError());
-    DLA(gemm(D, D->BF, s, launches));
-    DLA(gemm(D, D->BE, s, launches));
+    CU(cudaGetLastError());
+    LA(gemm(D, D->BF, s, launches));
+    LA(gemm(D, D->BE, s, launches));
     mbstd_gfeat_kernel<<<M, 128, 0, s>>>(D->gx4p.hi, D->gx4p.lo, B, M, C4, Cp, D->gfeat);
     mbstd_bwd_kernel<<<cdiv(static_cast<long long>(M) * 16 * C4, 256), 256, 0, s>>>(
         last.y.hi, last.y.lo, D->gx4p.hi, D->gx4p.lo, D->gfeat, last.y1.hi, last.y1.lo, B, G, C4, Cp, kSqrt2 * kSqrtHalf, 0.2f,
         d.conv_clamp >= 0.f ? d.conv_clamp * kSqrtHalf : d.conv_clamp, last.g_y.hi, last.g_y.lo, last.g_z1.hi, last.g_z1.lo);
-    DCU(cudaGetLastError());
+    CU(cudaGetLastError());
     if (launches) *launches += 4;
     for (int b = d.num_blocks - 1; b >= 0; --b) {
         Block& k = D->blk[b];
-        DLA(gemm(D, k.BS, s, launches));                              // g_ys = Ws^T g_y
-        DLA(gemm(D, k.B1, s, launches));                              // g_yb = conv1^T g_z1
-        DLA(upfir_forward(k.blur, s));                                // g_z0 = blur^T(g_yb) * act0'(x0)
+        LA(gemm(D, k.BS, s, launches));                              // g_ys = Ws^T g_y
+        LA(gemm(D, k.B1, s, launches));                              // g_yb = conv1^T g_z1
+        LA(upfir_forward(k.blur, s));                                // g_z0 = blur^T(g_yb) * act0'(x0)
         if (b == 0) {                                                 // + fused fromrgb backward: atomics into g_img
-            if (!accumulate) DCU(cudaMemsetAsync(g_img, 0, sizeof(float4) * static_cast<size_t>(B) * k.R * k.R, s));
+            if (!accumulate) CU(cudaMemsetAsync(g_img, 0, sizeof(float4) * static_cast<size_t>(B) * k.R * k.R, s));
             TapGemmParams P = k.B0;
             P.lin_rgb_g = g_img;
-            DLA(gemm(D, P, s, launches));
+            LA(gemm(D, P, s, launches));
         } else {
-            DLA(gemm(D, k.B0, s, launches));                          // conv0^T + FIRdown^T(g_ys) -> block input gradient
+            LA(gemm(D, k.B0, s, launches));                          // conv0^T + FIRdown^T(g_ys) -> block input gradient
         }
         if (launches) *launches += 1;
     }

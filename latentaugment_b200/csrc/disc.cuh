@@ -23,7 +23,6 @@ const float* disc_logits(const la_disc* D);
 int disc_batch(const la_disc* D);
 int disc_resolution(const la_disc* D);
 int disc_channels(const la_disc* D);
-const char* disc_last_error();
 
 // NCHW fp32 <-> float4-per-pixel image converters (stand-alone entry points)
 int nchw_to_f4(const float* src, int batch, int C, int res, float4* dst, cudaStream_t s);

@@ -11,23 +11,15 @@
 #include <stdlib.h>
 #include <string.h>
 
-#include <string>
-
 #include "../../include/latentaugment_b200.h"
+#include "common.cuh"
 #include "tapgemm.cuh"
 
 using namespace la;
 
-int la_fail_msg(int code, const char* msg);   // engine.cu
-
-#define DCU(x)                                                                           \
-    do {                                                                                 \
-        cudaError_t e_ = (x);                                                            \
-        if (e_ != cudaSuccess) return la_fail_msg(static_cast<int>(e_), cudaGetErrorString(e_)); \
-    } while (0)
-
 namespace {
 
+constexpr char kModule[] = "distance";
 typedef __nv_bfloat16 bf16;
 constexpr int kCand = 2;          // candidates kept per (query, 32-code chunk)
 constexpr int kChunk = 32;
@@ -40,12 +32,6 @@ constexpr int kMemberCap = 256;   // ambiguous (probe, point) pairs listed per p
 // (worst case, partial sums bounded by the sum of the magnitudes).  Cauchy-Schwarz: sum|x_k y_k| <= |x| |y|; the factor 2 of
 // the score doubles both.
 __host__ __device__ __forceinline__ float split_eps_coef(int K) { return 3.0518e-5f + static_cast<float>(K) * 3.612e-7f; }
-
-__device__ __forceinline__ double warp_sum_d(double v) {
-#pragma unroll
-    for (int o = 16; o >= 1; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-    return v;
-}
 
 // rows -> bf16 (hi [, lo] planes) + |row|^2 (fp64 accumulate, rounded once to fp32).  Warp per row.
 __global__ void split_rows_kernel(const float* __restrict__ src, int rows, int rows_padded, int K, bf16* hi, bf16* lo, float* sqnorm) {
@@ -376,8 +362,8 @@ NearestLayout nearest_layout(int n, int m, int K, DistanceMode mode = kSearch, i
     L.rows_padded = L.Hq * 16;
     L.n_blocks = (m + 255) / 256;
     L.ncand = mode == kMember ? 0 : L.n_blocks * (256 / kChunk) * kCand;
-    size_t off = 0;
-    auto take = [&](size_t b) { off = (off + 1023) & ~size_t(1023); size_t o = off; off += b; return o; };
+    Bump bp;                                     // null base: offsets only
+    auto take = [&](size_t b) { bp.take<char>(b); return bp.off - b; };
     L.off_xhi = take(static_cast<size_t>(L.rows_padded) * K * 2);
     L.off_xx = take(static_cast<size_t>(L.rows_padded) * 4);
     L.off_cs = take(static_cast<size_t>(n) * L.ncand * 4);
@@ -394,7 +380,7 @@ NearestLayout nearest_layout(int n, int m, int K, DistanceMode mode = kSearch, i
         L.off_flags = take(static_cast<size_t>(n) * 8);          // [n] hit | [n] list count (one memset)
         L.off_list = take(static_cast<size_t>(n) * kMemberCap * 4);
     }
-    L.total = off + 1024;
+    L.total = bp.off + 1024;
     return L;
 }
 
@@ -407,11 +393,11 @@ int distance_gemm(TapGemmParams& P, const float* d_X, int n, const void* d_bank,
     bf16* xlo = split ? reinterpret_cast<bf16*>(ws + L.off_xlo) : nullptr;
     float* xx = reinterpret_cast<float*>(ws + L.off_xx);
     split_rows_kernel<<<(L.rows_padded + 7) / 8, 256, 0, s>>>(d_X, n, L.rows_padded, K, xhi, xlo, xx);
-    DCU(cudaGetLastError());
+    CU(cudaGetLastError());
 
     int dev = 0, sms = 0;
-    DCU(cudaGetDevice(&dev));
-    DCU(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+    CU(cudaGetDevice(&dev));
+    CU(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
     P.th = 8; P.tw = 16; P.nb = 1;
     P.tiles_n = 1; P.batch = 1; P.nprob = 1;
     P.prob[0].tiles_h = L.Hq / 8; P.prob[0].tiles_w = 1; P.prob[0].vh = L.Hq; P.prob[0].vw = 16;
@@ -427,12 +413,12 @@ int distance_gemm(TapGemmParams& P, const float* d_X, int n, const void* d_bank,
         P.taps[0] = Tap{0, 0, 0, 0};      // one bf16 pass: bf16(x) . bf16(y); the exact re-rank absorbs its error (rerank_kernel)
         P.prob[0].tap_begin = 0; P.prob[0].ntaps = 1;
     }
-    if (tapgemm_finalize(P)) return la_fail_msg(-5, "tap grouping failed");
+    if (tapgemm_finalize(P)) return fail(-5, "tap grouping failed");
     uint64_t adims[4] = {static_cast<uint64_t>(K), 16, static_cast<uint64_t>(L.Hq), 1};
     uint64_t astr[3] = {static_cast<uint64_t>(K) * 2, static_cast<uint64_t>(K) * 32, static_cast<uint64_t>(K) * 32 * L.Hq};
     uint32_t abox[4] = {64, 16, 8, 1};
-    if (encode_tmap_bf16(&P.a_map[0], xhi, 4, adims, astr, abox)) return la_fail_msg(-5, "tensor map encoding failed (queries)");
-    if (split && encode_tmap_bf16(&P.a_map[1], xlo, 4, adims, astr, abox)) return la_fail_msg(-5, "tensor map encoding failed (queries, lo)");
+    if (encode_tmap_bf16(&P.a_map[0], xhi, 4, adims, astr, abox)) return fail(-5, "tensor map encoding failed (queries)");
+    if (split && encode_tmap_bf16(&P.a_map[1], xlo, 4, adims, astr, abox)) return fail(-5, "tensor map encoding failed (queries, lo)");
     uint64_t bdims[3] = {static_cast<uint64_t>(K), static_cast<uint64_t>(m), split ? 2u : 1u};
     uint64_t bstr[2] = {static_cast<uint64_t>(K) * 2, static_cast<uint64_t>(K) * 2 * m};
     // CTA pairs (cta_group::2: two query tiles per MMA, each CTA loads half of every bank tile) halve the bank operand
@@ -441,9 +427,9 @@ int distance_gemm(TapGemmParams& P, const float* d_X, int n, const void* d_bank,
     static const bool pair = getenv("LA_NEAREST_PAIR") && atoi(getenv("LA_NEAREST_PAIR")) == 1;
     P.cta2 = pair && L.Hq / 8 >= 2 ? 1 : 0;
     uint32_t bbox[3] = {64, static_cast<uint32_t>(P.cta2 ? 128 : 256), 1};
-    if (encode_tmap_bf16(&P.b_map, d_bank, 3, bdims, bstr, bbox)) return la_fail_msg(-5, "tensor map encoding failed (bank)");
+    if (encode_tmap_bf16(&P.b_map, d_bank, 3, bdims, bstr, bbox)) return fail(-5, "tensor map encoding failed (bank)");
     P.err_flag = reinterpret_cast<int*>(ws + L.off_err);
-    DCU(cudaMemsetAsync(P.err_flag, 0, sizeof(int), s));
+    CU(cudaMemsetAsync(P.err_flag, 0, sizeof(int), s));
     if (getenv("LA_DEBUG_SIMT_DIST")) {
         TapSimtOperands ops{};
         ops.a_ptrs[0] = xhi; ops.a_ptrs[1] = xlo;
@@ -451,10 +437,10 @@ int distance_gemm(TapGemmParams& P, const float* d_X, int n, const void* d_bank,
         ops.a_ws[0] = ops.a_ws[1] = 16; ops.a_hs[0] = ops.a_hs[1] = L.Hq;
         ops.w = d_bank;
         int r = launch_tapgemm_simt(P, ops, s);
-        if (r) return la_fail_msg(r, "launch_tapgemm_simt failed");
+        if (r) return fail(r, "launch_tapgemm_simt failed");
     } else {
         int r = launch_tapgemm(P, sms, s);
-        if (r) return la_fail_msg(r, "launch_tapgemm failed");
+        if (r) return fail(r, "launch_tapgemm failed");
     }
     return 0;
 }
@@ -471,7 +457,7 @@ int launch_rerank(const float* d_X, const float* xx, const float* d_Y, const flo
         case 1024: rerank_kernel<8><<<n, rb, 0, s>>>(d_X, xx, d_Y, d_bank_sqnorm, n, m, K, cs, ci, ncand, k, index_offset, d_dist, d_idx, split, fallback); break;
         default: rerank_kernel<0><<<n, rb, 0, s>>>(d_X, xx, d_Y, d_bank_sqnorm, n, m, K, cs, ci, ncand, k, index_offset, d_dist, d_idx, split, fallback); break;
     }
-    DCU(cudaGetLastError());
+    CU(cudaGetLastError());
     return 0;
 }
 
@@ -481,27 +467,27 @@ extern "C" {
 
 __attribute__((visibility("default")))
 int la_pairwise_sqdist(const float* d_X, int n, const float* d_Y, int m, int K, float* d_D, la_stream stream) {
-    if (!d_X || !d_Y || !d_D || n < 1 || m < 1 || K < 1) return la_fail_msg(-2, "bad arguments");
+    if (!d_X || !d_Y || !d_D || n < 1 || m < 1 || K < 1) return fail(-2, "bad arguments");
     const long long pairs = static_cast<long long>(m) * n;
     pairwise_kernel<<<static_cast<unsigned>((pairs + 7) / 8), 256, 0, static_cast<cudaStream_t>(stream)>>>(d_X, n, d_Y, m, K, d_D);
-    DCU(cudaGetLastError());
+    CU(cudaGetLastError());
     return 0;
 }
 
 __attribute__((visibility("default")))
 int la_bank_prepare(const float* d_Y, int m, int K, void* d_bank_bf16, float* d_bank_sqnorm, la_stream stream) {
-    if (!d_Y || !d_bank_bf16 || !d_bank_sqnorm || m < 1 || K < 64 || K % 64) return la_fail_msg(-2, "bad arguments (K must be a multiple of 64)");
+    if (!d_Y || !d_bank_bf16 || !d_bank_sqnorm || m < 1 || K < 64 || K % 64) return fail(-2, "bad arguments (K must be a multiple of 64)");
     bf16* hi = static_cast<bf16*>(d_bank_bf16);
     split_rows_kernel<<<(m + 7) / 8, 256, 0, static_cast<cudaStream_t>(stream)>>>(d_Y, m, m, K, hi, nullptr, d_bank_sqnorm);
-    DCU(cudaGetLastError());
+    CU(cudaGetLastError());
     max_sqnorm_kernel<<<1, 1024, 0, static_cast<cudaStream_t>(stream)>>>(d_bank_sqnorm, m);
-    DCU(cudaGetLastError());
+    CU(cudaGetLastError());
     return 0;
 }
 
 __attribute__((visibility("default")))
 int la_nearest_codes_workspace_bytes(int n, int m, int K, int k, size_t* bytes) {
-    if (!bytes || n < 1 || m < 1 || K % 64 || k < 1 || k > 8) return la_fail_msg(-2, "bad arguments (k <= 8, K % 64 == 0)");
+    if (!bytes || n < 1 || m < 1 || K % 64 || k < 1 || k > 8) return fail(-2, "bad arguments (k <= 8, K %% 64 == 0)");
     *bytes = nearest_layout(n, m, K).total;
     return 0;
 }
@@ -510,11 +496,10 @@ __attribute__((visibility("default")))
 int la_nearest_codes(const float* d_X, int n, const float* d_Y, const void* d_bank_bf16, const float* d_bank_sqnorm, int m, int K, int k,
                      long long index_offset, void* d_workspace, size_t workspace_bytes, float* d_dist, long long* d_idx,
                      la_stream stream) {
-    if (!d_X || !d_Y || !d_bank_bf16 || !d_bank_sqnorm || !d_workspace || !d_dist || !d_idx) return la_fail_msg(-2, "bad arguments");
-    if (k < 1 || k > 8 || K % 64 || K < 64) return la_fail_msg(-2, "k must be 1..8 and K a multiple of 64");
+    if (!d_X || !d_Y || !d_bank_bf16 || !d_bank_sqnorm || !d_workspace || !d_dist || !d_idx) return fail(-2, "bad arguments");
+    if (k < 1 || k > 8 || K % 64 || K < 64) return fail(-2, "k must be 1..8 and K a multiple of 64");
     const NearestLayout L = nearest_layout(n, m, K);
-    if (workspace_bytes < L.total) return la_fail_msg(-2, "nearest-codes workspace too small");
-    if (reinterpret_cast<uintptr_t>(d_workspace) & 1023) return la_fail_msg(-2, "workspace must be 1024-byte aligned");
+    if (int r = check_workspace("nearest-codes", L.total, workspace_bytes, d_workspace)) return r;
     cudaStream_t s = static_cast<cudaStream_t>(stream);
     char* ws = static_cast<char*>(d_workspace);
     float* cs = reinterpret_cast<float*>(ws + L.off_cs);
@@ -532,39 +517,39 @@ int la_nearest_codes(const float* d_X, int n, const float* d_Y, const void* d_ba
 __attribute__((visibility("default")))
 int la_merge_topk(const float* d_dist, const long long* d_idx, int shards, int n, int k, float* d_out_dist, long long* d_out_idx,
                   la_stream stream) {
-    if (!d_dist || !d_idx || !d_out_dist || !d_out_idx || shards < 1 || n < 1 || k < 1 || k > 8) return la_fail_msg(-2, "bad arguments");
+    if (!d_dist || !d_idx || !d_out_dist || !d_out_idx || shards < 1 || n < 1 || k < 1 || k > 8) return fail(-2, "bad arguments");
     const long long st = static_cast<long long>(n) * k;
     merge_topk_kernel<<<(n + 127) / 128, 128, 0, static_cast<cudaStream_t>(stream)>>>(d_dist, d_idx, shards, n, k, st, st, d_out_dist, d_out_idx);
-    DCU(cudaGetLastError());
+    CU(cudaGetLastError());
     return 0;
 }
 
 __attribute__((visibility("default")))
 int la_merge_topk_strided(const float* d_dist, const long long* d_idx, int shards, int n, int k, long long dist_shard_stride,
                           long long idx_shard_stride, float* d_out_dist, long long* d_out_idx, la_stream stream) {
-    if (!d_dist || !d_idx || !d_out_dist || !d_out_idx || shards < 1 || n < 1 || k < 1 || k > 8) return la_fail_msg(-2, "bad arguments");
+    if (!d_dist || !d_idx || !d_out_dist || !d_out_idx || shards < 1 || n < 1 || k < 1 || k > 8) return fail(-2, "bad arguments");
     merge_topk_kernel<<<(n + 127) / 128, 128, 0, static_cast<cudaStream_t>(stream)>>>(d_dist, d_idx, shards, n, k, dist_shard_stride,
                                                                                       idx_shard_stride, d_out_dist, d_out_idx);
-    DCU(cudaGetLastError());
+    CU(cudaGetLastError());
     return 0;
 }
 
 __attribute__((visibility("default")))
 int la_pr_manifold_prepare(const float* d_Y, int m, int K, void* d_planes, float* d_sqnorm, la_stream stream) {
-    if (!d_Y || !d_planes || !d_sqnorm || m < 1 || K < 64 || K % 64) return la_fail_msg(-2, "bad arguments (K must be a multiple of 64)");
+    if (!d_Y || !d_planes || !d_sqnorm || m < 1 || K < 64 || K % 64) return fail(-2, "bad arguments (K must be a multiple of 64)");
     bf16* hi = static_cast<bf16*>(d_planes);
     split_rows_kernel<<<(m + 7) / 8, 256, 0, static_cast<cudaStream_t>(stream)>>>(d_Y, m, m, K, hi, hi + static_cast<long long>(m) * K, d_sqnorm);
-    DCU(cudaGetLastError());
+    CU(cudaGetLastError());
     max_sqnorm_kernel<<<1, 1024, 0, static_cast<cudaStream_t>(stream)>>>(d_sqnorm, m);
-    DCU(cudaGetLastError());
+    CU(cudaGetLastError());
     return 0;
 }
 
 __attribute__((visibility("default")))
 int la_pr_radii_workspace_bytes(int n, int m, int K, int nhood, size_t* bytes) {
-    if (!bytes || n < 1 || K < 64 || K % 64) return la_fail_msg(-2, "bad arguments (K must be a multiple of 64)");
-    if (nhood < 1 || nhood > 7) return la_fail_msg(-2, "nhood must be 1..7");
-    if (m < nhood + 1) return la_fail_msg(-2, "the manifold needs at least nhood + 1 points");
+    if (!bytes || n < 1 || K < 64 || K % 64) return fail(-2, "bad arguments (K must be a multiple of 64)");
+    if (nhood < 1 || nhood > 7) return fail(-2, "nhood must be 1..7");
+    if (m < nhood + 1) return fail(-2, "the manifold needs at least nhood + 1 points");
     *bytes = nearest_layout(n, m, K, kRadii, nhood + 1).total;
     return 0;
 }
@@ -573,10 +558,9 @@ __attribute__((visibility("default")))
 int la_pr_radii(const float* d_X, int n, const float* d_Y, const void* d_planes, const float* d_sqnorm, int m, int K, int nhood,
                 void* d_workspace, size_t workspace_bytes, float* d_r2, int* d_fallback, la_stream stream) {
     size_t need = 0;
-    if (!d_X || !d_Y || !d_planes || !d_sqnorm || !d_workspace || !d_r2) return la_fail_msg(-2, "bad arguments");
+    if (!d_X || !d_Y || !d_planes || !d_sqnorm || !d_workspace || !d_r2) return fail(-2, "bad arguments");
     if (int r = la_pr_radii_workspace_bytes(n, m, K, nhood, &need)) return r;
-    if (workspace_bytes < need) return la_fail_msg(-2, "radii workspace too small");
-    if (reinterpret_cast<uintptr_t>(d_workspace) & 1023) return la_fail_msg(-2, "workspace must be 1024-byte aligned");
+    if (int r = check_workspace("radii", need, workspace_bytes, d_workspace)) return r;
     const int k = nhood + 1;
     const NearestLayout L = nearest_layout(n, m, K, kRadii, k);
     cudaStream_t s = static_cast<cudaStream_t>(stream);
@@ -594,14 +578,14 @@ int la_pr_radii(const float* d_X, int n, const float* d_Y, const void* d_planes,
                               reinterpret_cast<long long*>(ws + L.off_idx), 1, d_fallback, s))
         return r;
     // r2[i] = dist[i][nhood]: the (nhood + 1)-th smallest distance, the point itself included
-    DCU(cudaMemcpy2DAsync(d_r2, sizeof(float), dist + nhood, static_cast<size_t>(k) * sizeof(float), sizeof(float), n,
+    CU(cudaMemcpy2DAsync(d_r2, sizeof(float), dist + nhood, static_cast<size_t>(k) * sizeof(float), sizeof(float), n,
                           cudaMemcpyDeviceToDevice, s));
     return 0;
 }
 
 __attribute__((visibility("default")))
 int la_pr_member_workspace_bytes(int n, int m, int K, size_t* bytes) {
-    if (!bytes || n < 1 || m < 1 || K < 64 || K % 64) return la_fail_msg(-2, "bad arguments (K must be a multiple of 64)");
+    if (!bytes || n < 1 || m < 1 || K < 64 || K % 64) return fail(-2, "bad arguments (K must be a multiple of 64)");
     *bytes = nearest_layout(n, m, K, kMember).total;
     return 0;
 }
@@ -610,10 +594,9 @@ __attribute__((visibility("default")))
 int la_pr_member(const float* d_X, int n, const float* d_Y, const void* d_planes, const float* d_sqnorm, const float* d_r2, int m, int K,
                  void* d_workspace, size_t workspace_bytes, unsigned char* d_member, int* d_fallback, la_stream stream) {
     size_t need = 0;
-    if (!d_X || !d_Y || !d_planes || !d_sqnorm || !d_r2 || !d_workspace || !d_member) return la_fail_msg(-2, "bad arguments");
+    if (!d_X || !d_Y || !d_planes || !d_sqnorm || !d_r2 || !d_workspace || !d_member) return fail(-2, "bad arguments");
     if (int r = la_pr_member_workspace_bytes(n, m, K, &need)) return r;
-    if (workspace_bytes < need) return la_fail_msg(-2, "membership workspace too small");
-    if (reinterpret_cast<uintptr_t>(d_workspace) & 1023) return la_fail_msg(-2, "workspace must be 1024-byte aligned");
+    if (int r = check_workspace("membership", need, workspace_bytes, d_workspace)) return r;
     const NearestLayout L = nearest_layout(n, m, K, kMember);
     cudaStream_t s = static_cast<cudaStream_t>(stream);
     char* ws = static_cast<char*>(d_workspace);
@@ -622,8 +605,8 @@ int la_pr_member(const float* d_X, int n, const float* d_Y, const void* d_planes
     int* cnt = hit + n;
     int* list = reinterpret_cast<int*>(ws + L.off_list);
     member_table_kernel<<<(m + 255) / 256, 256, 0, s>>>(d_r2, d_sqnorm, m, tab);
-    DCU(cudaGetLastError());
-    DCU(cudaMemsetAsync(hit, 0, static_cast<size_t>(n) * 8, s));
+    CU(cudaGetLastError());
+    CU(cudaMemsetAsync(hit, 0, static_cast<size_t>(n) * 8, s));
     TapGemmParams P;
     memset(&P, 0, sizeof P);
     P.epilogue = kEpiMember;
@@ -635,7 +618,7 @@ int la_pr_member(const float* d_X, int n, const float* d_Y, const void* d_planes
     if (int r = distance_gemm(P, d_X, n, d_planes, m, K, L, ws, true, s)) return r;
     member_recheck_kernel<<<n, 32 * kRecheckWarps, 0, s>>>(d_X, reinterpret_cast<float*>(ws + L.off_xx), d_Y, tab, n, m, K, hit, cnt,
                                                            list, d_member, d_fallback);
-    DCU(cudaGetLastError());
+    CU(cudaGetLastError());
     return 0;
 }
 

@@ -11,6 +11,7 @@
 #include <vector>
 
 #include "../../include/latentaugment_b200.h"
+#include "common.cuh"
 #include "kernels.cuh"
 #include "tapgemm.cuh"
 #include "plan.cuh"
@@ -21,42 +22,8 @@ using namespace la;
 
 namespace {
 
-thread_local std::string g_err;
-
-int fail(int code, const char* fmt, ...) {
-    char buf[512];
-    va_list ap;
-    va_start(ap, fmt);
-    vsnprintf(buf, sizeof buf, fmt, ap);
-    va_end(ap);
-    g_err = buf;
-    return code ? code : -1;
-}
-
-#define CU(x)                                                                                              \
-    do {                                                                                                   \
-        cudaError_t e_ = (x);                                                                              \
-        if (e_ != cudaSuccess) return fail(static_cast<int>(e_), "%s: %s (%s:%d)", #x, cudaGetErrorString(e_), __FILE__, __LINE__); \
-    } while (0)
-#define LA(x)                                                                                              \
-    do {                                                                                                   \
-        int r_ = (x);                                                                                      \
-        if (r_) return fail(r_, "%s: %s (%s:%d)", #x, r_ > 0 ? cudaGetErrorString(static_cast<cudaError_t>(r_)) : "error", __FILE__, __LINE__); \
-    } while (0)
-
+constexpr char kModule[] = "engine";
 typedef __nv_bfloat16 bf16;
-
-struct Bump {
-    char* base = nullptr;
-    size_t off = 0;
-    template <class T>
-    T* take(size_t count) {
-        off = (off + 1023) & ~size_t(1023);
-        T* p = base ? reinterpret_cast<T*>(base + off) : nullptr;
-        off += count * sizeof(T);
-        return p;
-    }
-};
 
 struct Conv {
     int res_in, res, cin, cout, up, block, last_in_block, ws_idx, soff, doff;
@@ -580,7 +547,7 @@ int run_backward(la_engine* e, const la_augment_options& opt, bool project, cuda
     if (project) {
         CU(cudaMemsetAsync(top.g_img, 0, sizeof(float4) * static_cast<size_t>(B) * g.img_resolution * g.img_resolution, s));
         if (lpips_forward(e->lp, top.img, 1, s, &e->launches) || lpips_backward(e->lp, top.g_img, 1, e->lpips_loss, 1, s, &e->launches))
-            return fail(-7, "lpips: %s", lpips_last_error());
+            return -7;
     } else if (opt.w_pix > 0.f) {
         LA(pix_loss(top.img, e->bank_mean, e->bank_m2, B, g.img_resolution, g.img_channels, e->crop_off, e->crop_size, e->cur_w_pix,
                     top.g_img, e->loss_parts, &nparts, s));
@@ -590,11 +557,11 @@ int run_backward(la_engine* e, const la_augment_options& opt, bool project, cuda
     e->n_loss_parts = nparts;
     if (!project && opt.w_disc > 0.f) {          // realism term (util_latent_aug.py:363-371): + w_disc * mean softplus(-D(x))
         if (disc_forward(e->disc, top.img, s, &e->launches) || disc_backward(e->disc, opt.w_disc, top.g_img, 1, e->disc_loss, s, &e->launches))
-            return fail(-6, "discriminator: %s", disc_last_error());
+            return -6;
     }
     if (!project && opt.w_lpips > 0.f) {   // perceptual term (util_latent_aug.py:387-424): - w_lpips * pair-normalised LPIPS distance to the bank
         if (lpips_forward(e->lp, top.img, 0, s, &e->launches) || lpips_backward(e->lp, top.g_img, 1, e->lpips_loss, 0, s, &e->launches))
-            return fail(-7, "lpips: %s", lpips_last_error());
+            return -7;
     }
     for (int b = g.num_blocks - 1; b >= 0; --b) {
         Rgb& r = e->rgb[b];
@@ -683,9 +650,19 @@ int check_err_flag(la_engine* e, cudaStream_t s) {
     return 0;
 }
 
+thread_local std::string g_err;       // the text of la_last_error(), written by every module through la::fail
+
 }  // namespace
 
-int la_fail_msg(int code, const char* msg) { return fail(code, "%s", msg); }
+int la::fail(int code, const char* fmt, ...) {
+    char buf[512];
+    va_list ap;
+    va_start(ap, fmt);
+    vsnprintf(buf, sizeof buf, fmt, ap);
+    va_end(ap);
+    g_err = buf;
+    return code ? code : -1;
+}
 
 // ======================================================================================= C ABI
 #define LA_API __attribute__((visibility("default")))
@@ -724,8 +701,7 @@ LA_API int la_engine_create(const la_generator_desc* g, int batch, int precision
     e->split_min_res = upconv_split_min_res();
     size_t need = 0;
     int r = plan(e, static_cast<char*>(d_workspace), &need);
-    if (!r && need > workspace_bytes) r = fail(-2, "workspace too small: %zu < %zu", workspace_bytes, need);
-    if (!r && (reinterpret_cast<uintptr_t>(d_workspace) & 1023)) r = fail(-2, "workspace must be 1024-byte aligned");
+    if (!r) r = check_workspace(kModule, need, workspace_bytes, d_workspace);
     const int res = g->img_resolution;
     e->crop_size = static_cast<int>(sqrt(static_cast<double>(res) * res / 2.0));          // util_dataset.py:317-323
     e->crop_off = static_cast<int>(nearbyint((res - e->crop_size) / 2.0));               // torchvision CenterCrop
@@ -849,7 +825,7 @@ LA_API int la_augment(la_engine* e, const float* d_w0, const la_augment_options*
     CU(cudaMemsetAsync(e->loss_log, 0, sizeof(float) * LA_LOSS_COLS * LA_MAX_STEPS, w));
     if (opt->w_lpips > 0.f) {        // crop window of this call (util_dataset.py:284-309,325-332), absolute image coordinates
         if (lpips_set_call(e->lp, opt->lpips_crop_x, opt->lpips_crop_y, opt->w_lpips, opt->lpips_norm_mode, w))
-            return fail(-7, "lpips: %s", lpips_last_error());
+            return -7;
     }
     if ((e->cur_project || e->cur_w_pix != opt->w_pix || e->cur_w_disc != opt->w_disc || (e->cur_w_lpips > 0.f) != (opt->w_lpips > 0.f)) &&
         e->step_graph) {   // baked into the criterion launches
@@ -879,7 +855,7 @@ LA_API int la_set_projection_targets(la_engine* e, const float* d_img, la_stream
     Rgb& top = e->rgb.back();
     LA(bridge_in(e, s));
     LA(nchw_to_f4(d_img, e->batch, e->g.img_channels, e->g.img_resolution, top.img, e->work));
-    if (lpips_set_targets(e->lp, top.img, e->work, &e->launches)) return fail(-7, "lpips: %s", lpips_last_error());
+    if (lpips_set_targets(e->lp, top.img, e->work, &e->launches)) return -7;
     LA(bridge_out(e, s));
     return 0;
 }
@@ -895,7 +871,7 @@ LA_API int la_project(la_engine* e, const float* d_w0, int num_steps, const floa
     LA(bridge_in(e, s));
     const ProjConsts hc{d_lr, d_sigma, d_wnoise, num_steps};
     CU(cudaMemcpyAsync(e->proj, &hc, sizeof hc, cudaMemcpyHostToDevice, w));
-    if (lpips_set_call(e->lp, 0, 0, 1.f, 1, w)) return fail(-7, "lpips: %s", lpips_last_error());      // whole-image window
+    if (lpips_set_call(e->lp, 0, 0, 1.f, 1, w)) return -7;      // whole-image window
     CU(cudaMemcpyAsync(e->w_opt, d_w0, wbytes, cudaMemcpyDeviceToDevice, w));
     CU(cudaMemsetAsync(e->m, 0, wbytes, w));
     CU(cudaMemsetAsync(e->v, 0, wbytes, w));
@@ -916,7 +892,7 @@ LA_API int la_project(la_engine* e, const float* d_w0, int num_steps, const floa
 
 LA_API int la_disc_workspace_bytes(const la_disc_desc* d, int batch, int precision, size_t* bytes) {
     if (!d || !bytes || batch < 1) return fail(-2, "bad arguments");
-    if (disc_workspace_bytes(*d, batch, precision == LA_PRECISION_FP32_PARITY, bytes)) return fail(-2, "%s", disc_last_error());
+    if (disc_workspace_bytes(*d, batch, precision == LA_PRECISION_FP32_PARITY, bytes)) return -2;
     return 0;
 }
 
@@ -927,7 +903,7 @@ LA_API int la_set_discriminator(la_engine* e, const la_disc_desc* d, void* d_wor
     if (e->disc) { disc_destroy(e->disc); e->disc = nullptr; }
     if (e->step_graph) { cudaGraphExecDestroy(e->step_graph); e->step_graph = nullptr; }
     if (disc_create(*d, e->batch, e->split, e->num_sms, d_workspace, workspace_bytes, static_cast<cudaStream_t>(stream), &e->disc))
-        return fail(-6, "discriminator: %s", disc_last_error());
+        return -6;
     return 0;
 }
 
@@ -937,7 +913,7 @@ LA_API int la_disc_logits(la_engine* e, const float* d_img, float* d_logits, la_
     Rgb& top = e->rgb.back();
     LA(bridge_in(e, s));
     LA(nchw_to_f4(d_img, e->batch, e->g.img_channels, e->g.img_resolution, top.img, e->work));
-    if (disc_forward(e->disc, top.img, e->work, &e->launches)) return fail(-6, "discriminator: %s", disc_last_error());
+    if (disc_forward(e->disc, top.img, e->work, &e->launches)) return -6;
     CU(cudaMemcpyAsync(d_logits, disc_logits(e->disc), sizeof(float) * e->batch, cudaMemcpyDeviceToDevice, e->work));
     LA(bridge_out(e, s));
     return 0;
@@ -951,7 +927,7 @@ LA_API int la_disc_loss_grad(la_engine* e, const float* d_img, float w_disc, flo
     LA(nchw_to_f4(d_img, e->batch, e->g.img_channels, e->g.img_resolution, top.img, e->work));
     if (disc_forward(e->disc, top.img, e->work, &e->launches) ||
         disc_backward(e->disc, w_disc, top.g_img, 0, e->disc_loss, e->work, &e->launches))
-        return fail(-6, "discriminator: %s", disc_last_error());
+        return -6;
     LA(f4_to_nchw(top.g_img, e->batch, e->g.img_channels, e->g.img_resolution, d_grad, e->work));
     CU(cudaMemcpyAsync(d_loss, e->disc_loss, sizeof(float), cudaMemcpyDeviceToDevice, e->work));
     LA(bridge_out(e, s));
@@ -960,7 +936,7 @@ LA_API int la_disc_loss_grad(la_engine* e, const float* d_img, float w_disc, flo
 
 LA_API int la_lpips_workspace_bytes(const la_vgg_desc* v, int batch, int img_channels, int precision, size_t* bytes) {
     if (!v || !bytes || batch < 1) return fail(-2, "bad arguments");
-    if (lpips_workspace_bytes(*v, batch, img_channels, precision == LA_PRECISION_FP32_PARITY, bytes)) return fail(-2, "%s", lpips_last_error());
+    if (lpips_workspace_bytes(*v, batch, img_channels, precision == LA_PRECISION_FP32_PARITY, bytes)) return -2;
     return 0;
 }
 
@@ -970,7 +946,7 @@ LA_API int la_set_lpips(la_engine* e, const la_vgg_desc* v, void* d_workspace, s
     if (e->step_graph) { cudaGraphExecDestroy(e->step_graph); e->step_graph = nullptr; }
     if (lpips_create(*v, e->batch, e->g.img_channels, e->g.img_resolution, e->split, e->num_sms, d_workspace, workspace_bytes,
                      static_cast<cudaStream_t>(stream), &e->lp))
-        return fail(-7, "lpips: %s", lpips_last_error());
+        return -7;
     return 0;
 }
 
@@ -978,7 +954,7 @@ LA_API int la_set_feature_bank(la_engine* e, const float* d_crops, int M, la_str
     if (!e || !e->lp || !d_crops || M < 1) return fail(-2, "bad arguments (la_set_lpips first)");
     cudaStream_t s = static_cast<cudaStream_t>(stream);
     LA(bridge_in(e, s));
-    if (lpips_set_bank(e->lp, d_crops, M, e->work, &e->launches)) return fail(-7, "lpips: %s", lpips_last_error());
+    if (lpips_set_bank(e->lp, d_crops, M, e->work, &e->launches)) return -7;
     LA(bridge_out(e, s));
     return 0;
 }
@@ -994,7 +970,7 @@ LA_API int la_lpips_loss_grad(la_engine* e, const float* d_img, int crop_x, int 
         if (crop_x != 0 || crop_y != 0) return fail(-2, "norm_mode 2 (per-sample targets) uses the whole image: crop_x = crop_y = 0");
         if (lpips_set_call(e->lp, 0, 0, 1.f, 1, e->work) || lpips_forward(e->lp, top.img, 1, e->work, &e->launches) ||
             lpips_backward(e->lp, top.g_img, 0, e->lpips_loss, 1, e->work, &e->launches))
-            return fail(-7, "lpips: %s", lpips_last_error());
+            return -7;
         LA(f4_to_nchw(top.g_img, e->batch, e->g.img_channels, e->g.img_resolution, d_grad, e->work));
         CU(cudaMemcpyAsync(d_loss, e->lpips_loss, sizeof(float) * e->batch, cudaMemcpyDeviceToDevice, e->work));
         LA(bridge_out(e, s));
@@ -1003,7 +979,7 @@ LA_API int la_lpips_loss_grad(la_engine* e, const float* d_img, int crop_x, int 
     // (the term enters the objective with a minus sign; the stand-alone call returns d loss / d img, hence -w)
     if (lpips_set_call(e->lp, crop_x, crop_y, -w_lpips, norm_mode, e->work) ||
         lpips_forward(e->lp, top.img, 0, e->work, &e->launches) || lpips_backward(e->lp, top.g_img, 0, e->lpips_loss, 0, e->work, &e->launches))
-        return fail(-7, "lpips: %s", lpips_last_error());
+        return -7;
     LA(f4_to_nchw(top.g_img, e->batch, e->g.img_channels, e->g.img_resolution, d_grad, e->work));
     LA(prep_scale(e->lpips_loss, -1.f, e->lpips_loss, 1, e->work));
     CU(cudaMemcpyAsync(d_loss, e->lpips_loss, sizeof(float), cudaMemcpyDeviceToDevice, e->work));
@@ -1015,7 +991,7 @@ LA_API int la_lpips_tap(la_engine* e, int k, float* d_out, size_t* count, la_str
     if (!e || !e->lp) return fail(-2, "bad arguments (la_set_lpips first)");
     cudaStream_t s = static_cast<cudaStream_t>(stream);
     if (d_out) LA(bridge_in(e, s));
-    if (lpips_copy_tap(e->lp, k, d_out, count, e->work)) return fail(-7, "lpips: %s", lpips_last_error());
+    if (lpips_copy_tap(e->lp, k, d_out, count, e->work)) return -7;
     if (d_out) LA(bridge_out(e, s));
     return 0;
 }

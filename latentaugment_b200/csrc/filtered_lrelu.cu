@@ -13,8 +13,7 @@
 #include <stdint.h>
 
 #include "../../include/latentaugment_b200.h"
-
-int la_fail_msg(int code, const char* msg);   // engine.cu
+#include "common.cuh"
 
 namespace {
 
@@ -155,9 +154,9 @@ int la_filtered_lrelu(const float* d_x, int N, int C, int H, int W, const float*
                       const float* d_b, int up, int down, int px0, int px1, int py0, int py1, float gain, float slope, float clamp,
                       int flip_filter, const signed char* d_mask_in, signed char* d_mask_out, int mask_oy, int mask_ox, int mask_h, int mask_w,
                       float* d_y, la_stream stream) {
-    if (!d_x || !d_y || N < 1 || C < 1 || H < 1 || W < 1) return la_fail_msg(-2, "filtered_lrelu: bad arguments");
-    if (up < 1 || up > 4 || down < 1 || down > 4) return la_fail_msg(-2, "filtered_lrelu: up and down must be 1..4");
-    if (fu_taps < 0 || fu_taps > kMaxTaps || fd_taps < 0 || fd_taps > kMaxTaps) return la_fail_msg(-2, "filtered_lrelu: at most 32 separable taps per filter");
+    if (!d_x || !d_y || N < 1 || C < 1 || H < 1 || W < 1) return la::fail(-2, "filtered_lrelu: bad arguments");
+    if (up < 1 || up > 4 || down < 1 || down > 4) return la::fail(-2, "filtered_lrelu: up and down must be 1..4");
+    if (fu_taps < 0 || fu_taps > kMaxTaps || fd_taps < 0 || fd_taps > kMaxTaps) return la::fail(-2, "filtered_lrelu: at most 32 separable taps per filter");
     FlParams P{};
     P.x = d_x; P.b = d_b; P.y = d_y; P.mask_in = reinterpret_cast<const int8_t*>(d_mask_in); P.mask_out = reinterpret_cast<int8_t*>(d_mask_out);
     P.N = N; P.C = C; P.H = H; P.W = W; P.up = up; P.down = down; P.px0 = px0; P.py0 = py0;
@@ -171,7 +170,7 @@ int la_filtered_lrelu(const float* d_x, int N, int C, int H, int W, const float*
     P.mid_h = H * up + py0 + py1 - (P.fu_taps - 1);
     P.out_w = (P.mid_w - (P.fd_taps - 1) + down - 1) / down;
     P.out_h = (P.mid_h - (P.fd_taps - 1) + down - 1) / down;
-    if (P.mid_w < 1 || P.mid_h < 1 || P.out_w < 1 || P.out_h < 1) return la_fail_msg(-2, "filtered_lrelu: empty output");
+    if (P.mid_w < 1 || P.mid_h < 1 || P.out_w < 1 || P.out_h < 1) return la::fail(-2, "filtered_lrelu: empty output");
     if (d_mask_in || d_mask_out) {
         if (mask_h < 1 || mask_w < 1) { mask_oy = mask_ox = 0; mask_h = P.mid_h; mask_w = P.mid_w; }
         P.mask_oy = mask_oy; P.mask_ox = mask_ox; P.mask_h = mask_h; P.mask_w = mask_w;
@@ -180,8 +179,8 @@ int la_filtered_lrelu(const float* d_x, int N, int C, int H, int W, const float*
     P.in_t = (P.mid_t + P.fu_taps - 1 + up - 1) / up + 1;
     const size_t smem = sizeof(float) * (static_cast<size_t>(P.in_t) * P.in_t + static_cast<size_t>(P.in_t) * P.mid_t +
                                          static_cast<size_t>(P.mid_t) * P.mid_t + static_cast<size_t>(P.mid_t) * kTile + 2 * kMaxTaps);
-    if (P.mid_t > 256 || P.in_t > 256) return la_fail_msg(-2, "filtered_lrelu: filter footprint too large for one tile");
-    if (smem > 200 * 1024) return la_fail_msg(-2, "filtered_lrelu: filter footprint too large for one tile");
+    if (P.mid_t > 256 || P.in_t > 256) return la::fail(-2, "filtered_lrelu: filter footprint too large for one tile");
+    if (smem > 200 * 1024) return la::fail(-2, "filtered_lrelu: filter footprint too large for one tile");
     dim3 grid((P.out_w + kTile - 1) / kTile, (P.out_h + kTile - 1) / kTile, N * C);
     cudaStream_t cs = static_cast<cudaStream_t>(stream);
     cudaError_t e = cudaSuccess;
@@ -200,8 +199,7 @@ int la_filtered_lrelu(const float* d_x, int N, int C, int H, int W, const float*
         default: LA_FL(0, 0, 0, 0); break;
     }
 #undef LA_FL
-    if (e != cudaSuccess) return la_fail_msg(static_cast<int>(e), cudaGetErrorString(e));
-    e = cudaGetLastError();
-    if (e != cudaSuccess) return la_fail_msg(static_cast<int>(e), cudaGetErrorString(e));
+    if (e == cudaSuccess) e = cudaGetLastError();
+    if (e != cudaSuccess) return la::fail(static_cast<int>(e), "filtered_lrelu: %s", cudaGetErrorString(e));
     return 0;
 }

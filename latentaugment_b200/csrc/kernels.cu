@@ -4,28 +4,13 @@
 #include <cuda_bf16.h>
 
 #include "act.cuh"
+#include "common.cuh"
 #include "sm100.cuh"
 
 namespace la {
 
 namespace {
 
-__device__ __forceinline__ float warp_sum(float v) {
-#pragma unroll
-    for (int o = 16; o >= 1; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-    return v;
-}
-__device__ __forceinline__ double warp_sum_d(double v) {
-#pragma unroll
-    for (int o = 16; o >= 1; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-    return v;
-}
-__device__ __forceinline__ void split_store(__nv_bfloat16* hi, __nv_bfloat16* lo, long long i, float v) {
-    const __nv_bfloat16 h = __float2bfloat16_rn(v);
-    hi[i] = h;
-    if (lo) lo[i] = __float2bfloat16_rn(v - __bfloat162float(h));
-}
-inline int cdiv(long long a, long long b) { return static_cast<int>((a + b - 1) / b); }
 inline int last_err() { return static_cast<int>(cudaGetLastError()); }
 
 // ------------------------------------------------------------------------- weight preparation
@@ -55,8 +40,8 @@ __global__ void prep_conv_weights_kernel(const float* __restrict__ w, int cout, 
     if (up == 1) {
         for (int a = 0; a < 9; ++a) {
             const float v = k[a / 3][a % 3];
-            split_store(wf, wf_lo, a * msz + static_cast<long long>(o) * cin + i, v);
-            split_store(wb, wb_lo, a * msz + static_cast<long long>(i) * cout + o, v);
+            st_sp(wf, wf_lo, a * msz + static_cast<long long>(o) * cin + i, v);
+            st_sp(wb, wb_lo, a * msz + static_cast<long long>(i) * cout + o, v);
         }
     } else {
         for (int py = 0; py < 2; ++py)
@@ -74,10 +59,25 @@ __global__ void prep_conv_weights_kernel(const float* __restrict__ w, int cout, 
                             }
                         }
                         const int m = (py * 2 + px) * 9 + (dy + 1) * 3 + (dx + 1);
-                        split_store(wf, wf_lo, m * msz + static_cast<long long>(o) * cin + i, v);
-                        split_store(wb, wb_lo, m * msz + static_cast<long long>(i) * cout + o, v);
+                        st_sp(wf, wf_lo, m * msz + static_cast<long long>(o) * cin + i, v);
+                        st_sp(wb, wb_lo, m * msz + static_cast<long long>(i) * cout + o, v);
                     }
     }
+}
+
+// Plain (unmodulated) conv: w [cout, cin, k, k] -> wf [k*k][cout][cin_pad] and, unless wb is null, wb [k*k][cin_pad][cout],
+// both * scale, zero padded; with split the bf16 residual planes follow as a second stack of k*k matrices.
+__global__ void prep_plain_weights_kernel(const float* __restrict__ w, int cout, int cin, int k2, float scale, int cin_pad, int split,
+                                          __nv_bfloat16* wf, __nv_bfloat16* wb) {
+    const long long idx = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x;
+    const long long total = static_cast<long long>(k2) * cout * cin_pad;
+    if (idx >= total) return;
+    const int i = static_cast<int>(idx % cin_pad);
+    const int o = static_cast<int>((idx / cin_pad) % cout);
+    const int t = static_cast<int>(idx / (static_cast<long long>(cin_pad) * cout));
+    const float v = i < cin ? w[(static_cast<long long>(o) * cin + i) * k2 + t] * scale : 0.f;
+    st_sp(wf, split ? wf + total : nullptr, idx, v);
+    if (wb) st_sp(wb, split ? wb + total : nullptr, (static_cast<long long>(t) * cin_pad + i) * cout + o, v);
 }
 
 __global__ void prep_affine_kernel(const float* __restrict__ aw, const float* __restrict__ ab, int cin, int w_dim,
@@ -91,6 +91,10 @@ __global__ void prep_scale_kernel(const float* __restrict__ src, float scale, fl
     const long long idx = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x;
     if (idx < n) dst[idx] = src[idx] * scale;
 }
+__global__ void fill_kernel(float* p, float v, long long n) {
+    const long long i = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x;
+    if (i < n) p[i] = v;
+}
 
 __global__ void prep_const_kernel(const float* __restrict__ cst, int C, int hw, float* c_f32, __nv_bfloat16* hi,
                                   __nv_bfloat16* lo) {
@@ -99,7 +103,7 @@ __global__ void prep_const_kernel(const float* __restrict__ cst, int C, int hw, 
     const int p = idx / C, c = idx % C;
     const float v = cst[c * hw + p];
     c_f32[idx] = v;
-    split_store(hi, lo, idx, v);
+    st_sp(hi, lo, idx, v);
 }
 
 constexpr int kMaxRowRegs = 32;   // mapping network: a weight row of up to 1024 floats stays in a warp's registers
@@ -230,19 +234,10 @@ __global__ void const_modulate_kernel(const float* __restrict__ c_f32, const flo
     const int c = static_cast<int>(idx % C);
     const int p = static_cast<int>((idx / C) % hw);
     const int n = static_cast<int>(idx / (static_cast<long long>(C) * hw));
-    split_store(hi, lo, idx, c_f32[p * C + c] * s0[static_cast<long long>(n) * C + c]);
+    st_sp(hi, lo, idx, c_f32[p * C + c] * s0[static_cast<long long>(n) * C + c]);
 }
 
 // ------------------------------------------------------------------------- x2 up-sampling FIR passes
-__device__ __forceinline__ unsigned pack2(float a, float b) {
-    __nv_bfloat162 v = __floats2bfloat162_rn(a, b);
-    return *reinterpret_cast<unsigned*>(&v);
-}
-__device__ __forceinline__ void st_bf16x2(unsigned* hi, unsigned* lo, long long i, float a, float b) {
-    hi[i] = pack2(a, b);
-    if (lo) lo[i] = pack2(a - __bfloat162float(__float2bfloat16_rn(a)), b - __bfloat162float(__float2bfloat16_rn(b)));
-}
-
 // Sliding-window 4x4 FIR.  A block = (256 / cpb) consecutive output rows x cpb channel pairs; every thread
 // walks 32 output pixels along x keeping the 4x4 source window of its channel pair in registers, so each
 // step loads one new window column (4 coalesced 128-byte rows per warp) instead of 16 values; the 4-row
@@ -362,7 +357,7 @@ __global__ void __launch_bounds__(256, SEP ? 3 : 2) upfir_slide_kernel(const __g
                 const float s1 = __uint_as_float(sv & 0xffff0000u) + __uint_as_float(svl & 0xffff0000u);
                 const float thr = act_saved_clamp(P.act_clamp, P.act_saved_lo != nullptr);
                 const float g0 = act_grad(a0 * P.act_gain, s0, P.act_slope, thr), g1 = act_grad(a1 * P.act_gain, s1, P.act_slope, thr);
-                st_bf16x2(oh, ol, o, g0, g1);
+                st_sp2(oh, ol, o, g0, g1);
             } else if (FWD) {
                 float z0 = fmaf(a0, dm.x, nzv[u]) + bs.x, z1 = fmaf(a1, dm.y, nzv[u]) + bs.y;
                 z0 = (z0 > 0.f ? z0 : z0 * P.act_slope) * P.act_gain;
@@ -371,10 +366,10 @@ __global__ void __launch_bounds__(256, SEP ? 3 : 2) upfir_slide_kernel(const __g
                     z0 = fminf(fmaxf(z0, -P.act_clamp), P.act_clamp);
                     z1 = fminf(fmaxf(z1, -P.act_clamp), P.act_clamp);
                 }
-                st_bf16x2(oh, ol, o, z0, z1);
-                if (P.s_next) st_bf16x2(xsh, xsl, o, z0 * sn.x, z1 * sn.y);
+                st_sp2(oh, ol, o, z0, z1);
+                if (P.s_next) st_sp2(xsh, xsl, o, z0 * sn.x, z1 * sn.y);
             } else {
-                st_bf16x2(oh, ol, o, a0, a1);
+                st_sp2(oh, ol, o, a0, a1);
             }
         }
 #pragma unroll
@@ -1046,6 +1041,12 @@ int prep_conv_weights(const float* w, int cout, int cin, int up, const float* fi
                                                           static_cast<__nv_bfloat16*>(wb), w2, w2t);
     return last_err();
 }
+int prep_plain_weights(const float* w, int cout, int cin, int k2, float scale, int cin_pad, int split, __nv_bfloat16* wf,
+                       __nv_bfloat16* wb, cudaStream_t s) {
+    const long long total = static_cast<long long>(k2) * cout * cin_pad;
+    prep_plain_weights_kernel<<<cdiv(total, 256), 256, 0, s>>>(w, cout, cin, k2, scale, cin_pad, split, wf, wb);
+    return last_err();
+}
 int prep_affine(const float* aw, const float* ab, int cin, int w_dim, float wscale, float bscale, float* a_rows, float* b_rows,
                 cudaStream_t s) {
     prep_affine_kernel<<<cdiv(static_cast<long long>(cin) * w_dim, 256), 256, 0, s>>>(aw, ab, cin, w_dim, wscale, bscale, a_rows, b_rows);
@@ -1061,6 +1062,10 @@ int prep_axpy(const float* x, float a, float* y, long long n, cudaStream_t s) {
 }
 int prep_scale(const float* src, float scale, float* dst, long long n, cudaStream_t s) {
     prep_scale_kernel<<<cdiv(n, 256), 256, 0, s>>>(src, scale, dst, n);
+    return last_err();
+}
+int fill(float* p, float v, long long n, cudaStream_t s) {
+    fill_kernel<<<cdiv(n, 256), 256, 0, s>>>(p, v, n);
     return last_err();
 }
 int prep_const(const float* cst, int C, int hw, float* c_f32, void* hi, void* lo, cudaStream_t s) {

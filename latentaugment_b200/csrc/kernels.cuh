@@ -3,6 +3,7 @@
 // the fused Adam step on w, the mapping network and bank statistics.
 #pragma once
 #include <cuda.h>
+#include <cuda_bf16.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
 
@@ -35,9 +36,14 @@ struct LayerTable {
 // ---- one-time preparation
 int prep_conv_weights(const float* w, int cout, int cin, int up, const float* fir4x4, int split, void* wf, void* wb,
                       float* w2, float* w2t, cudaStream_t s);
+// Plain conv w [cout, cin, k, k] (k2 = k*k) -> wf [k2][cout][cin_pad] and, unless wb is null, wb [k2][cin_pad][cout], both
+// * scale, zero padded; split: residual planes behind the main ones.
+int prep_plain_weights(const float* w, int cout, int cin, int k2, float scale, int cin_pad, int split, __nv_bfloat16* wf,
+                       __nv_bfloat16* wb, cudaStream_t s);
 int prep_affine(const float* aw, const float* ab, int cin, int w_dim, float wscale, float bscale, float* a_cat_rows,
                 float* b_cat_rows, cudaStream_t s);
 int prep_scale(const float* src, float scale, float* dst, long long n, cudaStream_t s);
+int fill(float* p, float v, long long n, cudaStream_t s);
 int prep_axpy(const float* x, float a, float* y, long long n, cudaStream_t s);      // y += a x
 int prep_const(const float* cst /*[C,4,4]*/, int C, int hw, float* c_f32 /*[hw][C]*/, void* hi, void* lo, cudaStream_t s);
 

@@ -15,12 +15,10 @@
 
 #include <cuda_bf16.h>
 #include <math.h>
-#include <stdarg.h>
-#include <stdio.h>
 #include <string.h>
 
-#include <string>
-
+#include "common.cuh"
+#include "kernels.cuh"
 #include "plan.cuh"
 #include "tapgemm.cuh"
 #include "vgg.cuh"
@@ -29,61 +27,11 @@ using namespace la;
 
 namespace {
 
+constexpr char kModule[] = "lpips";
 typedef __nv_bfloat16 bf16;
-thread_local std::string g_lerr;
-
-int lfail(int code, const char* fmt, ...) {
-    char buf[512];
-    va_list ap;
-    va_start(ap, fmt);
-    vsnprintf(buf, sizeof buf, fmt, ap);
-    va_end(ap);
-    g_lerr = buf;
-    return code ? code : -1;
-}
-#define LCU(x)                                                                                               \
-    do {                                                                                                     \
-        cudaError_t e_ = (x);                                                                                \
-        if (e_ != cudaSuccess) return lfail(static_cast<int>(e_), "%s: %s (%s:%d)", #x, cudaGetErrorString(e_), __FILE__, __LINE__); \
-    } while (0)
-#define LLA(x)                                                                                               \
-    do {                                                                                                     \
-        int r_ = (x);                                                                                        \
-        if (r_) return lfail(r_, "%s failed (%d) (%s:%d)", #x, r_, __FILE__, __LINE__);                      \
-    } while (0)
-
-inline int cdiv(long long a, long long b) { return static_cast<int>((a + b - 1) / b); }
 
 static_assert(kNConv == LA_VGG_CONVS, "VGG16 has 13 convolutions");
 const int kTapConv[LA_VGG_TAPS] = {1, 3, 6, 9, 12};                        // conv whose ReLU output is tap t (a pool follows 1, 3, 6, 9)
-
-__device__ __forceinline__ float warp_sum(float v) {
-#pragma unroll
-    for (int o = 16; o >= 1; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-    return v;
-}
-__device__ __forceinline__ unsigned pack2(float a, float b) {
-    __nv_bfloat162 v = __floats2bfloat162_rn(a, b);
-    return *reinterpret_cast<unsigned*>(&v);
-}
-__device__ __forceinline__ float lo_f(unsigned u) { return __uint_as_float(u << 16); }
-__device__ __forceinline__ float hi_f(unsigned u) { return __uint_as_float(u & 0xffff0000u); }
-__device__ __forceinline__ float rnd(float v) { return __bfloat162float(__float2bfloat16_rn(v)); }
-__device__ __forceinline__ void st_sp(bf16* hi, bf16* lo, long long i, float v) {
-    const bf16 h = __float2bfloat16_rn(v);
-    hi[i] = h;
-    if (lo) lo[i] = __float2bfloat16_rn(v - __bfloat162float(h));
-}
-__device__ __forceinline__ void st_sp2(unsigned* hi, unsigned* lo, long long i, float a, float b) {
-    hi[i] = pack2(a, b);
-    if (lo) lo[i] = pack2(a - rnd(a), b - rnd(b));
-}
-__device__ __forceinline__ float2 ld_sp2(const unsigned* hi, const unsigned* lo, long long i) {
-    const unsigned u = __ldg(hi + i);
-    float2 v = make_float2(lo_f(u), hi_f(u));
-    if (lo) { const unsigned l = __ldg(lo + i); v.x += lo_f(l); v.y += hi_f(l); }
-    return v;
-}
 
 // per-call constants, device resident (one captured graph serves every call)
 struct CallConsts {
@@ -91,25 +39,6 @@ struct CallConsts {
     float w_lpips;
     float norm;              // pair normaliser: 1 / n (lpips_script form) or 1 (forward_tr form)
 };
-
-// ------------------------------------------------------------------------- weights
-// w [cout, cin, 3, 3] fp32 -> wf [9][cout][cin_pad] and wb [9][cin_pad][cout] (zero padded; wb may be null); split: residual
-// planes follow
-__global__ void prep_vgg_weights_kernel(const float* __restrict__ w, int cout, int cin, int cin_pad, int split, bf16* wf, bf16* wb) {
-    const long long idx = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x;
-    const long long total = 9LL * cout * cin_pad;
-    if (idx >= total) return;
-    const int i = static_cast<int>(idx % cin_pad);
-    const int o = static_cast<int>((idx / cin_pad) % cout);
-    const int t = static_cast<int>(idx / (static_cast<long long>(cin_pad) * cout));
-    const float v = i < cin ? w[(static_cast<long long>(o) * cin + i) * 9 + t] : 0.f;
-    st_sp(wf, split ? wf + total : nullptr, idx, v);
-    if (wb) st_sp(wb, split ? wb + total : nullptr, (static_cast<long long>(t) * cin_pad + i) * cout + o, v);
-}
-__global__ void fill_kernel(float* p, float v, long long n) {
-    const long long i = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x;
-    if (i < n) p[i] = v;
-}
 
 // ------------------------------------------------------------------------- crop (+ replicate + z-score) and its adjoint
 // x_in [crop = b*imgc + c][y][x][64]: channels 0..2 = (img[b, cy+y, cx+x].c - mean_k) / std_k, 3..63 = 0.
@@ -367,17 +296,6 @@ __global__ void lpips_target_loss_kernel(const double* S, int batch, float* loss
     for (int b = threadIdx.x; b < batch; b += blockDim.x) loss[b] = static_cast<float>(S[b]);
 }
 
-struct Bump {
-    char* base = nullptr;
-    size_t off = 0;
-    template <class T>
-    T* take(size_t count) {
-        off = (off + 1023) & ~size_t(1023);
-        T* p = base ? reinterpret_cast<T*>(base + off) : nullptr;
-        off += count * sizeof(T);
-        return p;
-    }
-};
 struct Conv {
     int R, cin, cin_pad, cout;
     bf16 *wf, *wb;
@@ -412,19 +330,12 @@ struct la_lpips {
 
 namespace {
 
-int choose_bn(int n, long long m_tiles) { return n % 128 ? 64 : pick_bn(n, m_tiles); }
 // blocks of 8 warps, a warp per pixel, grid-stride: at most 8 resident blocks per SM
 inline int tap_grid(long long pixels, int num_sms) {
     const long long want = (pixels + 7) / 8, cap = static_cast<long long>(num_sms > 0 ? num_sms : 148) * 8;
     return static_cast<int>(want < cap ? want : cap);
 }
 
-int dense_maps(int n, int split, TapGemmParams& P, const Pl& t, int C, int R) {
-    const long long sW = C, sH = static_cast<long long>(R) * C, sN = sH * R;
-    if (make_a_map(&P.a_map[0], t.hi, C, R, R, n, sW, sH, sN, P.tw, P.th + P.halo, P.nb)) return -1;
-    if (split && make_a_map(&P.a_map[1], t.lo, C, R, R, n, sW, sH, sN, P.tw, P.th + P.halo, P.nb)) return -1;
-    return 0;
-}
 int conv_taps(int split, TapGemmParams& P, bool flipped) {
     int nt = 0;
     P.prob[0].tap_begin = 0;
@@ -439,9 +350,9 @@ int conv_taps(int split, TapGemmParams& P, bool flipped) {
 int plan_lpips(la_lpips* L, char* ws, size_t* bytes_out) {
     const la_vgg_desc& d = L->d;
     const int cs = d.crop_size, split = L->split;
-    if (cs < 64 || (cs & (cs - 1))) return lfail(-2, "lpips: crop_size %d unsupported (power of two >= 64)", cs);
-    if (L->imgc < 1 || L->imgc > 3) return lfail(-2, "lpips: img_channels must be 1..3");
-    if (cs > L->res) return lfail(-2, "lpips: crop %d larger than the image %d", cs, L->res);
+    if (cs < 64 || (cs & (cs - 1))) return fail(-2, "lpips: crop_size %d unsupported (power of two >= 64)", cs);
+    if (L->imgc < 1 || L->imgc > 3) return fail(-2, "lpips: img_channels must be 1..3");
+    if (cs > L->res) return fail(-2, "lpips: crop %d larger than the image %d", cs, L->res);
     L->cs = cs;
     L->ncrops = L->batch * L->imgc;
     L->last_conv = -1; L->ntaps_used = 0;
@@ -451,7 +362,7 @@ int plan_lpips(la_lpips* L, char* ws, size_t* bytes_out) {
         T.conv = kTapConv[t]; T.C = kCout[T.conv]; T.R = cs >> kShift[T.conv]; T.lin_w = d.d_lin_weight[t];
         if (T.used) { L->last_conv = T.conv; ++L->ntaps_used; }
     }
-    if (L->last_conv < 0) return lfail(-2, "lpips: no tap has a lin weight");
+    if (L->last_conv < 0) return fail(-2, "lpips: no tap has a lin weight");
     Bump bp;
     bp.base = ws;
     const size_t n = L->ncrops, wm = split ? 2 : 1;
@@ -503,14 +414,14 @@ int build_lpips(la_lpips* L) {
         int pk = -1;
         for (int k = 0; k < 4; ++k) if (kTapConv[k] + 1 == i) { pooled_in = true; pk = k; }
         const Pl& in = i == 0 ? L->x_in : (pooled_in ? L->pool[pk] : L->conv[i - 1].x);
-        LLA(vgg_conv_fwd_plan(c.F, c.R, L->ncrops, c.cin_pad, c.cout, in, c.wf, split, L->d.d_conv_bias[i], L->ones, c.x, L->err_flag));
+        LA(vgg_conv_fwd_plan(c.F, c.R, L->ncrops, c.cin_pad, c.cout, in, c.wf, split, L->d.d_conv_bias[i], L->ones, c.x, L->err_flag));
         {   // data gradient: g_z (wrt this conv's pre-activation) -> gradient wrt its input
             TapGemmParams& P = c.B;
             memset(&P, 0, sizeof P);
             set_grid(P, c.R, L->ncrops, 1);
-            LLA(dense_maps(L->ncrops, split, P, L->gz[i & 1], c.cout, c.R));
+            LA(dense_maps(P, L->gz[i & 1], L->ncrops, c.cout, c.R, c.R, P.tw, P.th + P.halo, P.nb, split));
             const int bn = choose_bn(c.cin_pad, P.m_tiles);
-            LLA(make_b_map(P, c.wb, c.cout, c.cin_pad, 9 * wm, bn));
+            LA(make_b_map(P, c.wb, c.cout, c.cin_pad, 9 * wm, bn));
             P.kchunks = c.cout / 64;
             P.epilogue = kEpiLinear;
             P.n_total = c.cin_pad; P.n_blocks = c.cin_pad / bn;
@@ -520,7 +431,7 @@ int build_lpips(la_lpips* L) {
             else if (pooled_in) { P.lin_out = L->gp.hi; P.lin_out_lo = L->gp.lo; }
             else { P.lin_saved = L->conv[i - 1].x.hi; P.lin_gz = L->gz[(i - 1) & 1].hi; P.lin_gz_lo = L->gz[(i - 1) & 1].lo; }
             P.err_flag = L->err_flag;
-            LLA(conv_taps(split, P, true));
+            LA(conv_taps(split, P, true));
         }
     }
     return 0;
@@ -529,17 +440,16 @@ int build_lpips(la_lpips* L) {
 int prepare_lpips(la_lpips* L, cudaStream_t s) {
     for (int i = 0; i <= L->last_conv; ++i) {
         Conv& c = L->conv[i];
-        if (!L->d.d_conv_weight[i] || !L->d.d_conv_bias[i]) return lfail(-2, "lpips: missing parameters of conv %d", i);
-        LLA(vgg_prep_weights(L->d.d_conv_weight[i], c.cout, c.cin, c.cin_pad, L->split, c.wf, c.wb, s));
+        if (!L->d.d_conv_weight[i] || !L->d.d_conv_bias[i]) return fail(-2, "lpips: missing parameters of conv %d", i);
+        LA(vgg_prep_weights(L->d.d_conv_weight[i], c.cout, c.cin, c.cin_pad, L->split, c.wf, c.wb, s));
     }
     const long long n_ones = static_cast<long long>(L->ncrops) * 512;
-    fill_kernel<<<cdiv(n_ones, 256), 256, 0, s>>>(L->ones, 1.f, n_ones);
-    LCU(cudaGetLastError());
-    LCU(cudaMemsetAsync(L->err_flag, 0, sizeof(int), s));
-    LCU(cudaMemsetAsync(L->m2, 0, 4 * sizeof(float), s));
-    LCU(cudaMemsetAsync(L->S, 0, sizeof(double) * L->batch, s));
-    LCU(cudaMemsetAsync(L->cc, 0, sizeof(CallConsts), s));
-    LCU(cudaStreamSynchronize(s));
+    LA(fill(L->ones, 1.f, n_ones, s));
+    CU(cudaMemsetAsync(L->err_flag, 0, sizeof(int), s));
+    CU(cudaMemsetAsync(L->m2, 0, 4 * sizeof(float), s));
+    CU(cudaMemsetAsync(L->S, 0, sizeof(double) * L->batch, s));
+    CU(cudaMemsetAsync(L->cc, 0, sizeof(CallConsts), s));
+    CU(cudaStreamSynchronize(s));
     return 0;
 }
 
@@ -550,11 +460,11 @@ inline const unsigned* CU32(const bf16* p) { return reinterpret_cast<const unsig
 int run_network(la_lpips* L, cudaStream_t s, long long* launches) {
     for (int i = 0; i <= L->last_conv; ++i) {
         Conv& c = L->conv[i];
-        LLA(launch_tapgemm(c.F, L->num_sms, s));
+        LA(launch_tapgemm(c.F, L->num_sms, s));
         if (launches) ++*launches;
         for (int k = 0; k < 4; ++k)
             if (kTapConv[k] == i && i + 1 <= L->last_conv) {
-                LLA(vgg_pool_fwd(c.x, L->ncrops, c.R, c.cout, L->pool[k], s));
+                LA(vgg_pool_fwd(c.x, L->ncrops, c.R, c.cout, L->pool[k], s));
                 if (launches) ++*launches;
             }
     }
@@ -565,13 +475,8 @@ int run_network(la_lpips* L, cudaStream_t s, long long* launches) {
 
 namespace la {
 
-const char* lpips_last_error() { return g_lerr.c_str(); }
-
 int vgg_prep_weights(const float* w, int cout, int cin, int cin_pad, int split, bf16* wf, bf16* wb, cudaStream_t s) {
-    const long long total = 9LL * cout * cin_pad;
-    prep_vgg_weights_kernel<<<cdiv(total, 256), 256, 0, s>>>(w, cout, cin, cin_pad, split, wf, wb);
-    LCU(cudaGetLastError());
-    return 0;
+    return prep_plain_weights(w, cout, cin, 9, 1.f, cin_pad, split, wf, wb, s);
 }
 
 int vgg_conv_fwd_plan(TapGemmParams& P, int R, int n, int cin_pad, int cout, const Pl& in, const bf16* wf, int split, const float* bias,
@@ -579,9 +484,9 @@ int vgg_conv_fwd_plan(TapGemmParams& P, int R, int n, int cin_pad, int cout, con
     const int wm = split ? 2 : 1;
     memset(&P, 0, sizeof P);
     set_grid(P, R, n, 1);
-    LLA(dense_maps(n, split, P, in, cin_pad, R));
+    LA(dense_maps(P, in, n, cin_pad, R, R, P.tw, P.th + P.halo, P.nb, split));
     const int bn = choose_bn(cout, P.m_tiles);
-    LLA(make_b_map(P, wf, cin_pad, cout, 9 * wm, bn));
+    LA(make_b_map(P, wf, cin_pad, cout, 9 * wm, bn));
     P.kchunks = cin_pad / 64;
     P.epilogue = kEpiFwd;
     P.n_total = cout; P.n_blocks = cout / bn;
@@ -591,14 +496,14 @@ int vgg_conv_fwd_plan(TapGemmParams& P, int R, int n, int cin_pad, int cout, con
     P.x_hi = out.hi; P.x_lo = out.lo;
     P.staged = P.nb == 1 && !split && !getenv("LA_NO_STAGED");
     P.err_flag = err_flag;
-    LLA(conv_taps(split, P, false));
+    LA(conv_taps(split, P, false));
     return 0;
 }
 
 int vgg_pool_fwd(const Pl& x, int n, int R, int C, const Pl& out, cudaStream_t s) {
     const long long total = static_cast<long long>(n) * (R / 2) * (R / 2) * (C / 2);
     pool_fwd_kernel<<<cdiv(total, 256), 256, 0, s>>>(CU32(x.hi), CU32(x.lo), n, R, C, U32(out.hi), U32(out.lo));
-    LCU(cudaGetLastError());
+    CU(cudaGetLastError());
     return 0;
 }
 int lpips_has_bank(const la_lpips* L) { return L->has_bank; }
@@ -617,7 +522,7 @@ int lpips_create(const la_vgg_desc& d, int batch, int img_channels, int img_reso
     la_lpips* L = new la_lpips{};
     L->d = d; L->batch = batch; L->imgc = img_channels; L->res = img_resolution; L->split = split; L->num_sms = num_sms;
     for (int k = 0; k < 3; ++k) {
-        if (!(d.std[k] > 0.f)) { delete L; return lfail(-2, "lpips: std[%d] must be positive", k); }
+        if (!(d.std[k] > 0.f)) { delete L; return fail(-2, "lpips: std[%d] must be positive", k); }
         L->z.mean[k] = d.mean[k]; L->z.inv_std[k] = 1.f / d.std[k];
     }
     L->pool_f = 1;
@@ -625,14 +530,13 @@ int lpips_create(const la_vgg_desc& d, int batch, int img_channels, int img_reso
         if (img_resolution > 512 || (d.crop_size != img_resolution && 2 * d.crop_size != img_resolution) ||
             d.crop_size != (img_resolution < 256 ? img_resolution : 256)) {
             delete L;
-            return lfail(-2, "lpips: per-sample targets need crop_size == min(res, 256) and res <= 512 (crop %d, res %d)", d.crop_size, img_resolution);
+            return fail(-2, "lpips: per-sample targets need crop_size == min(res, 256) and res <= 512 (crop %d, res %d)", d.crop_size, img_resolution);
         }
         L->pool_f = img_resolution / d.crop_size;
     }
     size_t need = 0;
     int r = plan_lpips(L, static_cast<char*>(ws), &need);
-    if (!r && need > bytes) r = lfail(-2, "lpips workspace too small: %zu < %zu", bytes, need);
-    if (!r && (reinterpret_cast<uintptr_t>(ws) & 1023)) r = lfail(-2, "lpips workspace must be 1024-byte aligned");
+    if (!r) r = check_workspace(kModule, need, bytes, ws);
     if (!r) r = build_lpips(L);
     if (!r) r = prepare_lpips(L, s);
     if (r) { delete L; return r; }
@@ -644,26 +548,26 @@ void lpips_destroy(la_lpips* L) { delete L; }
 
 int lpips_set_call(la_lpips* L, int crop_x, int crop_y, float w_lpips, int norm_mode, cudaStream_t s) {
     if (crop_x < 0 || crop_y < 0 || crop_x + L->cs > L->res || crop_y + L->cs > L->res)
-        return lfail(-2, "lpips: crop window (%d, %d) + %d leaves the %d x %d image", crop_x, crop_y, L->cs, L->res, L->res);
+        return fail(-2, "lpips: crop window (%d, %d) + %d leaves the %d x %d image", crop_x, crop_y, L->cs, L->res, L->res);
     // (staged through pageable host memory: the copy is complete when the call returns, so the stack value may die)
     const CallConsts h{crop_x, crop_y, w_lpips, norm_mode ? 1.f : 1.f / static_cast<float>(L->batch)};
-    LCU(cudaMemcpyAsync(L->cc, &h, sizeof h, cudaMemcpyHostToDevice, s));
+    CU(cudaMemcpyAsync(L->cc, &h, sizeof h, cudaMemcpyHostToDevice, s));
     return 0;
 }
 
 int lpips_set_bank(la_lpips* L, const float* d_crops, int M, cudaStream_t s, long long* launches) {
-    if (M < 1) return lfail(-2, "lpips: empty bank");
+    if (M < 1) return fail(-2, "lpips: empty bank");
     for (int t = 0; t < LA_VGG_TAPS; ++t)
         if (L->tap[t].used)
-            LCU(cudaMemsetAsync(L->tap[t].bank_mean, 0, sizeof(float) * static_cast<size_t>(L->imgc) * L->tap[t].R * L->tap[t].R * L->tap[t].C, s));
-    LCU(cudaMemsetAsync(L->m2, 0, 4 * sizeof(float), s));
+            CU(cudaMemsetAsync(L->tap[t].bank_mean, 0, sizeof(float) * static_cast<size_t>(L->imgc) * L->tap[t].R * L->tap[t].R * L->tap[t].C, s));
+    CU(cudaMemsetAsync(L->m2, 0, 4 * sizeof(float), s));
     const long long npx = static_cast<long long>(L->ncrops) * L->cs * L->cs;
     for (int m0 = 0; m0 < M; m0 += L->batch) {
         const int nv = M - m0 < L->batch ? M - m0 : L->batch;
         lpips_crop_kernel<<<cdiv(npx, 256), 256, 0, s>>>(nullptr, d_crops + static_cast<long long>(m0) * L->imgc * L->cs * L->cs, nv, L->cc, L->res,
                                                         L->imgc, L->cs, L->ncrops, L->z, 0, L->x_in.hi, L->x_in.lo);
-        LCU(cudaGetLastError());
-        LLA(run_network(L, s, launches));
+        CU(cudaGetLastError());
+        LA(run_network(L, s, launches));
         for (int t = 0; t < LA_VGG_TAPS; ++t) {
             TapL& T = L->tap[t];
             if (!T.used) continue;
@@ -671,7 +575,7 @@ int lpips_set_bank(la_lpips* L, const float* d_crops, int M, cudaStream_t s, lon
             const long long pixels = static_cast<long long>(L->ncrops) * T.R * T.R;
             lpips_tap_kernel<1><<<tap_grid(pixels, L->num_sms), 256, 0, s>>>(CU32(c.x.hi), CU32(c.x.lo), L->ncrops, L->imgc, T.R * T.R, T.C, T.lin_w, T.bank_mean, L->cc,
                                                               nv * L->imgc, 1.f / M, nullptr, L->m2, 0, nullptr, nullptr, nullptr);
-            LCU(cudaGetLastError());
+            CU(cudaGetLastError());
         }
     }
     L->has_bank = 1;
@@ -682,7 +586,7 @@ int lpips_forward(la_lpips* L, const float4* img, int targets, cudaStream_t s, l
     const long long npx = static_cast<long long>(L->ncrops) * L->cs * L->cs;
     lpips_crop_kernel<<<cdiv(npx, 256), 256, 0, s>>>(img, nullptr, L->batch, L->cc, L->res, L->imgc, L->cs, L->ncrops, L->z, targets ? L->pool_f : 0,
                                                     L->x_in.hi, L->x_in.lo);
-    LCU(cudaGetLastError());
+    CU(cudaGetLastError());
     if (launches) ++*launches;
     return run_network(L, s, launches);
 }
@@ -692,9 +596,9 @@ int lpips_has_targets(const la_lpips* L) { return L->has_targets; }
 int lpips_set_targets(la_lpips* L, const float4* img, cudaStream_t s, long long* launches) {
     bool planned = false;
     for (int t = 0; t < LA_VGG_TAPS; ++t) planned = planned || L->tap[t].target;
-    if (!planned) return lfail(-2, "lpips: per-sample targets were not planned (la_vgg_desc.per_sample_targets = 0)");
-    LLA(lpips_set_call(L, 0, 0, 1.f, 1, s));
-    LLA(lpips_forward(L, img, 1, s, launches));
+    if (!planned) return fail(-2, "lpips: per-sample targets were not planned (la_vgg_desc.per_sample_targets = 0)");
+    LA(lpips_set_call(L, 0, 0, 1.f, 1, s));
+    LA(lpips_forward(L, img, 1, s, launches));
     for (int t = 0; t < LA_VGG_TAPS; ++t) {
         TapL& T = L->tap[t];
         if (!T.used) continue;
@@ -702,7 +606,7 @@ int lpips_set_targets(la_lpips* L, const float4* img, cudaStream_t s, long long*
         const long long pixels = static_cast<long long>(L->ncrops) * T.R * T.R;
         lpips_tap_kernel<1, true><<<tap_grid(pixels, L->num_sms), 256, 0, s>>>(CU32(c.x.hi), CU32(c.x.lo), L->ncrops, L->imgc, T.R * T.R, T.C, T.lin_w,
                                                                           T.target, L->cc, L->ncrops, 0.f, nullptr, nullptr, 0, nullptr, nullptr, nullptr);
-        LCU(cudaGetLastError());
+        CU(cudaGetLastError());
         if (launches) ++*launches;
     }
     L->has_targets = 1;
@@ -710,10 +614,10 @@ int lpips_set_targets(la_lpips* L, const float4* img, cudaStream_t s, long long*
 }
 
 int lpips_backward(la_lpips* L, float4* g_img, int accumulate, float* d_loss, int targets, cudaStream_t s, long long* launches) {
-    if (targets && !L->has_targets) return lfail(-2, "lpips: no per-sample targets (la_set_projection_targets)");
-    if (!targets && !L->has_bank) return lfail(-2, "lpips: no feature bank (la_set_feature_bank)");
-    LCU(cudaMemsetAsync(L->S, 0, sizeof(double) * (targets ? L->batch : 1), s));
-    if (!accumulate) LCU(cudaMemsetAsync(g_img, 0, sizeof(float4) * static_cast<size_t>(L->batch) * L->res * L->res, s));
+    if (targets && !L->has_targets) return fail(-2, "lpips: no per-sample targets (la_set_projection_targets)");
+    if (!targets && !L->has_bank) return fail(-2, "lpips: no feature bank (la_set_feature_bank)");
+    CU(cudaMemsetAsync(L->S, 0, sizeof(double) * (targets ? L->batch : 1), s));
+    if (!accumulate) CU(cudaMemsetAsync(g_img, 0, sizeof(float4) * static_cast<size_t>(L->batch) * L->res * L->res, s));
     for (int t = 0; t < LA_VGG_TAPS; ++t) {
         TapL& T = L->tap[t];
         if (!T.used) continue;
@@ -727,12 +631,12 @@ int lpips_backward(la_lpips* L, float4* g_img, int accumulate, float* d_loss, in
         else
             lpips_tap_kernel<0><<<tap_grid(pixels, L->num_sms), 256, 0, s>>>(CU32(c.x.hi), CU32(c.x.lo), L->ncrops, L->imgc, T.R * T.R, T.C, T.lin_w, T.bank_mean, L->cc,
                                                               L->ncrops, 0.f, L->S, nullptr, last ? 1 : 0, U32(out.hi), U32(out.lo), nullptr);
-        LCU(cudaGetLastError());
+        CU(cudaGetLastError());
         if (launches) ++*launches;
     }
     for (int i = L->last_conv; i >= 0; --i) {
         Conv& c = L->conv[i];
-        LLA(launch_tapgemm(c.B, L->num_sms, s));
+        LA(launch_tapgemm(c.B, L->num_sms, s));
         if (launches) ++*launches;
         if (i == 0) break;
         int pk = -1;
@@ -744,17 +648,17 @@ int lpips_backward(la_lpips* L, float4* g_img, int accumulate, float* d_loss, in
             pool_bwd_kernel<<<cdiv(total, 256), 256, 0, s>>>(CU32(L->gp.hi), CU32(L->gp.lo), CU32(pc.x.hi), CU32(pc.x.lo), T.used ? CU32(T.tg.hi) : nullptr,
                                                             T.used ? CU32(T.tg.lo) : nullptr, L->ncrops, pc.R, pc.cout, U32(L->gz[(i - 1) & 1].hi),
                                                             U32(L->gz[(i - 1) & 1].lo));
-            LCU(cudaGetLastError());
+            CU(cudaGetLastError());
             if (launches) ++*launches;
         }
     }
     const long long npx = static_cast<long long>(L->ncrops) * L->cs * L->cs;
     lpips_crop_bwd_kernel<<<cdiv(npx, 256), 256, 0, s>>>(L->g_in.hi, L->g_in.lo, L->cc, L->res, L->imgc, L->cs, L->ncrops, L->z,
                                                         targets ? L->pool_f : 0, g_img);
-    LCU(cudaGetLastError());
+    CU(cudaGetLastError());
     if (targets) lpips_target_loss_kernel<<<1, 128, 0, s>>>(L->S, L->batch, d_loss);
     else lpips_loss_kernel<<<1, 1, 0, s>>>(L->S, L->m2, L->imgc, L->batch, L->cc, d_loss);
-    LCU(cudaGetLastError());
+    CU(cudaGetLastError());
     if (launches) *launches += 2;
     return 0;
 }
@@ -772,10 +676,10 @@ int lpips_copy_tap(la_lpips* L, int k, float* d_out, size_t* count, cudaStream_t
         const long long pixels = static_cast<long long>(L->ncrops) * T.R * T.R;
         lpips_tap_kernel<2><<<tap_grid(pixels, L->num_sms), 256, 0, s>>>(CU32(c.x.hi), CU32(c.x.lo), L->ncrops, L->imgc, T.R * T.R, T.C, T.lin_w, nullptr, L->cc, 0, 0.f,
                                                           nullptr, nullptr, 0, nullptr, nullptr, d_out);
-        LCU(cudaGetLastError());
+        CU(cudaGetLastError());
         return 0;
     }
-    return lfail(-2, "lpips: tap %d does not exist", k);
+    return fail(-2, "lpips: tap %d does not exist", k);
 }
 
 }  // namespace la

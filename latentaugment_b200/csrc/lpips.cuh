@@ -15,7 +15,6 @@ int lpips_workspace_bytes(const la_vgg_desc& d, int batch, int img_channels, int
 int lpips_create(const la_vgg_desc& d, int batch, int img_channels, int img_resolution, int split, int num_sms, void* ws, size_t bytes,
                  cudaStream_t s, la_lpips** out);
 void lpips_destroy(la_lpips* L);
-const char* lpips_last_error();
 
 // Bank of real crops [M, img_channels, crop, crop] fp32 in [-1, 1] (already cropped by the caller, one random window
 // per image like util_latent_aug.py:564-579): only the bank MOMENTS of the normalised activations are kept.

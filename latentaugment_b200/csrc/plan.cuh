@@ -1,8 +1,9 @@
-// Host-side planning helpers shared by the generator engine (engine.cu) and the discriminator (disc.cu):
+// Host-side planning helpers shared by the clients of the tap-GEMM (engine, discriminator, VGG16 in lpips.cu / detector.cu):
 // tile geometry, column-block choice, TMA tensor maps and tap lists of one tap-GEMM launch.
 #pragma once
 #include <stdlib.h>
 
+#include "common.cuh"
 #include "tapgemm.cuh"
 
 namespace la {
@@ -32,6 +33,8 @@ inline int pick_bn(int n, long long m_tiles = 1 << 30) {
     if (m_tiles * (n / 128) <= 74) return 64;
     return n % 256 == 0 ? 256 : 128;
 }
+// Column block of a plain layer, whose channel count may be an odd multiple of 64
+inline int choose_bn(int n, long long m_tiles) { return n % 128 ? 64 : pick_bn(n, m_tiles); }
 
 inline int make_a_map(CUtensorMap* m, const void* base, int C, int W, int H, int N, long long sW, long long sH, long long sN, int tw, int th,
                int nb) {
@@ -39,6 +42,13 @@ inline int make_a_map(CUtensorMap* m, const void* base, int C, int W, int H, int
     uint64_t strides[3] = {static_cast<uint64_t>(sW) * 2, static_cast<uint64_t>(sH) * 2, static_cast<uint64_t>(sN) * 2};
     uint32_t box[4] = {64, static_cast<uint32_t>(tw), static_cast<uint32_t>(th), static_cast<uint32_t>(nb)};
     return encode_tmap_bf16(m, base, 4, dims, strides, box);
+}
+// A maps of a dense NHWC tensor [n, H, W, C] with box tw x th x nb: a_map[0] = hi plane, a_map[1] = lo plane (split)
+inline int dense_maps(TapGemmParams& P, const Pl& t, int n, int C, int W, int H, int tw, int th, int nb, int split) {
+    const long long sW = C, sH = static_cast<long long>(W) * C, sN = sH * H;
+    if (make_a_map(&P.a_map[0], t.hi, C, W, H, n, sW, sH, sN, tw, th, nb)) return -1;
+    if (split && make_a_map(&P.a_map[1], t.lo, C, W, H, n, sW, sH, sN, tw, th, nb)) return -1;
+    return 0;
 }
 // CTA pairs (cta_group::2, M = 256 MMAs over two SMs, each SM reading half the weight tile): measured on the C2
 // layers 8-12 % faster at BN = 256 / 64.  At BN = 128 a pair works on four M tiles (two per CTA); that wins for

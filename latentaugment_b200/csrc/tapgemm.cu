@@ -8,6 +8,7 @@
 #include <type_traits>
 
 #include "act.cuh"
+#include "common.cuh"
 #include "sm100.cuh"
 
 namespace la {
@@ -185,16 +186,9 @@ __device__ __forceinline__ void tile_range(const TapGemmParams& P, int& begin, i
     tile_range(P, begin, end, static_cast<int>(blockIdx.x), static_cast<int>(gridDim.x));
 }
 
-__device__ __forceinline__ uint32_t pack_bf16(float lo, float hi) {
-    __nv_bfloat162 v = __floats2bfloat162_rn(lo, hi);
-    return *reinterpret_cast<uint32_t*>(&v);
-}
 __device__ __forceinline__ void st_global_if(unsigned* p, unsigned v, bool ok) {
     asm volatile("{\n\t.reg .pred q;\n\tsetp.ne.b32 q, %2, 0;\n\t@q st.global.b32 [%0], %1;\n\t}" ::"l"(p), "r"(v), "r"(static_cast<int>(ok)));
 }
-__device__ __forceinline__ float bf16_round(float v) { return __bfloat162float(__float2bfloat16_rn(v)); }
-__device__ __forceinline__ float bf16lo_f(uint32_t u) { return __uint_as_float(u << 16); }
-__device__ __forceinline__ float bf16hi_f(uint32_t u) { return __uint_as_float(u & 0xffff0000u); }
 
 // store 32 consecutive values as bf16 (hi plane) and, if lo != null, the bf16 residual (lo plane)
 __device__ __forceinline__ void store_bf16x32(void* hi, void* lo, long long off, const float (&v)[32]) {
@@ -202,10 +196,10 @@ __device__ __forceinline__ void store_bf16x32(void* hi, void* lo, long long off,
 #pragma unroll
     for (int j = 0; j < 4; ++j) {
         uint4 o;
-        o.x = pack_bf16(v[8 * j + 0], v[8 * j + 1]);
-        o.y = pack_bf16(v[8 * j + 2], v[8 * j + 3]);
-        o.z = pack_bf16(v[8 * j + 4], v[8 * j + 5]);
-        o.w = pack_bf16(v[8 * j + 6], v[8 * j + 7]);
+        o.x = pack2(v[8 * j + 0], v[8 * j + 1]);
+        o.y = pack2(v[8 * j + 2], v[8 * j + 3]);
+        o.z = pack2(v[8 * j + 4], v[8 * j + 5]);
+        o.w = pack2(v[8 * j + 6], v[8 * j + 7]);
         dh[j] = o;
     }
     if (lo) {
@@ -214,12 +208,12 @@ __device__ __forceinline__ void store_bf16x32(void* hi, void* lo, long long off,
         for (int j = 0; j < 4; ++j) {
             float r[8];
 #pragma unroll
-            for (int i = 0; i < 8; ++i) r[i] = v[8 * j + i] - bf16_round(v[8 * j + i]);
+            for (int i = 0; i < 8; ++i) r[i] = v[8 * j + i] - rnd(v[8 * j + i]);
             uint4 o;
-            o.x = pack_bf16(r[0], r[1]);
-            o.y = pack_bf16(r[2], r[3]);
-            o.z = pack_bf16(r[4], r[5]);
-            o.w = pack_bf16(r[6], r[7]);
+            o.x = pack2(r[0], r[1]);
+            o.y = pack2(r[2], r[3]);
+            o.z = pack2(r[4], r[5]);
+            o.w = pack2(r[6], r[7]);
             dl[j] = o;
         }
     }
@@ -230,10 +224,10 @@ __device__ __forceinline__ void load_bf16x32(const void* p, long long off, float
 #pragma unroll
     for (int j = 0; j < 4; ++j) {
         const uint4 a = __ldg(s + j);
-        v[8 * j + 0] = bf16lo_f(a.x); v[8 * j + 1] = bf16hi_f(a.x);
-        v[8 * j + 2] = bf16lo_f(a.y); v[8 * j + 3] = bf16hi_f(a.y);
-        v[8 * j + 4] = bf16lo_f(a.z); v[8 * j + 5] = bf16hi_f(a.z);
-        v[8 * j + 6] = bf16lo_f(a.w); v[8 * j + 7] = bf16hi_f(a.w);
+        v[8 * j + 0] = lo_f(a.x); v[8 * j + 1] = hi_f(a.x);
+        v[8 * j + 2] = lo_f(a.y); v[8 * j + 3] = hi_f(a.y);
+        v[8 * j + 4] = lo_f(a.z); v[8 * j + 5] = hi_f(a.z);
+        v[8 * j + 6] = lo_f(a.w); v[8 * j + 7] = hi_f(a.w);
     }
 }
 
@@ -282,10 +276,10 @@ __device__ __forceinline__ void stage_bf16x32(uint8_t* stg, int lane, const floa
 #pragma unroll
     for (int j = 0; j < 4; ++j) {
         uint4 o;
-        o.x = pack_bf16(v[8 * j + 0], v[8 * j + 1]);
-        o.y = pack_bf16(v[8 * j + 2], v[8 * j + 3]);
-        o.z = pack_bf16(v[8 * j + 4], v[8 * j + 5]);
-        o.w = pack_bf16(v[8 * j + 6], v[8 * j + 7]);
+        o.x = pack2(v[8 * j + 0], v[8 * j + 1]);
+        o.y = pack2(v[8 * j + 2], v[8 * j + 3]);
+        o.z = pack2(v[8 * j + 4], v[8 * j + 5]);
+        o.w = pack2(v[8 * j + 6], v[8 * j + 7]);
         *reinterpret_cast<uint4*>(rowp + ((j ^ sw) << 4)) = o;
     }
 }
@@ -397,10 +391,10 @@ __device__ __forceinline__ void rowowner_warp_tile(const TapGemmParams& P, const
 #pragma unroll
                         for (int q = 0; q < 4; ++q) {
                             const uint4 a = __ldg(s + q);
-                            t[8 * q + 0] += bf16lo_f(a.x); t[8 * q + 1] += bf16hi_f(a.x);
-                            t[8 * q + 2] += bf16lo_f(a.y); t[8 * q + 3] += bf16hi_f(a.y);
-                            t[8 * q + 4] += bf16lo_f(a.z); t[8 * q + 5] += bf16hi_f(a.z);
-                            t[8 * q + 6] += bf16lo_f(a.w); t[8 * q + 7] += bf16hi_f(a.w);
+                            t[8 * q + 0] += lo_f(a.x); t[8 * q + 1] += hi_f(a.x);
+                            t[8 * q + 2] += lo_f(a.y); t[8 * q + 3] += hi_f(a.y);
+                            t[8 * q + 4] += lo_f(a.z); t[8 * q + 5] += hi_f(a.z);
+                            t[8 * q + 6] += lo_f(a.w); t[8 * q + 7] += hi_f(a.w);
                         }
                     }
 #pragma unroll
@@ -711,8 +705,8 @@ __device__ __forceinline__ void bwd_warp_tile(const TapGemmParams& P, const BwdT
         for (int i = 0; i < 16; ++i) {
             const unsigned o = soff[i];
             const float2 a = *reinterpret_cast<const float2*>(strans + i * kTransStride);
-            float x0 = bf16lo_f(xa[i]), x1 = bf16hi_f(xa[i]);
-            if (kSplit) { x0 += bf16lo_f(xl[i]); x1 += bf16hi_f(xl[i]); }
+            float x0 = lo_f(xa[i]), x1 = hi_f(xa[i]);
+            if (kSplit) { x0 += lo_f(xl[i]); x1 += hi_f(xl[i]); }
             r[0] = fmaf(a.x, x0, r[0]);
             r[1] = fmaf(a.y, x1, r[1]);
             float g0 = a.x * sc.x, g1 = a.y * sc.y;
@@ -733,8 +727,8 @@ __device__ __forceinline__ void bwd_warp_tile(const TapGemmParams& P, const BwdT
             r[3] = fmaf(gz1, z1 - (nz + bs.y), r[3]);
             const float y0 = gz0 * dm.x, y1 = gz1 * dm.y;
             const bool st_ok = o != kRowMasked && !last;
-            st_global_if(gy_step + o, pack_bf16(y0, y1), st_ok);
-            if (kSplit) st_global_if(gyl_step + o, pack_bf16(y0 - bf16_round(y0), y1 - bf16_round(y1)), st_ok);
+            st_global_if(gy_step + o, pack2(y0, y1), st_ok);
+            if (kSplit) st_global_if(gyl_step + o, pack2(y0 - rnd(y0), y1 - rnd(y1)), st_ok);
         }
     };
 
@@ -1393,7 +1387,7 @@ __global__ void __launch_bounds__(256) seed_stream_kernel(const __grid_constant_
 #pragma unroll
         for (int u = 0; u < U; ++u) {
             const int p = p0 + u * rlanes;
-            const float x0 = bf16lo_f(xu[u]) + bf16lo_f(xv[u]), x1 = bf16hi_f(xu[u]) + bf16hi_f(xv[u]);
+            const float x0 = lo_f(xu[u]) + lo_f(xv[u]), x1 = hi_f(xu[u]) + hi_f(xv[u]);
             const float g0 = fmaf(g[u].x, rw0.x, fmaf(g[u].y, rw0.y, g[u].z * rw0.z));
             const float g1 = fmaf(g[u].x, rw1.x, fmaf(g[u].y, rw1.y, g[u].z * rw1.z));
             r[2] = fmaf(x0, g[u].x, r[2]); r[3] = fmaf(x1, g[u].x, r[3]);
@@ -1407,8 +1401,8 @@ __global__ void __launch_bounds__(256) seed_stream_kernel(const __grid_constant_
             if (p < p_end) {
                 const float y0 = gz0 * dm.x, y1 = gz1 * dm.y;
                 const long long o = static_cast<long long>(p) * half_n;
-                gh[o] = pack_bf16(y0, y1);
-                if (gl) gl[o] = pack_bf16(y0 - bf16_round(y0), y1 - bf16_round(y1));
+                gh[o] = pack2(y0, y1);
+                if (gl) gl[o] = pack2(y0 - rnd(y0), y1 - rnd(y1));
             }
         }
     }
@@ -1493,7 +1487,7 @@ __global__ void __launch_bounds__(128) seed_bulk_kernel(const __grid_constant__ 
             const unsigned xu = xs[row * pairs + cp];
             const float4 g = gs[row];
             const float nz = nzp ? ns[row] * nscale : 0.f;
-            const float x0 = bf16lo_f(xu), x1 = bf16hi_f(xu);
+            const float x0 = lo_f(xu), x1 = hi_f(xu);
             const float g0 = fmaf(g.x, rw0.x, fmaf(g.y, rw0.y, g.z * rw0.z));
             const float g1 = fmaf(g.x, rw1.x, fmaf(g.y, rw1.y, g.z * rw1.z));
             r[2] = fmaf(x0, g.x, r[2]); r[3] = fmaf(x1, g.x, r[3]);
@@ -1504,7 +1498,7 @@ __global__ void __launch_bounds__(128) seed_bulk_kernel(const __grid_constant__ 
             const float z0 = x0 * (q0 ? inv_gain : inv_gain_slope), z1 = x1 * (q1 ? inv_gain : inv_gain_slope);
             r[0] = fmaf(gz0, z0 - nz - bs.x, r[0]);
             r[1] = fmaf(gz1, z1 - nz - bs.y, r[1]);
-            xs[row * pairs + cp] = pack_bf16(gz0 * dm.x, gz1 * dm.y);      // g_y in place
+            xs[row * pairs + cp] = pack2(gz0 * dm.x, gz1 * dm.y);      // g_y in place
         }
         fence_proxy_async();          // generic-proxy writes -> visible to the bulk store
         __syncthreads();

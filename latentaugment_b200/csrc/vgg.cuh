@@ -5,6 +5,7 @@
 #include <cuda_bf16.h>
 #include <cuda_runtime.h>
 
+#include "common.cuh"
 #include "tapgemm.cuh"
 
 namespace la {
@@ -15,10 +16,8 @@ constexpr int kCin[kNConv] = {3, 64, 64, 128, 128, 256, 256, 256, 512, 512, 512,
 constexpr int kShift[kNConv] = {0, 0, 1, 1, 2, 2, 2, 3, 3, 3, 4, 4, 4};       // resolution = input >> shift
 constexpr int kPoolConv[5] = {1, 3, 6, 9, 12};                                 // convs followed by a max-pool
 
-struct Pl { __nv_bfloat16* hi = nullptr; __nv_bfloat16* lo = nullptr; };
-
 // w [cout, cin, 3, 3] fp32 -> wf [9][cout][cin_pad] (forward operand) and, unless wb is null, wb [9][cin_pad][cout]
-// (data-gradient operand); zero padded, residual planes behind the main ones when split.  Errors: lpips_last_error().
+// (data-gradient operand); zero padded, residual planes behind the main ones when split.
 int vgg_prep_weights(const float* w, int cout, int cin, int cin_pad, int split, __nv_bfloat16* wf, __nv_bfloat16* wb, cudaStream_t s);
 // P <- the launch  out[n, R, R, cout] = ReLU(conv3x3(in[n, R, R, cin_pad], wf) + bias)  (ones: >= n * cout 1.0f).
 int vgg_conv_fwd_plan(TapGemmParams& P, int R, int n, int cin_pad, int cout, const Pl& in, const __nv_bfloat16* wf, int split,
