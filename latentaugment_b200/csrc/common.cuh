@@ -30,6 +30,11 @@ int fail(int code, const char* fmt, ...) __attribute__((format(printf, 2, 3)));
     } while (0)
 
 // ------------------------------------------------------------------------- workspace
+struct Pl {                 // a bf16 tensor as (hi [, lo]) planes; lo only in split (fp32_parity) precision
+    __nv_bfloat16* hi = nullptr;
+    __nv_bfloat16* lo = nullptr;
+};
+
 // Places buffers in a caller-owned workspace, each 1024-byte aligned.  With a null base it only counts: `off` is then the
 // size the same plan needs.
 struct Bump {
@@ -42,6 +47,12 @@ struct Bump {
         off += count * sizeof(T);
         return p;
     }
+    Pl take_pl(size_t count, int split) {          // count elements as (hi [, lo]) planes
+        Pl t;
+        t.hi = take<__nv_bfloat16>(count);
+        t.lo = split ? take<__nv_bfloat16>(count) : nullptr;
+        return t;
+    }
 };
 
 // A plan that needs `need` bytes, placed in the caller's workspace ws of `bytes` bytes: reject a short or misaligned one.
@@ -52,13 +63,11 @@ inline int check_workspace(const char* owner, size_t need, size_t bytes, const v
 }
 
 inline int cdiv(long long a, long long b) { return static_cast<int>((a + b - 1) / b); }
+// a bf16 plane as bf16x2 pairs
+inline unsigned* U32(__nv_bfloat16* p) { return reinterpret_cast<unsigned*>(p); }
+inline const unsigned* CU32(const __nv_bfloat16* p) { return reinterpret_cast<const unsigned*>(p); }
 
 // ------------------------------------------------------------------------- split-bf16 planes
-struct Pl {                 // a bf16 tensor as (hi [, lo]) planes; lo only in split (fp32_parity) precision
-    __nv_bfloat16* hi = nullptr;
-    __nv_bfloat16* lo = nullptr;
-};
-
 __device__ __forceinline__ unsigned pack2(float a, float b) {      // a in the low half, b in the high half
     __nv_bfloat162 v = __floats2bfloat162_rn(a, b);
     return *reinterpret_cast<unsigned*>(&v);

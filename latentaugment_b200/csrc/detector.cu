@@ -5,12 +5,11 @@
 //   the perceptual term) -> NCHW flatten -> fc6 + ReLU -> fc7 + ReLU -> [n, 4096] fp32.
 //
 // The convolutions ping-pong between two NHWC activation buffers (the largest, 224^2 x 64, sets their size).  fc6 and fc7
-// are one-tap GEMMs whose M rows are images (a [64, 1, 1, 128 images] box, as the discriminator's dense layers): fc6
+// are one-tap dense layers whose M rows are images (plan.cuh LayerTaps::kDense, as the discriminator's dense layers): fc6
 // contracts K = 25088 over the NHWC view [n, 1, 1, 7 * 7 * 512] of the pool5 output, with its weights permuted from
 // torchvision's NCHW flatten order at preparation time.  fc7 stores raw fp32 accumulators and a small kernel adds the bias
 // and applies the ReLU, so the embedding is never rounded to bf16.
 #include <cuda_bf16.h>
-#include <string.h>
 
 #include "../../include/latentaugment_b200.h"
 #include "common.cuh"
@@ -122,9 +121,8 @@ size_t plan_detector(la_detector* D, char* ws) {
     Bump bp;
     bp.base = ws;
     const size_t B = D->batch, wm = D->split ? 2 : 1;
-    auto take_pl = [&](size_t cnt) { Pl t; t.hi = bp.take<bf16>(cnt); t.lo = D->split ? bp.take<bf16>(cnt) : nullptr; return t; };
-    for (int k = 0; k < 2; ++k) D->buf[k] = take_pl(B * kIn * kIn * 64);
-    D->h6 = take_pl(B * kFc);
+    for (int k = 0; k < 2; ++k) D->buf[k] = bp.take_pl(B * kIn * kIn * 64, D->split);
+    D->h6 = bp.take_pl(B * kFc, D->split);
     for (int i = 0; i < kNConv; ++i) D->wconv[i] = bp.take<bf16>(wm * 9 * kCout[i] * ((kCin[i] + 63) / 64 * 64));
     D->w6 = bp.take<bf16>(wm * kFc * kPool5);
     D->w7 = bp.take<bf16>(wm * kFc * kFc);
@@ -135,52 +133,25 @@ size_t plan_detector(la_detector* D, char* ws) {
     return bp.off;
 }
 
-// M rows = images: 128 images x one pixel per tile, one tap of K = k_total over the [batch, 1, 1, k_total] view of `in`
-int dense_layer(la_detector* D, TapGemmParams& P, const Pl& in, int k_total, const bf16* w) {
-    const int B = D->batch, split = D->split;
-    memset(&P, 0, sizeof P);
-    P.th = 1; P.tw = 1; P.nb = 128; P.halo = 0;
-    P.tiles_n = (B + 127) / 128; P.batch = B; P.nprob = 1;
-    P.prob[0].vh = P.prob[0].vw = 1; P.prob[0].tiles_h = P.prob[0].tiles_w = 1; P.prob[0].tile_begin = 0;
-    P.m_tiles = P.tiles_n;
-    if (make_a_map(&P.a_map[0], in.hi, k_total, 1, 1, B, k_total, k_total, k_total, 1, 1, 128)) return -1;
-    if (split && make_a_map(&P.a_map[1], in.lo, k_total, 1, 1, B, k_total, k_total, k_total, 1, 1, 128)) return -1;
-    const int bn = pick_bn(kFc, P.m_tiles);
-    if (make_b_map(P, w, k_total, kFc, split ? 2 : 1, bn)) return -1;
-    P.kchunks = k_total / 64;
-    P.n_total = kFc; P.n_blocks = kFc / bn;
-    P.OH = P.OW = 1; P.osy = P.osx = 1; P.split = split;
-    P.act_gain = 1.f; P.act_clamp = -1.f; P.act_slope = 0.f;
-    P.err_flag = D->err_flag;
-    int nt = 0;
-    add_tap(P, nt, 0, 0, 0, 0, 1, 1, split);
-    P.prob[0].tap_begin = 0; P.prob[0].ntaps = nt;
-    return tapgemm_finalize(P);
-}
-
 int build_detector(la_detector* D) {
+    const int B = D->batch, split = D->split;
     int cur = 1;
     for (int i = 0; i < kNConv; ++i) {
         const int R = kIn >> kShift[i];
-        LA(vgg_conv_fwd_plan(D->conv[i], R, D->batch, (kCin[i] + 63) / 64 * 64, kCout[i], D->buf[cur], D->wconv[i], D->split, D->d.d_conv_bias[i],
-                               D->ones, D->buf[cur ^ 1], D->err_flag));
+        LA(plan_layer(D->conv[i], LayerTaps::k3x3, D->buf[cur], B, R, (kCin[i] + 63) / 64 * 64, kCout[i], D->wconv[i], split, D->err_flag));
+        fwd_epilogue(D->conv[i], D->ones, D->d.d_conv_bias[i], 1.f, -1.f, 0.f, D->buf[cur ^ 1]);          // ReLU
         cur ^= 1;
         for (int k = 0; k < 5; ++k) if (kPoolConv[k] == i) cur ^= 1;
     }
     D->pool5 = cur;
-    {   // fc6 + ReLU -> h6 (bf16, the A operand of fc7)
-        TapGemmParams& P = D->fc6;
-        LA(dense_layer(D, P, D->buf[cur], kPool5, D->w6));
-        P.epilogue = kEpiFwd;
-        P.demod = D->ones; P.bias = D->d.d_fc6_bias;
-        P.x_hi = D->h6.hi; P.x_lo = D->h6.lo;
-    }
-    {   // fc7 -> raw fp32 accumulators (bias + ReLU follow)
-        TapGemmParams& P = D->fc7;
-        LA(dense_layer(D, P, D->h6, kFc, D->w7));
-        P.epilogue = kEpiRawF32;
-        P.raw_out = D->raw7;
-    }
+    // fc6 + ReLU -> h6 (bf16, the A operand of fc7)
+    LA(plan_layer(D->fc6, LayerTaps::kDense, D->buf[cur], B, 1, kPool5, kFc, D->w6, split, D->err_flag));
+    fwd_epilogue(D->fc6, D->ones, D->d.d_fc6_bias, 1.f, -1.f, 0.f, D->h6);
+    // fc7 -> raw fp32 accumulators (bias + ReLU follow); the activation constants are a linear layer's
+    LA(plan_layer(D->fc7, LayerTaps::kDense, D->h6, B, 1, kFc, kFc, D->w7, split, D->err_flag));
+    linear_epilogue(D->fc7, 0.f);
+    D->fc7.epilogue = kEpiRawF32;
+    D->fc7.raw_out = D->raw7;
     return 0;
 }
 

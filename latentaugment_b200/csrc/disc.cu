@@ -302,22 +302,6 @@ struct la_disc {
 
 namespace {
 
-void fwd_epi(TapGemmParams& P, const la_disc* D, const float* bias, const Pl& out, float gain, float clamp, int n_total, int bn, int res) {
-    P.epilogue = kEpiFwd;
-    P.n_total = n_total; P.n_blocks = n_total / bn;
-    P.OH = P.OW = res; P.osy = P.osx = 1; P.split = D->split;
-    P.act_gain = gain; P.act_clamp = clamp; P.act_slope = 0.2f;
-    P.demod = D->ones; P.bias = bias; P.noise = nullptr; P.s_next = nullptr; P.rgbw = nullptr;
-    P.x_hi = out.hi; P.x_lo = out.lo;
-    P.staged = P.nb == 1 && !D->split && !getenv("LA_NO_STAGED");
-}
-void lin_epi(TapGemmParams& P, const la_disc* D, int n_total, int bn, int oh, int ow) {
-    P.epilogue = kEpiLinear;
-    P.n_total = n_total; P.n_blocks = n_total / bn;
-    P.OH = oh; P.OW = ow; P.osy = P.osx = 1; P.split = D->split;
-    P.act_gain = 1.f; P.act_clamp = -1.f; P.act_slope = 0.2f;
-}
-
 int plan_disc(la_disc* D, char* ws, size_t* bytes_out) {
     const la_disc_desc& d = D->d;
     const int B = D->batch, split = D->split;
@@ -329,7 +313,6 @@ int plan_disc(la_disc* D, char* ws, size_t* bytes_out) {
         if (d.channels[b] % 64 || d.channels[b] < 64 || d.channels[b] > 1024) return fail(-2, "discriminator: channels[%d]=%d unsupported", b, d.channels[b]);
     Bump bp;
     bp.base = ws;
-    auto take_pl = [&](size_t n) { Pl t; t.hi = bp.take<bf16>(n); t.lo = split ? bp.take<bf16>(n) : nullptr; return t; };
     const size_t wm = split ? 2 : 1;            // weight stacks carry the residual planes behind the main ones
     D->blk.assign(d.num_blocks, Block{});
     size_t max_full = 0, max_half = 0, max_t = 0;
@@ -342,12 +325,12 @@ int plan_disc(la_disc* D, char* ws, size_t* bytes_out) {
         k.w1f = bp.take<bf16>(wm * 9 * Cn * C); k.w1b = bp.take<bf16>(wm * 9 * Cn * C);
         k.wsf = bp.take<bf16>(wm * Cn * C); k.wsb = bp.take<bf16>(wm * Cn * C);
         const size_t full = B * R * R * C, half = B * (R / 2) * (R / 2) * Cn;
-        k.x_in = b == 0 ? take_pl(full) : D->blk[b - 1].y;
-        k.x0 = take_pl(full);
-        k.y1 = take_pl(half);
-        k.y = take_pl(half);
-        k.g_y = take_pl(half);
-        k.g_z1 = take_pl(half);
+        k.x_in = b == 0 ? bp.take_pl(full, split) : D->blk[b - 1].y;
+        k.x0 = bp.take_pl(full, split);
+        k.y1 = bp.take_pl(half, split);
+        k.y = bp.take_pl(half, split);
+        k.g_y = bp.take_pl(half, split);
+        k.g_z1 = bp.take_pl(half, split);
         max_full = full > max_full ? full : max_full;
         const size_t hs = B * (R / 2) * (R / 2) * C;
         max_half = hs > max_half ? hs : max_half;
@@ -356,17 +339,17 @@ int plan_disc(la_disc* D, char* ws, size_t* bytes_out) {
         cmax = k.C > cmax ? k.C : cmax;
         cmax = k.Cn > cmax ? k.Cn : cmax;
     }
-    D->yb = take_pl(max_t); D->g_yb = take_pl(max_t);
-    D->ys = take_pl(max_half); D->g_ys = take_pl(max_half);
-    D->g_z0 = take_pl(max_full);
+    D->yb = bp.take_pl(max_t, split); D->g_yb = bp.take_pl(max_t, split);
+    D->ys = bp.take_pl(max_half, split); D->g_ys = bp.take_pl(max_half, split);
+    D->g_z0 = bp.take_pl(max_full, split);
     const int C4 = d.channels[d.num_blocks], Cp = C4 + 64;
     D->C4 = C4; D->Cp = Cp;
     cmax = 16 * C4 > cmax ? 16 * C4 : cmax;
     D->ones = bp.take<float>(static_cast<size_t>(B) * cmax);
     D->rgb_w4 = bp.take<float>(4 * static_cast<size_t>(d.channels[0]));
-    D->x4p = take_pl(static_cast<size_t>(B) * 16 * Cp); D->gx4p = take_pl(static_cast<size_t>(B) * 16 * Cp);
-    D->x5 = take_pl(static_cast<size_t>(B) * 16 * C4); D->gz5 = take_pl(static_cast<size_t>(B) * 16 * C4);
-    D->x6 = take_pl(static_cast<size_t>(B) * C4); D->gz6 = take_pl(static_cast<size_t>(B) * C4);
+    D->x4p = bp.take_pl(static_cast<size_t>(B) * 16 * Cp, split); D->gx4p = bp.take_pl(static_cast<size_t>(B) * 16 * Cp, split);
+    D->x5 = bp.take_pl(static_cast<size_t>(B) * 16 * C4, split); D->gz5 = bp.take_pl(static_cast<size_t>(B) * 16 * C4, split);
+    D->x6 = bp.take_pl(static_cast<size_t>(B) * C4, split); D->gz6 = bp.take_pl(static_cast<size_t>(B) * C4, split);
     D->wef = bp.take<bf16>(wm * 9 * C4 * Cp); D->web = bp.take<bf16>(wm * 9 * C4 * Cp);
     D->wff = bp.take<bf16>(wm * 16 * C4 * C4); D->wfb = bp.take<bf16>(wm * 16 * C4 * C4);
     D->feat = bp.take<float>(B); D->gfeat = bp.take<float>(B); D->logits = bp.take<float>(B); D->gl = bp.take<float>(B);
@@ -376,169 +359,60 @@ int plan_disc(la_disc* D, char* ws, size_t* bytes_out) {
     return 0;
 }
 
-// 3x3 taps over map 0 (lo map 1)
-int conv_taps(const la_disc* D, TapGemmParams& P, bool flipped) {
-    int nt = 0;
-    P.prob[0].tap_begin = 0;
-    for (int t = 0; t < 9; ++t) {
-        const int dy = t / 3 - 1, dx = t % 3 - 1;
-        add_tap(P, nt, flipped ? -dy : dy, flipped ? -dx : dx, t, 0, 1, 9, D->split);
-    }
-    P.prob[0].ntaps = nt;
-    return tapgemm_finalize(P);
-}
-int one_tap(const la_disc* D, TapGemmParams& P) {
-    int nt = 0;
-    add_tap(P, nt, 0, 0, 0, 0, 1, 1, D->split);
-    P.prob[0].tap_begin = 0; P.prob[0].ntaps = nt;
-    return tapgemm_finalize(P);
-}
-
 int build_disc(la_disc* D) {
     const la_disc_desc& d = D->d;
     const int B = D->batch, split = D->split;
-    const int wm = split ? 2 : 1;
     const float clamp = d.conv_clamp;
     for (int b = 0; b < d.num_blocks; ++b) {
         Block& k = D->blk[b];
-        const int R = k.R, C = k.C, Cn = k.Cn, Ro = R / 2, TH = R + 1, TWp = R + 2;
+        const int R = k.R, C = k.C, Cn = k.Cn, Ro = R / 2;
         // ---- conv0 forward: x_in -> x0
-        {
-            TapGemmParams& P = k.F0;
-            memset(&P, 0, sizeof P);
-            set_grid(P, R, B, 1);
-            LA(dense_maps(P, k.x_in, D->batch, C, R, R, P.tw, P.th + P.halo, P.nb, D->split));
-            const int bn = choose_bn(C, P.m_tiles);
-            LA(make_b_map(P, k.w0f, C, C, 9 * wm, bn));
-            P.kchunks = C / 64;
-            fwd_epi(P, D, k.p.d_conv0_bias, k.x0, kSqrt2, clamp, C, bn, R);
-            P.err_flag = D->err_flag;
-            LA(conv_taps(D, P, false));
-        }
+        LA(plan_layer(k.F0, LayerTaps::k3x3, k.x_in, B, R, C, C, k.w0f, split, D->err_flag));
+        fwd_epilogue(k.F0, D->ones, k.p.d_conv0_bias, kSqrt2, clamp, 0.2f, k.x0);
         // ---- blur (pad 2): x0 -> yb, and its adjoint fused with conv0's activation gradient: g_yb -> g_z0
         {
             UpFirParams& U = k.blur;
             memset(&U, 0, sizeof U);
-            U.B = B; U.OH = U.OW = R; U.C = C; U.TH = TH; U.TWp = TWp; U.split = split;
+            U.B = B; U.OH = U.OW = R; U.C = C; U.TH = R + 1; U.TWp = R + 2; U.split = split;
             // kernel forms: forward out[o] = sum_j fk[j] in[o + j - 1], backward out[u] = sum_j fk[j] in[u - j + 1]; the blur
             // yb[u] = sum_j c[j] x0[u + j - 2] (c = flipped filter) and its adjoint both need fk = the unflipped filter
             for (int i = 0; i < 16; ++i) U.fk[i] = D->fir[15 - i];
-            {
-                int bi = 0;
-                for (int i = 1; i < 16; ++i) if (fabsf(U.fk[i]) > fabsf(U.fk[bi])) bi = i;
-                const int by = bi / 4, bx = bi % 4;
-                U.separable = U.fk[bi] != 0.f;
-                for (int i = 0; i < 4 && U.separable; ++i) { U.fy[i] = U.fk[i * 4 + bx] / U.fk[bi]; U.fx[i] = U.fk[by * 4 + i]; }
-                for (int i = 0; i < 16 && U.separable; ++i)
-                    if (fabsf(U.fy[i / 4] * U.fx[i % 4] - U.fk[i]) > 1e-6f * fabsf(U.fk[bi])) U.separable = 0;
-            }
             U.gy_hi = k.x0.hi; U.gy_lo = k.x0.lo; U.gt_hi = D->yb.hi; U.gt_lo = D->yb.lo;      // "backward" FIR direction = the blur
             U.t_hi = D->g_yb.hi; U.t_lo = D->g_yb.lo; U.x_hi = D->g_z0.hi; U.x_lo = D->g_z0.lo; U.act_saved = k.x0.hi; U.act_saved_lo = k.x0.lo;
             U.act_gain = kSqrt2; U.act_clamp = clamp; U.act_slope = 0.2f;
-            if (!split && U.separable && R >= 32 && !getenv("LA_NO_FIR_TMA")) {
-                const uint64_t Cc = C, Rr = R;
-                const uint64_t tdims[4] = {Cc, Rr + 1, Rr + 1, static_cast<uint64_t>(B)};
-                const uint64_t tstr[3] = {Cc * 2, static_cast<uint64_t>(TWp) * Cc * 2, static_cast<uint64_t>(TH) * TWp * Cc * 2};
-                const uint64_t ydims[4] = {Cc, Rr, Rr, static_cast<uint64_t>(B)};
-                const uint64_t ystr[3] = {Cc * 2, Rr * Cc * 2, Rr * Rr * Cc * 2};
-                const uint32_t lbox[4] = {64, 35, 1, 1}, sbox[4] = {64, 8, 1, 1};
-                int r = encode_tmap_bf16(&U.fwd_in, D->g_yb.hi, 4, tdims, tstr, lbox, 0);
-                r |= encode_tmap_bf16(&U.fwd_out_x, D->g_z0.hi, 4, ydims, ystr, sbox, 0);
-                r |= encode_tmap_bf16(&U.bwd_in, k.x0.hi, 4, ydims, ystr, lbox, 0);
-                r |= encode_tmap_bf16(&U.bwd_out, D->yb.hi, 4, tdims, tstr, sbox, 0);
-                if (r) return fail(-5, "tensor map encoding failed (discriminator blur)");
-                U.use_tma = 1;
-            }
+            if (upfir_plan(U)) return fail(-5, "tensor map encoding failed (discriminator blur)");
         }
         // ---- conv1 forward: 3x3 stride 2 over the four phase views of yb -> y1
         {
             TapGemmParams& P = k.F1;
             memset(&P, 0, sizeof P);
             set_grid(P, Ro, B, 1);
-            const long long gW = 2LL * C, gH = 2LL * TWp * C, gN = static_cast<long long>(TH) * TWp * C;
-            for (int ph = 0; ph < 4; ++ph) {
-                const int py = ph / 2, px = ph % 2;
-                const int ph_h = Ro + (py == 0), ph_w = Ro + (px == 0);
-                const long long off = (static_cast<long long>(py) * TWp + px) * C;
-                LA(make_a_map(&P.a_map[ph], D->yb.hi + off, C, ph_w, ph_h, B, gW, gH, gN, P.tw, P.th + P.halo, P.nb));
-                if (split) LA(make_a_map(&P.a_map[4 + ph], D->yb.lo + off, C, ph_w, ph_h, B, gW, gH, gN, P.tw, P.th + P.halo, P.nb));
-            }
             int nt = 0;
-            for (int a = 0; a < 3; ++a)
-                for (int bb = 0; bb < 3; ++bb) {
-                    const int ph = (a & 1) * 2 + (bb & 1);
-                    add_tap(P, nt, a >> 1, bb >> 1, a * 3 + bb, ph, 4 + ph, 9, split);
-                }
-            P.prob[0].tap_begin = 0; P.prob[0].ntaps = nt;
-            const int bn = choose_bn(Cn, P.m_tiles);
-            LA(make_b_map(P, k.w1f, C, Cn, 9 * wm, bn));
-            P.kchunks = C / 64;
-            fwd_epi(P, D, k.p.d_conv1_bias, k.y1, kSqrt2 * kSqrtHalf, clamp >= 0.f ? clamp * kSqrtHalf : clamp, Cn, bn, Ro);
+            LA(phase_view_taps(P, nt, D->yb, B, R, C, split));
+            P.prob[0].ntaps = nt;
+            LA(plan_columns(P, k.w1f, C, Cn, 9, split));
+            P.OH = P.OW = Ro; P.osy = P.osx = 1;
+            fwd_epilogue(P, D->ones, k.p.d_conv1_bias, kSqrt2 * kSqrtHalf, clamp >= 0.f ? clamp * kSqrtHalf : clamp, 0.2f, k.y1);
             P.err_flag = D->err_flag;
             LA(tapgemm_finalize(P));
         }
         // ---- skip forward: 1x1 on the decimated blur, + y1 -> y
-        {
-            TapGemmParams& P = k.FS;
-            memset(&P, 0, sizeof P);
-            set_grid(P, Ro, B, 1);
-            LA(dense_maps(P, D->ys, D->batch, C, Ro, Ro, P.tw, P.th + P.halo, P.nb, D->split));
-            const int bn = choose_bn(Cn, P.m_tiles);
-            LA(make_b_map(P, k.wsf, C, Cn, wm, bn));
-            P.kchunks = C / 64;
-            lin_epi(P, D, Cn, bn, Ro, Ro);
-            P.lin_add = k.y1.hi; P.lin_add_lo = k.y1.lo; P.lin_out = k.y.hi; P.lin_out_lo = k.y.lo;
-            P.err_flag = D->err_flag;
-            LA(one_tap(D, P));
-        }
+        LA(plan_layer(k.FS, LayerTaps::k1x1, D->ys, B, Ro, C, Cn, k.wsf, split, D->err_flag));
+        linear_epilogue(k.FS, 0.2f);
+        k.FS.lin_add = k.y1.hi; k.FS.lin_add_lo = k.y1.lo; k.FS.lin_out = k.y.hi; k.FS.lin_out_lo = k.y.lo;
         // ---- skip backward: g_ys = Ws^T g_y
-        {
-            TapGemmParams& P = k.BS;
-            memset(&P, 0, sizeof P);
-            set_grid(P, Ro, B, 1);
-            LA(dense_maps(P, k.g_y, D->batch, Cn, Ro, Ro, P.tw, P.th + P.halo, P.nb, D->split));
-            const int bn = choose_bn(C, P.m_tiles);
-            LA(make_b_map(P, k.wsb, Cn, C, wm, bn));
-            P.kchunks = Cn / 64;
-            lin_epi(P, D, C, bn, Ro, Ro);
-            P.lin_out = D->g_ys.hi; P.lin_out_lo = D->g_ys.lo;
-            P.err_flag = D->err_flag;
-            LA(one_tap(D, P));
-        }
+        LA(plan_layer(k.BS, LayerTaps::k1x1, k.g_y, B, Ro, Cn, C, k.wsb, split, D->err_flag));
+        linear_epilogue(k.BS, 0.2f);
+        k.BS.lin_out = D->g_ys.hi; k.BS.lin_out_lo = D->g_ys.lo;
         // ---- conv1 backward: transposed stride-2 convolution, g_z1 -> g_yb (four output phases)
-        {
-            TapGemmParams& P = k.B1;
-            memset(&P, 0, sizeof P);
-            const int gh[4] = {Ro + 1, Ro + 1, Ro, Ro}, gw[4] = {Ro + 1, Ro, Ro + 1, Ro};
-            set_grid(P, Ro, B, 4, gh, gw);
-            LA(dense_maps(P, k.g_z1, D->batch, Cn, Ro, Ro, P.tw, P.th + P.halo, P.nb, D->split));
-            int nt = 0;
-            for (int ph = 0; ph < 4; ++ph) {
-                P.prob[ph].tap_begin = nt;
-                for (int ay = ph / 2; ay < 3; ay += 2)
-                    for (int ax = ph % 2; ax < 3; ax += 2) add_tap(P, nt, -(ay >> 1), -(ax >> 1), ay * 3 + ax, 0, 1, 9, split);
-                P.prob[ph].ntaps = nt - P.prob[ph].tap_begin;
-                P.prob[ph].oy0 = ph / 2; P.prob[ph].ox0 = ph % 2;
-            }
-            const int bn = choose_bn(C, P.m_tiles);
-            LA(make_b_map(P, k.w1b, Cn, C, 9 * wm, bn));
-            P.kchunks = Cn / 64; P.n_total = C; P.n_blocks = C / bn;
-            P.epilogue = kEpiStoreBf16; P.OH = TH; P.OW = TWp; P.osy = P.osx = 2; P.split = split;
-            P.x_hi = D->g_yb.hi; P.x_lo = D->g_yb.lo;
-            P.staged = P.nb == 1 && !split && !getenv("LA_NO_STAGED");
-            P.err_flag = D->err_flag;
-            LA(tapgemm_finalize(P));
-        }
+        memset(&k.B1, 0, sizeof k.B1);
+        k.B1.err_flag = D->err_flag;
+        LA(plan_upconv(k.B1, k.g_z1, B, Ro, Cn, C, k.w1b, split, D->g_yb));
         // ---- conv0 backward: g_z0 -> (+ skip-branch gradient) -> gradient wrt the block input, raw and through the producer's activation
         {
             TapGemmParams& P = k.B0;
-            memset(&P, 0, sizeof P);
-            set_grid(P, R, B, 1);
-            LA(dense_maps(P, D->g_z0, D->batch, C, R, R, P.tw, P.th + P.halo, P.nb, D->split));
-            const int bn = choose_bn(C, P.m_tiles);
-            LA(make_b_map(P, k.w0b, C, C, 9 * wm, bn));
-            P.kchunks = C / 64;
-            lin_epi(P, D, C, bn, R, R);
+            LA(plan_layer(P, LayerTaps::k3x3Flipped, D->g_z0, B, R, C, C, k.w0b, split, D->err_flag));
+            linear_epilogue(P, 0.2f);
             P.lin_add_down = D->g_ys.hi; P.lin_add_down_lo = D->g_ys.lo;      // FIRdown^T(g_ys) is evaluated inside the epilogue
             for (int i = 0; i < 16; ++i) P.lin_fir[i] = D->fir[i];
             if (b == 0) {                     // the producer is fromrgb (lrelu*sqrt2, clamp): its backward is fused (atomics into g_img)
@@ -549,73 +423,25 @@ int build_disc(la_disc* D) {
                 P.lin_out = up.g_y.hi; P.lin_out_lo = up.g_y.lo; P.lin_saved = up.y1.hi; P.lin_saved_lo = up.y1.lo; P.lin_gz = up.g_z1.hi; P.lin_gz_lo = up.g_z1.lo;
                 P.act_gain = kSqrt2 * kSqrtHalf; P.act_clamp = clamp >= 0.f ? clamp * kSqrtHalf : clamp;
             }
-            P.err_flag = D->err_flag;
-            LA(conv_taps(D, P, true));
         }
     }
     // ------------------------------------------------------------------ 4x4 epilogue
     const int C4 = D->C4, Cp = D->Cp;
-    {   // 3x3 conv on [x | stddev] : x4p -> x5
-        TapGemmParams& P = D->FE;
-        memset(&P, 0, sizeof P);
-        set_grid(P, 4, B, 1);
-        LA(dense_maps(P, D->x4p, D->batch, Cp, 4, 4, P.tw, P.th + P.halo, P.nb, D->split));
-        const int bn = choose_bn(C4, P.m_tiles);
-        LA(make_b_map(P, D->wef, Cp, C4, 9 * wm, bn));
-        P.kchunks = Cp / 64;
-        fwd_epi(P, D, d.d_b4_conv_bias, D->x5, kSqrt2, d.conv_clamp, C4, bn, 4);
-        P.err_flag = D->err_flag;
-        LA(conv_taps(D, P, false));
-    }
-    auto sample_rows = [&](TapGemmParams& P) {        // M rows = samples: 128 samples x one pixel per tile
-        P.th = 1; P.tw = 1; P.nb = 128; P.halo = 0;
-        P.tiles_n = (B + 127) / 128; P.batch = B; P.nprob = 1;
-        P.prob[0].vh = P.prob[0].vw = 1; P.prob[0].tiles_h = P.prob[0].tiles_w = 1; P.prob[0].tile_begin = 0;
-        P.m_tiles = P.tiles_n;
-    };
-    {   // dense 16*C4 -> C4 as 16 taps over the 4x4 positions of x5
-        TapGemmParams& P = D->FF;
-        memset(&P, 0, sizeof P);
-        sample_rows(P);
-        LA(dense_maps(P, D->x5, D->batch, C4, 4, 4, 1, 1, 128, D->split));
-        int nt = 0;
-        for (int hw = 0; hw < 16; ++hw) add_tap(P, nt, hw / 4, hw % 4, hw, 0, 1, 16, split);
-        P.prob[0].tap_begin = 0; P.prob[0].ntaps = nt;
-        const int bn = 64;
-        LA(make_b_map(P, D->wff, C4, C4, 16 * wm, bn));
-        P.kchunks = C4 / 64;
-        fwd_epi(P, D, d.d_b4_fc_bias, D->x6, kSqrt2, -1.f, C4, bn, 1);
-        P.staged = 0;
-        P.err_flag = D->err_flag;
-        LA(tapgemm_finalize(P));
-    }
-    {   // dense backward: gz6 [B, C4] -> gradient wrt x5 (all 16 positions as columns), through conv's activation -> gz5
-        TapGemmParams& P = D->BF;
-        memset(&P, 0, sizeof P);
-        sample_rows(P);
-        LA(dense_maps(P, D->gz6, D->batch, C4, 1, 1, 1, 1, 128, D->split));
-        const int bn = 64;
-        LA(make_b_map(P, D->wfb, C4, 16 * C4, wm, bn));
-        P.kchunks = C4 / 64;
-        lin_epi(P, D, 16 * C4, bn, 1, 1);
-        P.lin_saved = D->x5.hi; P.lin_saved_lo = D->x5.lo; P.lin_gz = D->gz5.hi; P.lin_gz_lo = D->gz5.lo;
-        P.act_gain = kSqrt2; P.act_clamp = d.conv_clamp;
-        P.err_flag = D->err_flag;
-        LA(one_tap(D, P));
-    }
-    {   // 3x3 conv backward: gz5 -> gradient wrt [x | stddev]
-        TapGemmParams& P = D->BE;
-        memset(&P, 0, sizeof P);
-        set_grid(P, 4, B, 1);
-        LA(dense_maps(P, D->gz5, D->batch, C4, 4, 4, P.tw, P.th + P.halo, P.nb, D->split));
-        const int bn = 64;
-        LA(make_b_map(P, D->web, C4, Cp, 9 * wm, bn));
-        P.kchunks = C4 / 64;
-        lin_epi(P, D, Cp, bn, 4, 4);
-        P.lin_out = D->gx4p.hi; P.lin_out_lo = D->gx4p.lo;
-        P.err_flag = D->err_flag;
-        LA(conv_taps(D, P, true));
-    }
+    // 3x3 conv on [x | stddev] : x4p -> x5
+    LA(plan_layer(D->FE, LayerTaps::k3x3, D->x4p, B, 4, Cp, C4, D->wef, split, D->err_flag));
+    fwd_epilogue(D->FE, D->ones, d.d_b4_conv_bias, kSqrt2, clamp, 0.2f, D->x5);
+    // dense 16*C4 -> C4 as 16 taps over the 4x4 positions of x5
+    LA(plan_layer(D->FF, LayerTaps::kDense, D->x5, B, 4, C4, C4, D->wff, split, D->err_flag, 64));
+    fwd_epilogue(D->FF, D->ones, d.d_b4_fc_bias, kSqrt2, -1.f, 0.2f, D->x6);
+    // dense backward: gz6 [B, C4] -> gradient wrt x5 (all 16 positions as columns), through conv's activation -> gz5
+    LA(plan_layer(D->BF, LayerTaps::kDense, D->gz6, B, 1, C4, 16 * C4, D->wfb, split, D->err_flag, 64));
+    linear_epilogue(D->BF, 0.2f);
+    D->BF.lin_saved = D->x5.hi; D->BF.lin_saved_lo = D->x5.lo; D->BF.lin_gz = D->gz5.hi; D->BF.lin_gz_lo = D->gz5.lo;
+    D->BF.act_gain = kSqrt2; D->BF.act_clamp = clamp;
+    // 3x3 conv backward: gz5 -> gradient wrt [x | stddev]
+    LA(plan_layer(D->BE, LayerTaps::k3x3Flipped, D->gz5, B, 4, C4, Cp, D->web, split, D->err_flag, 64));
+    linear_epilogue(D->BE, 0.2f);
+    D->BE.lin_out = D->gx4p.hi; D->BE.lin_out_lo = D->gx4p.lo;
     return 0;
 }
 
@@ -652,8 +478,6 @@ int gemm(la_disc* D, const TapGemmParams& P, cudaStream_t s, long long* launches
     if (launches) ++*launches;
     return launch_tapgemm(P, D->num_sms, s);
 }
-inline unsigned* U32(bf16* p) { return reinterpret_cast<unsigned*>(p); }
-inline const unsigned* CU32(const bf16* p) { return reinterpret_cast<const unsigned*>(p); }
 
 }  // namespace
 

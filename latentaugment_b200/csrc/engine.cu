@@ -236,99 +236,61 @@ int build_params(la_engine* e) {
         // ---------------------------------------------------------------- forward
         TapGemmParams& F = c.fwd;
         memset(&F, 0, sizeof F);
-        if (c.split_up) {       // T[2m+py, 2n+px]: even phases have one more row / column (T is (2H+1) x (2W+1))
-            const int gh[4] = {c.res_in + 1, c.res_in + 1, c.res_in, c.res_in};
-            const int gw[4] = {c.res_in + 1, c.res_in, c.res_in + 1, c.res_in};
-            set_grid(F, c.res_in, B, 4, gh, gw);
-            if (getenv("LA_INTERLEAVE")) set_interleaved(F);      // tuning switch: the cost-balanced contiguous split measured better
-        } else {
-            set_grid(F, c.res_in, B, c.up == 2 ? 4 : 1);
-        }
-        const bf16* a_hi = e->xs_hi[l & 1];
-        const bf16* a_lo = e->xs_lo[l & 1];
+        const Pl a{e->xs_hi[l & 1], e->xs_lo[l & 1]};
         const long long sW = c.cin, sH = static_cast<long long>(c.res_in) * c.cin, sN = sH * c.res_in;
-        LA(make_a_map(&F.a_map[0], a_hi, c.cin, c.res_in, c.res_in, B, sW, sH, sN, F.tw, F.th + F.halo, F.nb));
-        if (split) LA(make_a_map(&F.a_map[1], a_lo, c.cin, c.res_in, c.res_in, B, sW, sH, sN, F.tw, F.th + F.halo, F.nb));
         c.fwd_ops = TapSimtOperands{};
-        c.fwd_ops.a_ptrs[0] = a_hi; c.fwd_ops.a_ptrs[1] = a_lo;
+        c.fwd_ops.a_ptrs[0] = a.hi; c.fwd_ops.a_ptrs[1] = a.lo;
         c.fwd_ops.a_sw = sW; c.fwd_ops.a_sh = sH; c.fwd_ops.a_sn = sN;
         set_ops_dims(c.fwd_ops, c.res_in, c.res_in);
         c.fwd_ops.w = c.wf;
-        const int bn = pick_bn(c.cout, F.m_tiles);
-        LA(make_b_map(F, c.wf, c.cin, c.cout, nmat * (split ? 2 : 1), bn, c.split_up ? 0 : 1));
-        int nt = 0;
-        for (int ph = 0; ph < F.nprob; ++ph) {
-            F.prob[ph].tap_begin = nt;
-            if (c.split_up) {   // transposed conv, stride 2: T[2i+a] += x[i] W[a]  ->  taps with a = phase (mod 2), x offset -(a >> 1)
-                for (int ay = ph / 2; ay < 3; ay += 2)
-                    for (int ax = ph % 2; ax < 3; ax += 2) add_tap(F, nt, -(ay >> 1), -(ax >> 1), ay * 3 + ax, 0, 1, nmat, split);
-            } else {
-                for (int t = 0; t < 9; ++t) add_tap(F, nt, t / 3 - 1, t % 3 - 1, ph * 9 + t, 0, 1, nmat, split);
-            }
-            F.prob[ph].ntaps = nt - F.prob[ph].tap_begin;
-            F.prob[ph].oy0 = c.up == 2 ? ph / 2 : 0;
-            F.prob[ph].ox0 = c.up == 2 ? ph % 2 : 0;
-        }
-        F.kchunks = c.cin / 64; F.n_total = c.cout; F.n_blocks = c.cout / bn;
-        F.epilogue = kEpiFwd;
-        F.OH = F.OW = c.res; F.osy = F.osx = c.up; F.split = split;
+        // the layer's epilogue constants (the split layers' FIR pass applies them)
         F.act_gain = 1.41421356237309515f; F.act_clamp = g.conv_clamp; F.act_slope = 0.2f;
         F.demod = e->d_cat + static_cast<size_t>(B) * c.doff;
         F.bias = c.p.d_bias;
         F.noise = c.p.d_noise_const; F.noise_stride_n = 0; F.noise_scale = c.p.noise_strength;
-        F.s_next = next ? e->s_cat + static_cast<size_t>(B) * next->soff : nullptr;
-        F.x_hi = c.x_hi; F.x_lo = c.x_lo;
-        F.xs_hi = e->xs_hi[(l + 1) & 1]; F.xs_lo = e->xs_lo[(l + 1) & 1];
-        F.rgbw = rgb ? e->rgbw + static_cast<size_t>(B) * rgb->roff : nullptr;
-        F.rgb_part = rgb ? rgb->parts : nullptr;
         F.err_flag = e->err_flag;
-        const int TH = c.res + 1, TWp = c.res + 2;      // T rows / row pitch of the split up-sampling layers
-        if (c.split_up) {
+        const float* s_next = next ? e->s_cat + static_cast<size_t>(B) * next->soff : nullptr;
+        const Pl xs{e->xs_hi[(l + 1) & 1], e->xs_lo[(l + 1) & 1]};
+        if (c.split_up) {       // the GEMM stores T, the FIR pass applies the layer's epilogue
             UpFirParams& U = c.fir;
             memset(&U, 0, sizeof U);
             U.t_hi = e->t_hi; U.t_lo = e->t_lo;
-            U.B = B; U.OH = U.OW = c.res; U.C = c.cout; U.TH = TH; U.TWp = TWp; U.split = split;
+            U.B = B; U.OH = U.OW = c.res; U.C = c.cout; U.TH = c.res + 1; U.TWp = c.res + 2; U.split = split;
             U.demod = F.demod; U.bias = F.bias; U.noise = F.noise; U.noise_stride_n = 0; U.noise_scale = F.noise_scale;
-            U.s_next = F.s_next; U.x_hi = F.x_hi; U.x_lo = F.x_lo; U.xs_hi = F.xs_hi; U.xs_lo = F.xs_lo;
+            U.s_next = s_next; U.x_hi = c.x_hi; U.x_lo = c.x_lo; U.xs_hi = xs.hi; U.xs_lo = xs.lo;
             U.act_gain = F.act_gain; U.act_clamp = F.act_clamp; U.act_slope = F.act_slope;
             for (int jy = 0; jy < 4; ++jy)       // true convolution (flipped filter), gain up^2 = 4 (upfirdn2d.py:196-199)
                 for (int jx = 0; jx < 4; ++jx) U.fk[jy * 4 + jx] = e->fir_host[(3 - jy) * 4 + (3 - jx)] * 4.f;
-            {   // rank-1 test: fk = fy (x) fx with fy = column of the largest entry / that entry, fx = its row
-                int bi = 0;
-                for (int k = 1; k < 16; ++k) if (fabsf(U.fk[k]) > fabsf(U.fk[bi])) bi = k;
-                const int by = bi / 4, bx = bi % 4;
-                U.separable = U.fk[bi] != 0.f;
-                for (int k = 0; k < 4 && U.separable; ++k) { U.fy[k] = U.fk[k * 4 + bx] / U.fk[bi]; U.fx[k] = U.fk[by * 4 + k]; }
-                for (int k = 0; k < 16 && U.separable; ++k)
-                    if (fabsf(U.fy[k / 4] * U.fx[k % 4] - U.fk[k]) > 1e-6f * fabsf(U.fk[bi])) U.separable = 0;
-            }
             U.gy_hi = e->gy_hi[l & 1]; U.gy_lo = e->gy_lo[l & 1]; U.gt_hi = e->t_hi; U.gt_lo = e->t_lo;
-            static const bool no_fir_tma = getenv("LA_NO_FIR_TMA") != nullptr;
-            if (!split && U.separable && c.res >= 32 && c.cout % 64 == 0 && !no_fir_tma) {
-                const uint64_t C = c.cout, R = c.res;
-                const uint64_t tdims[4] = {C, R + 1, R + 1, static_cast<uint64_t>(B)};          // T: (2H+1) x (2W+1), row pitch TWp
-                const uint64_t tstr[3] = {C * 2, static_cast<uint64_t>(TWp) * C * 2, static_cast<uint64_t>(TH) * TWp * C * 2};
-                const uint64_t ydims[4] = {C, R, R, static_cast<uint64_t>(B)};
-                const uint64_t ystr[3] = {C * 2, R * C * 2, R * R * C * 2};
-                const uint32_t lbox[4] = {64, 35, 1, 1}, sbox[4] = {64, 8, 1, 1};
-                int r = encode_tmap_bf16(&U.fwd_in, e->t_hi, 4, tdims, tstr, lbox, 0);
-                r |= encode_tmap_bf16(&U.fwd_out_x, c.x_hi, 4, ydims, ystr, sbox, 0);
-                if (next) r |= encode_tmap_bf16(&U.fwd_out_xs, e->xs_hi[(l + 1) & 1], 4, ydims, ystr, sbox, 0);
-                r |= encode_tmap_bf16(&U.bwd_in, e->gy_hi[l & 1], 4, ydims, ystr, lbox, 0);
-                r |= encode_tmap_bf16(&U.bwd_out, e->t_hi, 4, tdims, tstr, sbox, 0);
-                if (r) return fail(-5, "tensor map encoding failed (FIR pass)");
-                U.use_tma = 1;
+            if (upfir_plan(U)) return fail(-5, "tensor map encoding failed (FIR pass)");
+            // tuning switch LA_INTERLEAVE: the cost-balanced contiguous split measured better
+            LA(plan_upconv(F, a, B, c.res_in, c.cin, c.cout, c.wf, split, Pl{e->t_hi, e->t_lo}, getenv("LA_INTERLEAVE") != nullptr));
+        } else {
+            set_grid(F, c.res_in, B, c.up == 2 ? 4 : 1);
+            LA(make_a_map(&F.a_map[0], a.hi, c.cin, c.res_in, c.res_in, B, sW, sH, sN, F.tw, F.th + F.halo, F.nb));
+            if (split) LA(make_a_map(&F.a_map[1], a.lo, c.cin, c.res_in, c.res_in, B, sW, sH, sN, F.tw, F.th + F.halo, F.nb));
+            const int bn = pick_bn(c.cout, F.m_tiles);
+            LA(make_b_map(F, c.wf, c.cin, c.cout, nmat * (split ? 2 : 1), bn, 1));
+            int nt = 0;
+            for (int ph = 0; ph < F.nprob; ++ph) {
+                F.prob[ph].tap_begin = nt;
+                for (int t = 0; t < 9; ++t) add_tap(F, nt, t / 3 - 1, t % 3 - 1, ph * 9 + t, 0, 1, nmat, split);
+                F.prob[ph].ntaps = nt - F.prob[ph].tap_begin;
+                F.prob[ph].oy0 = c.up == 2 ? ph / 2 : 0;
+                F.prob[ph].ox0 = c.up == 2 ? ph % 2 : 0;
             }
-            // the GEMM only stores T
-            F.epilogue = kEpiStoreBf16;
-            F.OH = TH; F.OW = TWp;
-            F.x_hi = e->t_hi; F.x_lo = e->t_lo;
-            F.xs_hi = F.xs_lo = nullptr; F.s_next = nullptr; F.rgbw = nullptr;
+            F.kchunks = c.cin / 64; F.n_total = c.cout; F.n_blocks = c.cout / bn;
+            F.epilogue = kEpiFwd;
+            F.OH = F.OW = c.res; F.osy = F.osx = c.up; F.split = split;
+            F.s_next = s_next;
+            F.x_hi = c.x_hi; F.x_lo = c.x_lo;
+            F.xs_hi = xs.hi; F.xs_lo = xs.lo;
+            F.rgbw = rgb ? e->rgbw + static_cast<size_t>(B) * rgb->roff : nullptr;
+            F.rgb_part = rgb ? rgb->parts : nullptr;
+            // staged stores + coefficient tables in the row-owner epilogues (bf16 mode, one sample per tile)
+            if (!split && !no_staged() && F.nb == 1 && c.up == 1) F.staged = 1;
+            if (tapgemm_finalize(F)) return fail(-2, "tap grouping failed");
         }
-
-        // staged stores + coefficient tables in the row-owner epilogues (bf16 mode, one sample per tile)
-        static const bool no_staged = getenv("LA_NO_STAGED") != nullptr;
-        if (!split && !no_staged && F.nb == 1 && (c.split_up || c.up == 1)) F.staged = 1;
 
         // ---------------------------------------------------------------- data gradient
         TapGemmParams& G = c.bwd;
@@ -338,8 +300,7 @@ int build_params(la_engine* e) {
         const bf16* gy_lo = e->gy_lo[l & 1];
         c.bwd_ops = TapSimtOperands{};
         c.bwd_ops.w = c.wb;
-        nt = 0;
-        G.prob[0].tap_begin = 0;
+        int nt = 0;
         if (c.up == 1) {
             const long long gW = c.cout, gH = static_cast<long long>(c.res) * c.cout, gN = gH * c.res;
             LA(make_a_map(&G.a_map[0], gy_hi, c.cout, c.res, c.res, B, gW, gH, gN, G.tw, G.th + G.halo, G.nb));
@@ -350,26 +311,7 @@ int build_params(la_engine* e) {
             for (int t = 0; t < 9; ++t) add_tap(G, nt, 1 - t / 3, 1 - t % 3, t, 0, 1, nmat, split);
         } else if (c.split_up) {
             // g_xs[i] = sum_a g_T[2i + a] W[a]^T : four phase-strided views of g_T, 9 taps
-            const long long gW = 2LL * c.cout, gH = 2LL * TWp * c.cout, gN = static_cast<long long>(TH) * TWp * c.cout;
-            c.bwd_ops.a_sw = gW; c.bwd_ops.a_sh = gH; c.bwd_ops.a_sn = gN;
-            for (int ph = 0; ph < 4; ++ph) {
-                const int py = ph / 2, px = ph % 2;
-                const int ph_h = c.res_in + (py == 0), ph_w = c.res_in + (px == 0);
-                const long long off = (static_cast<long long>(py) * TWp + px) * c.cout;
-                LA(make_a_map(&G.a_map[ph], e->t_hi + off, c.cout, ph_w, ph_h, B, gW, gH, gN, G.tw, G.th + G.halo, G.nb));
-                c.bwd_ops.a_ptrs[ph] = e->t_hi + off;
-                c.bwd_ops.a_ws[ph] = ph_w; c.bwd_ops.a_hs[ph] = ph_h;
-                if (split) {
-                    LA(make_a_map(&G.a_map[4 + ph], e->t_lo + off, c.cout, ph_w, ph_h, B, gW, gH, gN, G.tw, G.th + G.halo, G.nb));
-                    c.bwd_ops.a_ptrs[4 + ph] = e->t_lo + off;
-                    c.bwd_ops.a_ws[4 + ph] = ph_w; c.bwd_ops.a_hs[4 + ph] = ph_h;
-                }
-            }
-            for (int ay = 0; ay < 3; ++ay)
-                for (int ax = 0; ax < 3; ++ax) {
-                    const int ph = (ay & 1) * 2 + (ax & 1);
-                    add_tap(G, nt, ay >> 1, ax >> 1, ay * 3 + ax, ph, 4 + ph, nmat, split);
-                }
+            LA(phase_view_taps(G, nt, Pl{e->t_hi, e->t_lo}, B, c.res, c.cout, split, &c.bwd_ops));
         } else {
             const long long gW = 2LL * c.cout, gH = 2LL * c.res * c.cout, gN = static_cast<long long>(c.res) * c.res * c.cout;
             for (int ph = 0; ph < 4; ++ph) {
@@ -387,7 +329,7 @@ int build_params(la_engine* e) {
                 for (int t = 0; t < 9; ++t) add_tap(G, nt, -(t / 3 - 1), -(t % 3 - 1), ph * 9 + t, ph, 4 + ph, nmat, split);
         }
         G.prob[0].ntaps = nt;
-        if (tapgemm_finalize(F) || tapgemm_finalize(G)) return fail(-2, "tap grouping failed");
+        if (tapgemm_finalize(G)) return fail(-2, "tap grouping failed");
         F.no_pair = G.no_pair = getenv("LA_NO_PAIR") != nullptr;
         F.dbg_skip_epi = G.dbg_skip_epi = getenv("LA_DBG_SKIP_EPI") != nullptr;     // timing experiment (DESIGN.md §7): wrong results
         const int bnb = pick_bn(c.cin, G.m_tiles);

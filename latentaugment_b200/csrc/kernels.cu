@@ -2,10 +2,12 @@
 #include "kernels.cuh"
 
 #include <cuda_bf16.h>
+#include <stdlib.h>
 
 #include "act.cuh"
 #include "common.cuh"
 #include "sm100.cuh"
+#include "tapgemm.cuh"
 
 namespace la {
 
@@ -1078,6 +1080,34 @@ static int max_cin(const LayerTable& T, bool conv, bool rgb) {
     if (conv) for (int i = 0; i < T.nconv; ++i) m = T.conv[i].cin > m ? T.conv[i].cin : m;
     if (rgb) for (int i = 0; i < T.nrgb; ++i) m = T.rgb[i].cin > m ? T.rgb[i].cin : m;
     return m;
+}
+
+int upfir_plan(UpFirParams& U) {
+    {   // rank-1 test: fk = fy (x) fx with fy = column of the largest entry / that entry, fx = its row
+        int bi = 0;
+        for (int k = 1; k < 16; ++k) if (fabsf(U.fk[k]) > fabsf(U.fk[bi])) bi = k;
+        const int by = bi / 4, bx = bi % 4;
+        U.separable = U.fk[bi] != 0.f;
+        for (int k = 0; k < 4 && U.separable; ++k) { U.fy[k] = U.fk[k * 4 + bx] / U.fk[bi]; U.fx[k] = U.fk[by * 4 + k]; }
+        for (int k = 0; k < 16 && U.separable; ++k)
+            if (fabsf(U.fy[k / 4] * U.fx[k % 4] - U.fk[k]) > 1e-6f * fabsf(U.fk[bi])) U.separable = 0;
+    }
+    static const bool no_fir_tma = getenv("LA_NO_FIR_TMA") != nullptr;
+    if (U.split || !U.separable || U.OW < 32 || U.C % 64 || no_fir_tma) return 0;
+    const uint64_t C = U.C, B = U.B;
+    const uint64_t tdims[4] = {C, static_cast<uint64_t>(U.OW) + 1, static_cast<uint64_t>(U.TH), B};     // T's valid columns, pitch TWp
+    const uint64_t tstr[3] = {C * 2, static_cast<uint64_t>(U.TWp) * C * 2, static_cast<uint64_t>(U.TH) * U.TWp * C * 2};
+    const uint64_t ydims[4] = {C, static_cast<uint64_t>(U.OW), static_cast<uint64_t>(U.OH), B};
+    const uint64_t ystr[3] = {C * 2, static_cast<uint64_t>(U.OW) * C * 2, static_cast<uint64_t>(U.OH) * U.OW * C * 2};
+    const uint32_t lbox[4] = {64, 35, 1, 1}, sbox[4] = {64, 8, 1, 1};
+    int r = encode_tmap_bf16(&U.fwd_in, U.t_hi, 4, tdims, tstr, lbox, 0);
+    r |= encode_tmap_bf16(&U.fwd_out_x, U.x_hi, 4, ydims, ystr, sbox, 0);
+    if (U.s_next) r |= encode_tmap_bf16(&U.fwd_out_xs, U.xs_hi, 4, ydims, ystr, sbox, 0);
+    r |= encode_tmap_bf16(&U.bwd_in, U.gy_hi, 4, ydims, ystr, lbox, 0);
+    r |= encode_tmap_bf16(&U.bwd_out, U.gt_hi, 4, tdims, tstr, sbox, 0);
+    if (r) return -5;
+    U.use_tma = 1;
+    return 0;
 }
 
 static int upfir_launch(const UpFirParams& p, bool fwd, cudaStream_t s) {

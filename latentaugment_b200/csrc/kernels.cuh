@@ -72,6 +72,10 @@ struct UpFirParams {
     alignas(64) CUtensorMap fwd_in, fwd_out_x, fwd_out_xs;     // T -> x, x * s_next
     alignas(64) CUtensorMap bwd_in, bwd_out;                   // g_y -> g_T
 };
+// Completes U once its sizes, buffers and fk are set: fk's rank-1 factorisation fy (x) fx (separable) and, where the TMA
+// variant applies (LA_NO_FIR_TMA switches it off), its tensor maps: fwd_in <- t_hi, fwd_out_x <- x_hi, fwd_out_xs <- xs_hi
+// (when s_next is set), bwd_in <- gy_hi, bwd_out <- gt_hi.  Returns 0 or -5.
+int upfir_plan(UpFirParams& U);
 int upfir_forward(const UpFirParams& p, cudaStream_t s);
 int upfir_backward(const UpFirParams& p, cudaStream_t s);
 

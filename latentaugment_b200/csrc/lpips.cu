@@ -336,17 +336,6 @@ inline int tap_grid(long long pixels, int num_sms) {
     return static_cast<int>(want < cap ? want : cap);
 }
 
-int conv_taps(int split, TapGemmParams& P, bool flipped) {
-    int nt = 0;
-    P.prob[0].tap_begin = 0;
-    for (int t = 0; t < 9; ++t) {
-        const int dy = t / 3 - 1, dx = t % 3 - 1;
-        add_tap(P, nt, flipped ? -dy : dy, flipped ? -dx : dx, t, 0, 1, 9, split);
-    }
-    P.prob[0].ntaps = nt;
-    return tapgemm_finalize(P);
-}
-
 int plan_lpips(la_lpips* L, char* ws, size_t* bytes_out) {
     const la_vgg_desc& d = L->d;
     const int cs = d.crop_size, split = L->split;
@@ -366,9 +355,8 @@ int plan_lpips(la_lpips* L, char* ws, size_t* bytes_out) {
     Bump bp;
     bp.base = ws;
     const size_t n = L->ncrops, wm = split ? 2 : 1;
-    auto take_pl = [&](size_t cnt) { Pl t; t.hi = bp.take<bf16>(cnt); t.lo = split ? bp.take<bf16>(cnt) : nullptr; return t; };
-    L->x_in = take_pl(n * cs * cs * 64);
-    L->g_in = take_pl(n * cs * cs * 64);
+    L->x_in = bp.take_pl(n * cs * cs * 64, split);
+    L->g_in = bp.take_pl(n * cs * cs * 64, split);
     size_t max_x = 0, max_p = 0;
     for (int i = 0; i <= L->last_conv; ++i) {
         Conv& c = L->conv[i];
@@ -376,24 +364,24 @@ int plan_lpips(la_lpips* L, char* ws, size_t* bytes_out) {
         c.wf = bp.take<bf16>(wm * 9 * c.cout * c.cin_pad);
         c.wb = bp.take<bf16>(wm * 9 * c.cout * c.cin_pad);
         const size_t xs = n * c.R * c.R * c.cout;
-        c.x = take_pl(xs);
+        c.x = bp.take_pl(xs, split);
         max_x = xs > max_x ? xs : max_x;
     }
     for (int k = 0; k < 4; ++k) {
         const int ci = kTapConv[k];
         if (ci + 1 > L->last_conv) break;
         const size_t ps = n * (L->conv[ci].R / 2) * (L->conv[ci].R / 2) * L->conv[ci].cout;
-        L->pool[k] = take_pl(ps);
+        L->pool[k] = bp.take_pl(ps, split);
         max_p = ps > max_p ? ps : max_p;
     }
-    L->gp = take_pl(max_p ? max_p : 64);
-    L->gz[0] = take_pl(max_x);
-    L->gz[1] = take_pl(max_x);
+    L->gp = bp.take_pl(max_p ? max_p : 64, split);
+    L->gz[0] = bp.take_pl(max_x, split);
+    L->gz[1] = bp.take_pl(max_x, split);
     for (int t = 0; t < LA_VGG_TAPS; ++t) {
         TapL& T = L->tap[t];
         if (!T.used) continue;
         T.bank_mean = bp.take<float>(static_cast<size_t>(L->imgc) * T.R * T.R * T.C);
-        if (T.conv != L->last_conv) T.tg = take_pl(n * T.R * T.R * T.C);
+        if (T.conv != L->last_conv) T.tg = bp.take_pl(n * T.R * T.R * T.C, split);
         T.target = d.per_sample_targets ? bp.take<float>(n * T.R * T.R * T.C) : nullptr;    // fp32, ~32 MB per crop at a 256 window
     }
     L->ones = bp.take<float>(n * 512);
@@ -407,32 +395,22 @@ int plan_lpips(la_lpips* L, char* ws, size_t* bytes_out) {
 }
 
 int build_lpips(la_lpips* L) {
-    const int split = L->split, wm = split ? 2 : 1;
+    const int split = L->split;
     for (int i = 0; i <= L->last_conv; ++i) {
         Conv& c = L->conv[i];
         bool pooled_in = false;
         int pk = -1;
         for (int k = 0; k < 4; ++k) if (kTapConv[k] + 1 == i) { pooled_in = true; pk = k; }
         const Pl& in = i == 0 ? L->x_in : (pooled_in ? L->pool[pk] : L->conv[i - 1].x);
-        LA(vgg_conv_fwd_plan(c.F, c.R, L->ncrops, c.cin_pad, c.cout, in, c.wf, split, L->d.d_conv_bias[i], L->ones, c.x, L->err_flag));
-        {   // data gradient: g_z (wrt this conv's pre-activation) -> gradient wrt its input
-            TapGemmParams& P = c.B;
-            memset(&P, 0, sizeof P);
-            set_grid(P, c.R, L->ncrops, 1);
-            LA(dense_maps(P, L->gz[i & 1], L->ncrops, c.cout, c.R, c.R, P.tw, P.th + P.halo, P.nb, split));
-            const int bn = choose_bn(c.cin_pad, P.m_tiles);
-            LA(make_b_map(P, c.wb, c.cout, c.cin_pad, 9 * wm, bn));
-            P.kchunks = c.cout / 64;
-            P.epilogue = kEpiLinear;
-            P.n_total = c.cin_pad; P.n_blocks = c.cin_pad / bn;
-            P.OH = P.OW = c.R; P.osy = P.osx = 1; P.split = split;
-            P.act_gain = 1.f; P.act_clamp = -1.f; P.act_slope = 0.f;
-            if (i == 0) { P.lin_out = L->g_in.hi; P.lin_out_lo = L->g_in.lo; }
-            else if (pooled_in) { P.lin_out = L->gp.hi; P.lin_out_lo = L->gp.lo; }
-            else { P.lin_saved = L->conv[i - 1].x.hi; P.lin_gz = L->gz[(i - 1) & 1].hi; P.lin_gz_lo = L->gz[(i - 1) & 1].lo; }
-            P.err_flag = L->err_flag;
-            LA(conv_taps(split, P, true));
-        }
+        LA(plan_layer(c.F, LayerTaps::k3x3, in, L->ncrops, c.R, c.cin_pad, c.cout, c.wf, split, L->err_flag));
+        fwd_epilogue(c.F, L->ones, L->d.d_conv_bias[i], 1.f, -1.f, 0.f, c.x);                  // ReLU
+        // data gradient: g_z (wrt this conv's pre-activation) -> gradient wrt its input
+        TapGemmParams& P = c.B;
+        LA(plan_layer(P, LayerTaps::k3x3Flipped, L->gz[i & 1], L->ncrops, c.R, c.cout, c.cin_pad, c.wb, split, L->err_flag));
+        linear_epilogue(P, 0.f);
+        if (i == 0) { P.lin_out = L->g_in.hi; P.lin_out_lo = L->g_in.lo; }
+        else if (pooled_in) { P.lin_out = L->gp.hi; P.lin_out_lo = L->gp.lo; }
+        else { P.lin_saved = L->conv[i - 1].x.hi; P.lin_gz = L->gz[(i - 1) & 1].hi; P.lin_gz_lo = L->gz[(i - 1) & 1].lo; }
     }
     return 0;
 }
@@ -452,9 +430,6 @@ int prepare_lpips(la_lpips* L, cudaStream_t s) {
     CU(cudaStreamSynchronize(s));
     return 0;
 }
-
-inline unsigned* U32(bf16* p) { return reinterpret_cast<unsigned*>(p); }
-inline const unsigned* CU32(const bf16* p) { return reinterpret_cast<const unsigned*>(p); }
 
 // convs + pools from x_in up to the last used tap
 int run_network(la_lpips* L, cudaStream_t s, long long* launches) {
@@ -477,27 +452,6 @@ namespace la {
 
 int vgg_prep_weights(const float* w, int cout, int cin, int cin_pad, int split, bf16* wf, bf16* wb, cudaStream_t s) {
     return prep_plain_weights(w, cout, cin, 9, 1.f, cin_pad, split, wf, wb, s);
-}
-
-int vgg_conv_fwd_plan(TapGemmParams& P, int R, int n, int cin_pad, int cout, const Pl& in, const bf16* wf, int split, const float* bias,
-                      const float* ones, const Pl& out, int* err_flag) {
-    const int wm = split ? 2 : 1;
-    memset(&P, 0, sizeof P);
-    set_grid(P, R, n, 1);
-    LA(dense_maps(P, in, n, cin_pad, R, R, P.tw, P.th + P.halo, P.nb, split));
-    const int bn = choose_bn(cout, P.m_tiles);
-    LA(make_b_map(P, wf, cin_pad, cout, 9 * wm, bn));
-    P.kchunks = cin_pad / 64;
-    P.epilogue = kEpiFwd;
-    P.n_total = cout; P.n_blocks = cout / bn;
-    P.OH = P.OW = R; P.osy = P.osx = 1; P.split = split;
-    P.act_gain = 1.f; P.act_clamp = -1.f; P.act_slope = 0.f;           // ReLU
-    P.demod = ones; P.bias = bias;
-    P.x_hi = out.hi; P.x_lo = out.lo;
-    P.staged = P.nb == 1 && !split && !getenv("LA_NO_STAGED");
-    P.err_flag = err_flag;
-    LA(conv_taps(split, P, false));
-    return 0;
 }
 
 int vgg_pool_fwd(const Pl& x, int n, int R, int C, const Pl& out, cudaStream_t s) {

@@ -1,7 +1,9 @@
 // Host-side planning helpers shared by the clients of the tap-GEMM (engine, discriminator, VGG16 in lpips.cu / detector.cu):
-// tile geometry, column-block choice, TMA tensor maps and tap lists of one tap-GEMM launch.
+// tile geometry, column-block choice, TMA tensor maps and tap lists of one tap-GEMM launch, and the planners of the plain
+// layers, of the four-phase transposed stride-2 convolution and of the stride-2 convolution over its phase views.
 #pragma once
 #include <stdlib.h>
+#include <string.h>
 
 #include "common.cuh"
 #include "tapgemm.cuh"
@@ -59,6 +61,11 @@ inline int pair_mode() {
     static const int v = getenv("LA_CTA2") ? atoi(getenv("LA_CTA2")) : 1;
     return v;
 }
+// LA_NO_STAGED: the row-owner epilogues store bf16 outputs per element instead of staging them (A-B switch).
+inline bool no_staged() {
+    static const bool v = getenv("LA_NO_STAGED") != nullptr;
+    return v;
+}
 // Weight tensor map of a launch [K, rows, nmat]; decides the CTA-pair mode of the launch: a pair's CTAs load
 // half a column block each.
 inline int make_b_map(TapGemmParams& P, const void* base, int K, int rows, int nmat, int bn, int pair128 = 0) {
@@ -109,5 +116,120 @@ inline void set_interleaved(TapGemmParams& P) {
     P.interleave = 1;
 }
 
+// ------------------------------------------------------------------------- plain layers
+// Every planner below returns 0 or the failing call's code; the caller reports it under its own module name.
+
+// Weights w [nmat][N][K] (residual planes behind them when split) of a launch whose grid is set: N columns in blocks of bn
+// (0: choose_bn), K / 64 chunks per tap.
+inline int plan_columns(TapGemmParams& P, const __nv_bfloat16* w, int K, int N, int nmat, int split, int bn = 0) {
+    if (!bn) bn = choose_bn(N, P.m_tiles);
+    if (int r = make_b_map(P, w, K, N, nmat * (split ? 2 : 1), bn)) return r;
+    P.kchunks = K / 64; P.n_total = N; P.n_blocks = N / bn; P.split = split;
+    return 0;
+}
+
+enum class LayerTaps {
+    k3x3,          // 3x3 convolution, pad 1: out[y, x] += in[y + dy, x + dx] W[(dy + 1) * 3 + dx + 1]
+    k3x3Flipped,   // its data gradient (offsets negated)
+    k1x1,
+    kDense,        // fully connected over the whole R x R x K input: one tap per input position, a 1 x 1 output, so
+                   // the M rows are samples (128 per tile, tile_geometry of a 1 x 1 grid)
+};
+
+// P <- a launch over the dense NHWC input in [n, R, R, K] (hi, plus lo when split) with N output columns and weights w
+// [taps][N][K]: everything but the epilogue, which fwd_epilogue / linear_epilogue (or the caller) sets.  bn = 0: choose_bn.
+inline int plan_layer(TapGemmParams& P, LayerTaps taps, const Pl& in, int n, int R, int K, int N, const __nv_bfloat16* w, int split,
+                      int* err_flag, int bn = 0) {
+    const bool dense = taps == LayerTaps::kDense;
+    const int g = dense ? 1 : R;
+    const int nmat = dense ? R * R : taps == LayerTaps::k1x1 ? 1 : 9;
+    memset(&P, 0, sizeof P);
+    set_grid(P, g, n, 1);
+    if (int r = dense_maps(P, in, n, K, R, R, P.tw, P.th + P.halo, P.nb, split)) return r;
+    if (int r = plan_columns(P, w, K, N, nmat, split, bn)) return r;
+    P.OH = P.OW = g; P.osy = P.osx = 1;
+    P.err_flag = err_flag;
+    int nt = 0;
+    for (int t = 0; t < nmat; ++t) {
+        int dy = 0, dx = 0;
+        if (dense) { dy = t / R; dx = t % R; }
+        else if (nmat == 9) { dy = t / 3 - 1; dx = t % 3 - 1; }
+        if (taps == LayerTaps::k3x3Flipped) { dy = -dy; dx = -dx; }
+        add_tap(P, nt, dy, dx, t, 0, 1, nmat, split);
+    }
+    P.prob[0].ntaps = nt;
+    return tapgemm_finalize(P);
+}
+
+// Unmodulated forward epilogue: out = act(acc + bias) (act.cuh: gain, clamp, slope), demod = ones (>= batch * N 1.0f).
+inline void fwd_epilogue(TapGemmParams& P, const float* ones, const float* bias, float gain, float clamp, float slope, const Pl& out) {
+    P.epilogue = kEpiFwd;
+    P.act_gain = gain; P.act_clamp = clamp; P.act_slope = slope;
+    P.demod = ones; P.bias = bias;
+    P.x_hi = out.hi; P.x_lo = out.lo;
+    P.staged = P.nb == 1 && !P.split && !no_staged();
+}
+// kEpiLinear with gain 1 and no clamp; slope is the producer activation's (its gradient, when lin_gz is set).
+inline void linear_epilogue(TapGemmParams& P, float slope) {
+    P.epilogue = kEpiLinear;
+    P.act_gain = 1.f; P.act_clamp = -1.f; P.act_slope = slope;
+}
+
+// ------------------------------------------------------------------------- stride-2 convolutions through T
+// T [n, 2R + 1, 2R + 2, C] (rows, row pitch) holds a transposed stride-2 3x3 convolution of an R x R input before its FIR pass
+// (the x2 up-sampling of the generator, the gradient of the discriminator's stride-2 conv1).
+
+// P <- the transposed stride-2 3x3 convolution of the dense NHWC input in [n, R, R, K] into T = t with N channels (weights w
+// [9][N][K]): T[2i + a] += in[i] W[a], so output phase (py, px) = (T[2i + py], T[2j + px]) is problem py * 2 + px of the launch
+// with the taps whose a = phase (mod 2); the even phases have one more row / column.  kEpiStoreBf16.  Does not clear P: fields
+// the caller set before stay.  interleave: walk the phases interleaved (set_interleaved).
+inline int plan_upconv(TapGemmParams& P, const Pl& in, int n, int R, int K, int N, const __nv_bfloat16* w, int split, const Pl& t,
+                       bool interleave = false) {
+    const int gh[4] = {R + 1, R + 1, R, R}, gw[4] = {R + 1, R, R + 1, R};
+    set_grid(P, R, n, 4, gh, gw);
+    if (interleave) set_interleaved(P);
+    if (int r = dense_maps(P, in, n, K, R, R, P.tw, P.th + P.halo, P.nb, split)) return r;
+    if (int r = plan_columns(P, w, K, N, 9, split)) return r;
+    int nt = 0;
+    for (int ph = 0; ph < 4; ++ph) {
+        P.prob[ph].tap_begin = nt;
+        for (int ay = ph / 2; ay < 3; ay += 2)
+            for (int ax = ph % 2; ax < 3; ax += 2) add_tap(P, nt, -(ay >> 1), -(ax >> 1), ay * 3 + ax, 0, 1, 9, split);
+        P.prob[ph].ntaps = nt - P.prob[ph].tap_begin;
+        P.prob[ph].oy0 = ph / 2; P.prob[ph].ox0 = ph % 2;
+    }
+    P.epilogue = kEpiStoreBf16;
+    P.OH = 2 * R + 1; P.OW = 2 * R + 2; P.osy = P.osx = 2;
+    P.x_hi = t.hi; P.x_lo = t.lo;
+    P.staged = P.nb == 1 && !split && !no_staged();
+    return tapgemm_finalize(P);
+}
+
+// A maps and taps of the stride-2 3x3 convolution over T = t [n, R + 1, R + 2, K] (plan_upconv's output for an R / 2 input),
+// read as its four phase views (py, px) = T[2i + py, 2j + px]: hi maps 0-3, lo maps 4-7, tap W[a] reads view a (mod 2) at
+// offset a >> 1.  P's grid (R / 2) must be set; the taps are appended at nt (as add_tap does) and the caller finalizes.  ops,
+// when given, gets the same views for the SIMT twin.
+inline int phase_view_taps(TapGemmParams& P, int& nt, const Pl& t, int n, int R, int K, int split, TapSimtOperands* ops = nullptr) {
+    const int TH = R + 1, TWp = R + 2, Ro = R / 2;
+    const long long gW = 2LL * K, gH = 2LL * TWp * K, gN = static_cast<long long>(TH) * TWp * K;
+    if (ops) { ops->a_sw = gW; ops->a_sh = gH; ops->a_sn = gN; }
+    for (int ph = 0; ph < 4; ++ph) {
+        const int py = ph / 2, px = ph % 2;
+        const int ph_h = Ro + (py == 0), ph_w = Ro + (px == 0);
+        const long long off = (static_cast<long long>(py) * TWp + px) * K;
+        for (int plane = 0; plane <= split; ++plane) {
+            const int m = ph + 4 * plane;
+            const __nv_bfloat16* base = (plane ? t.lo : t.hi) + off;
+            if (int r = make_a_map(&P.a_map[m], base, K, ph_w, ph_h, n, gW, gH, gN, P.tw, P.th + P.halo, P.nb)) return r;
+            if (ops) { ops->a_ptrs[m] = base; ops->a_ws[m] = ph_w; ops->a_hs[m] = ph_h; }
+        }
+    }
+    for (int ay = 0; ay < 3; ++ay)
+        for (int ax = 0; ax < 3; ++ax) {
+            const int ph = (ay & 1) * 2 + (ax & 1);
+            add_tap(P, nt, ay >> 1, ax >> 1, ay * 3 + ax, ph, 4 + ph, 9, split);
+        }
+    return 0;
+}
 
 }  // namespace la

@@ -1,12 +1,12 @@
 // Forward half of torchvision's VGG16 `features` on the tap-GEMM, shared by the perceptual term (lpips.cu) and the
-// VGG16 detector (detector.cu): weight preparation, the planning of one 3x3 convolution + bias + ReLU launch, and the
-// 2x2 max-pool.  Activations are NHWC bf16 (hi, plus the lo plane in split precision).  Implemented in lpips.cu.
+// VGG16 detector (detector.cu): weight preparation and the 2x2 max-pool.  Each 3x3 convolution + bias + ReLU is a plain
+// layer of plan.cuh (plan_layer, then fwd_epilogue with gain 1, no clamp and slope 0).  Activations are NHWC bf16 (hi, plus
+// the lo plane in split precision).  Implemented in lpips.cu.
 #pragma once
 #include <cuda_bf16.h>
 #include <cuda_runtime.h>
 
 #include "common.cuh"
-#include "tapgemm.cuh"
 
 namespace la {
 
@@ -19,9 +19,6 @@ constexpr int kPoolConv[5] = {1, 3, 6, 9, 12};                                 /
 // w [cout, cin, 3, 3] fp32 -> wf [9][cout][cin_pad] (forward operand) and, unless wb is null, wb [9][cin_pad][cout]
 // (data-gradient operand); zero padded, residual planes behind the main ones when split.
 int vgg_prep_weights(const float* w, int cout, int cin, int cin_pad, int split, __nv_bfloat16* wf, __nv_bfloat16* wb, cudaStream_t s);
-// P <- the launch  out[n, R, R, cout] = ReLU(conv3x3(in[n, R, R, cin_pad], wf) + bias)  (ones: >= n * cout 1.0f).
-int vgg_conv_fwd_plan(TapGemmParams& P, int R, int n, int cin_pad, int cout, const Pl& in, const __nv_bfloat16* wf, int split,
-                      const float* bias, const float* ones, const Pl& out, int* err_flag);
 // 2x2 max-pool x [n, R, R, C] -> out [n, R/2, R/2, C].
 int vgg_pool_fwd(const Pl& x, int n, int R, int C, const Pl& out, cudaStream_t s);
 
